@@ -2,6 +2,7 @@
 """bench.py -- MPC solves/sec (BASELINE.json metric) for the B200-native batched MPC solver.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--workload roadmap|line]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: B = 65 536 independent MPC::Solve problems
 (N=25 horizon).  Default workload = BASELINE.json configs[3]: a degree-3 reference fitted (on the GPU, K4) to
@@ -11,13 +12,17 @@ torch.distributed (NCCL) is used only for the barrier and the max-over-ranks of 
 gives every GPU its own B problems per step instead.
 
 value        whole-job solves/s with inputs already resident in HBM (device-pointer C-ABI call, CUDA events; the timed
-             region repeats the K-step sequence until it lasts --min-seconds)
+             region is exactly K steps)
 e2e          the same through the host-buffer C-ABI call the reference's MPC::Solve would bind: pinned host buffers,
-             H2D + D2H inside the timed region
+             H2D + D2H inside the timed region (K steps)
 lone_caller  one handle, one stream, one call at a time (the figures above overlap consecutive steps on several handles)
 one_process_multi_gpu (N > 1)  b200mpc_solve_batch_multi on the whole batch from rank 0: every GPU's shard queued from one host thread, host
              gather, per-call latency percentiles
 weak_scaling (N > 1)  the weak-scaling figure next to the strong one
+
+--dump-outputs DIR writes what the last timed step returned to its caller (out8 (8, B), obj, status, iters of the whole
+batch, as float64 .npy files; a fixed sample of problems with its index.npy when that would exceed 64 MB).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -233,6 +238,25 @@ class ClockSampler:
                     reasons=sorted(reasons), samples=len(self.rows), samples_under_load=len(sm))
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, outs):
+    """Writes the per-problem result arrays `outs` (problem index on the last axis) to path/<name>.npy as float64.  When
+    they would take more than DUMP_MAX_BYTES, a fixed seeded sample of problems is written instead, with its indices
+    (index.npy), so that the same arguments always select the same problems."""
+    n = next(iter(outs.values())).shape[-1]
+    per_problem = 8 * (sum(int(np.prod(a.shape[:-1])) for a in outs.values()) + 1)
+    budget = DUMP_MAX_BYTES - 4096   # room for the .npy headers
+    os.makedirs(path, exist_ok=True)
+    if n * per_problem > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // per_problem, replace=False))
+        outs = {k: a[..., idx] for k, a in outs.items()}
+        np.save(os.path.join(path, "index.npy"), idx.astype(np.float64))
+    for k, a in outs.items():
+        np.save(os.path.join(path, f"{k}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def auto_streams(per_gpu_batch):
     """Solver handles / streams whose consecutive steps overlap: 6 at 65 536 problems per GPU and step, more for the
     smaller per-GPU shards of a strong-scaled batch (about 6 x 65 536 problems in flight per GPU), at most 16."""
@@ -353,23 +377,27 @@ def run_ours(args):
     # warm-up: at least W steps, and every (solver handle, input set) pair once -- each pair is its own CUDA graph,
     # captured and instantiated at its first use
     wsteps = max(W, S * nsets // math.gcd(S, nsets))
-    e0, e1 = timed_device_region(dev_handles, streams, Bl, d_in, d_out, wsteps)
+    timed_device_region(dev_handles, streams, Bl, d_in, d_out, wsteps)
     barrier()
-    # the timed region is R repetitions of the K-step sequence, R chosen so that it lasts >= --min-seconds
-    e0, e1 = timed_device_region(dev_handles, streams, Bl, d_in, d_out, K)
-    barrier()
-    est_ms, _ = agreed(e0.elapsed_time(e1))
-    R = max(1, int(math.ceil(args.min_seconds * 1e3 / max(est_ms, 1e-3))))
     launches0 = sum(m.launch_count() for m in mpcs)
     sampler = ClockSampler(local)
     sampler.start()
     barrier()
-    e0, e1 = timed_device_region(dev_handles, streams, Bl, d_in, d_out, K * R)
+    e0, e1 = timed_device_region(dev_handles, streams, Bl, d_in, d_out, K)
     barrier()
     ms_total, per_rank_total = agreed(e0.elapsed_time(e1))
     launches = sum(m.launch_count() for m in mpcs) - launches0
-    per_rank_ms = [x / (K * R) for x in per_rank_total]
-    value = throughput(total_per_step, K * R, ms_total)
+    per_rank_ms = [x / K for x in per_rank_total]
+    value = throughput(total_per_step, K, ms_total)
+    if args.dump_outputs:   # step K - 1 wrote the output set of its handle, which no later leg touches
+        last = {k: v.cpu().numpy() for k, v in d_out[(K - 1) % len(dev_handles)].items()}
+        if world > 1:   # rank 0 writes the whole batch (strong) or its own copy of it (weak)
+            shards = [None] * world if rank == 0 else None
+            dist.gather_object(last, shards, dst=0, group=cpu_group)
+            if rank == 0 and strong:
+                last = {k: np.concatenate([s[k] for s in shards], axis=-1) for k in last}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last)
 
     # ---- one caller, one call at a time: 1 handle (library defaults: the call is cut into 4 concurrent sub-batches
     # inside), 1 stream; every solve bracketed by CUDA events inside the C ABI (b200mpc_set_timing)
@@ -453,7 +481,7 @@ def run_ours(args):
     for i in range(max(3, S)):   # every handle of the leg allocates its staging buffers and captures its graph here
         host_step(i, i % S)
     barrier()
-    n_e2e = K * R
+    n_e2e = K
     with ThreadPoolExecutor(T) as ex:
         t0 = time.perf_counter()
         list(ex.map(lambda k: worker(k, n_e2e), range(T)))
@@ -528,7 +556,7 @@ def run_ours(args):
         # device time of the solver kernels per step, read both ways: (a) with S overlapped streams the per-step share of
         # the timed region (the intervals of consecutive steps overlap); (b) one stream, one call at a time: the
         # first-to-last-kernel interval of each solve (CUDA events inside the C ABI)
-        avg_kernel_ms = ms_total / (K * R)
+        avg_kernel_ms = ms_total / K
         lone_kernel_ms = lone_kern_ms / max(1, lone_kern_n)
         achieved = flop_per_step / (avg_kernel_ms * 1e-3) / 1e12 / world      # per GPU
         lone_achieved = f_iter(HORIZON) * mean_it * Bl / (lone_kernel_ms * 1e-3) / 1e12
@@ -540,11 +568,10 @@ def run_ours(args):
         prof = profiled_counters()
         traffic = prof.get("dram_bytes_per_step")
         line = dict(
-            metric=METRIC, value=value, unit=UNIT, n_gpus=world, steps=K, warmup=W, ms_per_step=ms_total / (K * R),
+            metric=METRIC, value=value, unit=UNIT, n_gpus=world, steps=K, warmup=W, ms_per_step=ms_total / K,
             higher_is_better=True, scaling=args.scaling, vs_baseline=None, dtype="f64", data="synthetic",
             config=config_dict(args),
-            timed=dict(passes=K * R, repeats_of_the_k_step_sequence=R, seconds=ms_total * 1e-3, min_seconds=args.min_seconds,
-                       problems_per_gpu_per_step=Bl, streams=S, batch_split=split, handover_below=(args.handover if S > 1 and args.handover >= 0 else 1184), solver_handles=len(set(id(m) for m in dev_handles)),
+            timed=dict(passes=K, seconds=ms_total * 1e-3, problems_per_gpu_per_step=Bl, streams=S, batch_split=split, handover_below=(args.handover if S > 1 and args.handover >= 0 else 1184), solver_handles=len(set(id(m) for m in dev_handles)),
                        pipeline_depth=args.pipeline,
                        note="value = problems_per_step x passes / seconds (max over ranks of the CUDA-event time)"),
             e2e=dict(value=e2e_value, unit=UNIT, h2d_bytes_per_step=total_per_step * (6 + ncoef) * 8,
@@ -637,7 +664,6 @@ def main():
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="strong (default, BASELINE configs[3]): one --batch-problem batch per step sharded by index over the GPUs; "
                          "weak: every GPU solves its own --batch problems per step")
-    ap.add_argument("--min-seconds", type=float, default=2.0, help="the timed regions repeat the K-step sequence until they last this long")
     ap.add_argument("--ref-per-core", type=int, default=200, help="--impl reference: solves per host core per step")
     ap.add_argument("--no-multi-leg", action="store_true", help="N > 1: skip the one-process b200mpc_solve_batch_multi leg")
     ap.add_argument("--no-weak-leg", action="store_true", help="N > 1: skip the weak-scaling figure")
@@ -657,7 +683,13 @@ def main():
     ap.add_argument("--pipeline-slots", type=int, default=0, help="problems a tail context holds (0 = max(1024, batch / 16))")
     ap.add_argument("--mode", default="perpass", choices=["perpass", "fused"], help="solver execution mode (include/b200mpc.h)")
     ap.add_argument("--rounds", type=int, default=0, help="per-pass mode: rounds before the fused finisher (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: write the results of the last timed step to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     claim_stdout()
     if args.impl == "reference":

@@ -119,7 +119,7 @@ def main():
     print("golden fixtures written to", HERE)
 
 
-if __name__ == "__main__" and not {"--config3", "--n100", "--resto", "--soft", "--long-filter", "--rare-paths", "--weights", "--frontend"} & set(sys.argv):
+if __name__ == "__main__" and not {"--config3", "--n100", "--resto", "--soft", "--long-filter", "--rare-paths", "--weights", "--frontend", "--loops"} & set(sys.argv):
     main()
 
 
@@ -321,3 +321,45 @@ def long_filter():
 
 if __name__ == "__main__" and ("--long-filter" in sys.argv or "--rare-paths" in sys.argv):
     long_filter()
+
+
+def _solver():
+    """The reference's binaries when they are built (oracle/_ref), else the C restatement of its algorithm
+    (oracle/libmpc_oracle.so), which reproduces the reference's iterates on the fixtures above."""
+    return ("reference", ob.ref_solve) if ob.ref_available() else ("port", ob.port_solve)
+
+
+def loops():
+    """Fixtures of two GPU tests that solve one problem at a time on the CPU and compare:
+      * roadmap_closed_loop_12x8.npz: solution/main.cpp:51-76 for 12 vehicles of roadmap_256.npz (every 20th), 8 steps,
+        each step starting from the state the previous solve predicted;
+      * straggler_set3.npz: the problem with the most interior-point iterations (68) of bench.py's input set 3
+        (synth.SEED + 3000 / 3001, 65 536 roadmap problems), index 31134."""
+    from udacitympc_b200 import synth
+    src, solve = _solver()
+    g = np.load(os.path.join(HERE, "roadmap_256.npz"))
+    sel = np.arange(0, 240, 20)
+    K, J = 8, len(sel)
+    out8 = np.zeros((K, J, 8)); obj = np.zeros((K, J)); st = np.zeros((K, J), dtype=np.int32); it = np.zeros((K, J), dtype=np.int32)
+    for j, b in enumerate(sel):
+        s = g["states"][b].copy()
+        for k in range(K):
+            r = solve(s, g["fit"][b])
+            out8[k, j], obj[k, j], st[k, j], it[k, j] = r["out8"], r["obj"], r["status"], r["iters"]
+            s = r["out8"][:6].copy()
+    # the first step is a problem of roadmap_256.npz: the solver used here must reproduce the reference's result there
+    assert (it[0] == g["iters"][sel]).all() and np.abs(out8[0] - g["out8"][sel]).max() < 1e-9
+    np.savez_compressed(os.path.join(HERE, "roadmap_closed_loop_12x8.npz"), index=sel, out8=out8, obj=obj, status=st, iters=it,
+                        source=np.array(src))
+    B, j = 65536, 31134
+    xs, ys = synth.roadmap_windows(B, synth.MT19937_64(synth.SEED + 3000))
+    fit = ob.port_polyfit(xs[j], ys[j], 3)
+    state = synth.roadmap_problems(B, np.tile(fit, (B, 1)), synth.MT19937_64(synth.SEED + 3001))[j]
+    r = solve(state, fit)
+    np.savez_compressed(os.path.join(HERE, "straggler_set3.npz"), index=j, state=state, coeffs=fit, x=r["x"], out8=r["out8"], obj=r["obj"],
+                        status=r["status"], iters=r["iters"], source=np.array(src))
+    print(src, "loop iterations", it.sum(), "straggler", r["status"], r["iters"])
+
+
+if __name__ == "__main__" and "--loops" in sys.argv:
+    loops()

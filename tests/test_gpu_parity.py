@@ -67,20 +67,21 @@ def test_config1_closed_loop_on_device(mpc):
 
 def test_closed_loop_of_several_vehicles_vs_reference_loop(mpc):
     """solution/main.cpp:51-76 for 12 vehicles with their own degree-3 references, 8 steps, on the device
-    (b200mpc_closed_loop_batch) against the same loop run with the reference binaries, one MPC::Solve at a time."""
+    (b200mpc_closed_loop_batch) against the same loop run on the CPU one MPC::Solve at a time (make_golden.py --loops);
+    its first step is the reference's own result in roadmap_256.npz."""
     g = golden("roadmap_256.npz")
+    loop = golden("roadmap_closed_loop_12x8.npz")
     sel = np.arange(0, 240, 20)
+    assert np.array_equal(loop["index"], sel)
     st, cf = g["states"][sel], g["fit"][sel]
     r = mpc.closed_loop(st, cf, 8)
+    np.testing.assert_allclose(r["hist8"][0], g["out8"][sel], rtol=0, atol=1e-7)
     for j in range(len(sel)):
-        s = st[j].copy()
         for k in range(8):
-            o = ob.ref_solve(s, cf[j])
-            assert o["status"] == 0
-            np.testing.assert_allclose(r["hist8"][k, j], o["out8"], rtol=0, atol=1e-7)
-            assert abs(r["cost"][k, j] - o["obj"]) <= TOL_OBJ * abs(o["obj"])
-            assert r["iters"][k, j] == o["iters"]
-            s = o["out8"][:6].copy()
+            assert loop["status"][k, j] == 0
+            np.testing.assert_allclose(r["hist8"][k, j], loop["out8"][k, j], rtol=0, atol=1e-7)
+            assert abs(r["cost"][k, j] - loop["obj"][k, j]) <= TOL_OBJ * abs(loop["obj"][k, j])
+            assert r["iters"][k, j] == loop["iters"][k, j]
 
 
 def test_warm_started_closed_loop(mpc):
@@ -648,11 +649,14 @@ def test_overlapped_solves_are_deterministic():
         for o in outs[1:]:
             assert torch.equal(o["out8"], outs[0]["out8"]) and torch.equal(o["iters"], outs[0]["iters"])
             assert torch.equal(o["status"], outs[0]["status"])
-        # the straggler against the reference binaries
+        # the straggler against its one-at-a-time CPU solve (make_golden.py --loops)
         j = int(outs[0]["iters"].argmax())
-        r = ob.ref_solve(st[j], fit[j])
+        r = golden("straggler_set3.npz")
+        assert j == r["index"]
+        np.testing.assert_allclose(st[j], r["state"], rtol=0, atol=1e-9)
+        np.testing.assert_allclose(fit[j], r["coeffs"], rtol=0, atol=1e-9)
         got = outs[0]["out8"][:, j].cpu().numpy()
-        print("straggler", j, "iters", int(outs[0]["iters"][j]), "reference iters", r["iters"], "status", r["status"])
+        print("straggler", j, "iters", int(outs[0]["iters"][j]), "CPU iters", r["iters"], "status", r["status"])
         assert r["status"] == 0
         np.testing.assert_allclose(got[6:], [r["x"][6 * 25], r["x"][7 * 25 - 1]], rtol=0, atol=TOL_ACT)
         np.testing.assert_allclose(got[:6], [r["x"][k * 25 + 1] for k in range(6)], rtol=0, atol=TOL_TRAJ)

@@ -216,7 +216,8 @@ def test_warm_started_closed_loop_reaches_the_same_trajectory(hostsim):
 
 def test_invalid_numbers_stop_at_the_starting_point(hostsim):
     """NaN / Inf in the state or the coefficients: the reference's Ipopt returns Invalid_Number_Detected (-13) without an
-    iteration; so do both execution shapes of the solver core."""
+    iteration; so do the C port and both execution shapes of the solver core.  (The reference's binaries, which are
+    not part of the repository, are checked too where they are built.)"""
     import oracle_bindings as ob
     g = golden("line_256.npz")
     cases = []
@@ -224,8 +225,9 @@ def test_invalid_numbers_stop_at_the_starting_point(hostsim):
     st = g["states"][0].copy(); st[3] = np.inf; cases.append((st, g["coeffs"][0]))
     cf = g["coeffs"][0].copy(); cf[0] = np.nan; cases.append((g["states"][0], cf))
     for st, cf in cases:
-        o = ob.ref_solve(st, cf)
-        assert o["status"] == -13 and o["iters"] == 0
+        if ob.ref_available():
+            o = ob.ref_solve(st, cf)
+            assert o["status"] == -13 and o["iters"] == 0
         o = ob.port_solve(st, cf)
         assert o["status"] == -13 and o["iters"] == 0
         for mode in (0, 1, 2):

@@ -12,7 +12,7 @@ python - <<'P'
 import json,glob
 for f in sorted(glob.glob('gpurun_out/r2_bench*.json')):
     try:
-        d=json.load(open(f)); print(f, round(d['value']/1e6,3), 'M/s e2e', round(d['e2e']['value']/1e6,3), 'lone', round(d['lone_caller']['value']/1e6,3), 'p99', round(d['e2e']['p99_batch_latency_ms'],2), 'R', d['timed']['repeats_of_the_k_step_sequence'], 'S', d['timed']['streams'], 'frac', round(d['roofline']['frac'],3))
+        d=json.load(open(f)); print(f, round(d['value']/1e6,3), 'M/s e2e', round(d['e2e']['value']/1e6,3), 'lone', round(d['lone_caller']['value']/1e6,3), 'p99', round(d['e2e']['p99_batch_latency_ms'],2), 'S', d['timed']['streams'], 'frac', round(d['roofline']['frac'],3))
     except Exception as e: print(f, 'ERR', e)
 P
 tail -5 gpurun_out/r2_bench1.err

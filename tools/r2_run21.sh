@@ -9,7 +9,7 @@ import json
 d=json.load(open('gpurun_out/r2_bench21.json'))
 print(round(d['value']/1e6,3),'M/s e2e',round(d['e2e']['value']/1e6,3),'lone',round(d['lone_caller']['value']/1e6,3),'p50',round(d['e2e']['p50_batch_latency_ms'],2),'p99',round(d['e2e']['p99_batch_latency_ms'],2),'cpu',d['cpu_baseline']['value'], d['cpu_baseline']['cores'])
 P
-CMD="python bench.py --steps 2 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --min-seconds 0 --latency-reps 1"
+CMD="python bench.py --steps 2 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --latency-reps 1"
 $CMD > gpurun_out/r2_final_plain.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum,smsp__sass_thread_inst_executed_op_dfma_pred_on.sum,smsp__sass_thread_inst_executed_op_dadd_pred_on.sum,smsp__sass_thread_inst_executed_op_dmul_pred_on.sum,smsp__inst_executed.sum --clock-control none -k regex:mpc_ -c 200 --csv --log-file gpurun_out/r2_final_launches_counters.csv $CMD > gpurun_out/r2_final_ncu.log 2>&1
 echo "ncu list rc=$?"

@@ -3,7 +3,7 @@
 # round 2, GPU call 26: ncu launch list (durations, DRAM bytes, instructions) of one solve with the fused step + factor
 # sweep (B200MPC_FUSE=1) and with the separate kernels (B200MPC_FUSE=0)
 mkdir -p gpurun_out
-CMD="python bench.py --steps 1 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --min-seconds 0 --latency-reps 1"
+CMD="python bench.py --steps 1 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --latency-reps 1"
 for f in 1 0; do
 B200MPC_FUSE=$f ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum,smsp__inst_executed.sum --clock-control none -k regex:mpc_ -c 120 --csv --log-file gpurun_out/r2_fuse${f}_launches.csv $CMD > gpurun_out/r2_fuse${f}_ncu.log 2>&1
 echo "ncu fuse=$f rc=$?"

@@ -16,7 +16,7 @@ python bench.py --streams $s --no-cpu-baseline --no-sweep --latency-reps 5 > gpu
 python -c "
 import json; d=json.load(open('gpurun_out/r2_bench27_s$s.json')); print('streams $s:', round(d['value']/1e6,3), 'M/s e2e', round(d['e2e']['value']/1e6,3))"
 done
-CMD="python bench.py --steps 2 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --min-seconds 0 --latency-reps 1"
+CMD="python bench.py --steps 2 --warmup 3 --streams 1 --split 1 --no-cpu-baseline --no-sweep --latency-reps 1"
 $CMD > gpurun_out/r2_final27_plain.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum,smsp__sass_thread_inst_executed_op_dfma_pred_on.sum,smsp__sass_thread_inst_executed_op_dadd_pred_on.sum,smsp__sass_thread_inst_executed_op_dmul_pred_on.sum,smsp__inst_executed.sum --clock-control none -k regex:mpc_ -c 200 --csv --log-file gpurun_out/r2_final27_launches_counters.csv $CMD > gpurun_out/r2_final27_ncu.log 2>&1
 echo "ncu list rc=$?"
