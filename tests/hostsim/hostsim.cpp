@@ -32,25 +32,7 @@ struct HostExec {   // the cooperative solver's primitives on one CPU thread: la
   }
 };
 
-static long long g_factor_calls = 0;   // kernel_factor calls of the per-pass emulations (how often the fused STEP pass saved one)
-static int g_fuse = 0;    // per-pass emulation: the STEP pass is Solver::kernel_stepfactor (what mpc_stepfactor_kernel runs)
-template <class S_>
-static void step_pass_of(S_& S) {
-#if MPC_FUSE_FACTOR
-  if (g_fuse) {
-    double rcarry[kRicCarry];
-    S.rq = rcarry; S.rqs = 1;
-    S.kernel_stepfactor();
-    return;
-  }
-#endif
-  S.kernel_step();
-}
-
 extern "C" {
-void hostsim_set_fuse(int on) { g_fuse = on; }
-long long hostsim_factor_calls() { return g_factor_calls; }
-
 struct hostsim_params {
   int N;
   double dt, Lf, ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da, delta_max, a_max, tol;
@@ -139,9 +121,9 @@ int hostsim_solve_mode(const hostsim_params* hp, const double* state6, const dou
         S.cr = carry; S.cs = 1;
         if (S.load_phase() != k) continue;
         S.set_coeffs(coeffs, ncoef);
-        if (k == PH_FACTOR) { S.kernel_factor(); ++g_factor_calls; }
+        if (k == PH_FACTOR) S.kernel_factor();
         else if (k == PH_FORWARD) S.kernel_forward();
-        else step_pass_of(S);
+        else S.kernel_step();
         phase = S.load_phase();
         if (k == PH_STEP) { S.load_state(); log_row(S); }
         if (mode == -2 && phase != PH_DONE) repack();
@@ -261,9 +243,9 @@ int hostsim_batch_interleaved(const hostsim_params* hp, int B, const double* sta
         S.cr = carry; S.cs = 1;
         if (S.load_phase() != k) continue;
         S.set_coeffs(coeffs + (size_t)ncoef * b, ncoef);
-        if (k == PH_FACTOR) { S.kernel_factor(); ++g_factor_calls; }
+        if (k == PH_FACTOR) S.kernel_factor();
         else if (k == PH_FORWARD) S.kernel_forward();
-        else step_pass_of(S);
+        else S.kernel_step();
       }
       Solver<32> S(P, base(cur, slot), slot & 31);
       if (S.load_phase() == PH_RESTO || (max_rounds > 0 && round + 1 >= max_rounds && S.load_phase() != PH_DONE)) {   // finisher

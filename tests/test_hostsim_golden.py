@@ -310,68 +310,3 @@ def test_filter_reset_heuristic_and_soft_step_after_a_failed_soc(hostsim):
             np.testing.assert_allclose(r["x"], g["x"][b], rtol=0, atol=1e-7)
         o = ob.port_solve(g["states"][b], g["coeffs"][b])
         assert o["status"] == 0 and o["iters"] == g["iters"][b]
-
-
-def test_step_sweep_with_the_next_factorisation_riding_on_it(hostsim_fuse):
-    """Solver::kernel_stepfactor (mpc_stepfactor_kernel): the Riccati factorisation of the next iteration's system rides on
-    the STEP sweep, with the feed-forward split as ka + mu kb.  Against the plain loop (mode 0) on the per-pass
-    emulation (fresh Solver per pass, modes 1 / -1 / -2 = also moved into a NaN-poisoned workspace after every round /
-    pass): same status and iteration count on every problem -- including regularisation, backtracking, second-order
-    correction, long filters and the restoration cases -- and the same solution up to the rounding of the split (1e-10);
-    and the factor pass really is skipped (two per solve remain: multiplier initialisation and first iteration).
-    MPC_FUSE_FACTOR is an experiment the product is built without (13 % slower on the B200, mpc_core.cuh); this test and
-    the next keep it compiling and correct."""
-    import ctypes
-    hostsim = hostsim_fuse
-    lib = hostsim.lib
-    lib.hostsim_factor_calls.restype = ctypes.c_longlong
-    sets = [("line_256.npz", {}, range(0, 256, 8)), ("roadmap_256.npz", {}, range(0, 256, 8)), ("roadmap_N50_64.npz", dict(N=50), range(0, 64, 2))]
-    g = golden("line_params_64.npz")
-    N, dt, Lf, ref_v, dmax, amax = g["params"]
-    sets.append(("line_params_64.npz", dict(N=int(N), dt=dt, Lf=Lf, ref_v=ref_v, delta_max=dmax, a_max=amax), range(0, 64, 2)))
-    sets.append(("line_256.npz", dict(ref_v=6.0), range(0, 6)))
-    sets.append(("long_filter_N25_12.npz", {}, range(12)))
-    sets.append(("resto_N25_wild_32.npz", {}, range(0, 32, 2)))
-    try:
-        for name, kw, idx in sets:
-            g = golden(name)
-            cf = g["coeffs"] if "coeffs" in g.files else g["fit"]
-            for b in idx:
-                lib.hostsim_set_fuse(0)
-                a = hostsim.solve(g["states"][b], cf[b], mode=0, **kw)
-                lib.hostsim_set_fuse(1)
-                for mode in (1, -1, -2):
-                    c = hostsim.solve(g["states"][b], cf[b], mode=mode, **kw)
-                    assert a["status"] == c["status"] and a["iters"] == c["iters"], (name, b, mode)
-                    np.testing.assert_allclose(c["x"], a["x"], rtol=0, atol=1e-10)
-        g = golden("roadmap_256.npz")
-        calls = {}
-        for fuse in (0, 1):
-            lib.hostsim_set_fuse(fuse)
-            c0 = lib.hostsim_factor_calls()
-            iters = sum(hostsim.solve(g["states"][b], g["fit"][b], mode=1)["iters"] for b in range(16))
-            calls[fuse] = lib.hostsim_factor_calls() - c0
-        assert calls[0] >= iters + 16 and calls[1] == 2 * 16, calls
-    finally:
-        lib.hostsim_set_fuse(0)
-
-
-def test_device_memory_layout_on_the_host_with_the_fused_step(hostsim_fuse):
-    """The device layout emulation (warp-interleaved groups, two regions, compaction into a poisoned region, guard words)
-    with kernel_stepfactor as the STEP pass: problems are moved while they wait for their FORWARD sweep, owning the
-    current iterate and the Riccati factors only (repack_problem)."""
-    hostsim = hostsim_fuse
-    a, b, c = golden("long_filter_N25_12.npz"), golden("resto_N25_wild_32.npz"), golden("roadmap_256.npz")
-    st = np.concatenate([a["states"], b["states"], c["states"][:26]])
-    cf = np.concatenate([a["coeffs"], b["coeffs"], c["fit"][:26]])
-    try:
-        hostsim.lib.hostsim_set_fuse(1)
-        r = hostsim.batch_interleaved(st, cf, compact=True)
-    finally:
-        hostsim.lib.hostsim_set_fuse(0)
-    assert r["rc"] == 0, "a write landed outside a workspace region"
-    for k in range(len(st)):
-        one = hostsim.solve(st[k], cf[k])
-        assert r["status"][k] == one["status"] == 0 and r["iters"][k] == one["iters"]
-        np.testing.assert_allclose(r["out8"][k], one["out8"], rtol=0, atol=1e-10)
-

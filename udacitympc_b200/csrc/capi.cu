@@ -328,7 +328,6 @@ int b200mpc_create(const b200mpc_params* p, int device, b200mpc_handle** out) {
   h->device = device;
   if (const char* e = getenv("B200MPC_NO_GRAPHS")) h->use_graphs = !(e[0] == '1');
   if (const char* e = getenv("B200MPC_NO_COOP")) h->cfg.coop = !(e[0] == '1');
-  if (const char* e = getenv("B200MPC_FUSE")) h->cfg.fuse_factor = (e[0] == '1');   // experiment (builds with -DMPC_FUSE_FACTOR=1 only): step + next factor in one sweep
   if (const char* e = getenv("B200MPC_RESTORATION")) { int v = atoi(e); if (v >= 0 && v <= 2) h->P.resto = v; }
   h->resto_mode = h->P.resto;
   e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);

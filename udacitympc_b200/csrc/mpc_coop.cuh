@@ -100,7 +100,7 @@ struct CoopSolver {
     const double gv2 = 2.0 * P.w_v * df, ge2 = 2.0 * P.w_epsi * df, gc2 = 2.0 * P.w_cte * df;
     const int r = S.rec(t) + kX * pub->cur;
     double sp, cp, se, ce, p0, p1, p2, p3;
-    S.trig_of(r, c.s, sp, cp, se, ce);
+    S.trig_of(r, sp, cp, se, ce);
     c.tr[0] = sp; c.tr[1] = cp; c.tr[2] = se; c.tr[3] = ce;
     poly_eval(S.cf, c.s[0], p0, p1, p2, p3);
     const Lin A = make_lin(P, c.s[3], c.u[0], sp, cp, se, ce, p1, p2);
@@ -373,9 +373,7 @@ struct CoopSolver {
         sincos(c.sn[2], &spn, &cpn);
         sincos(c.sn[5], &sen, &cen);
         c.trn[0] = spn; c.trn[1] = cpn; c.trn[2] = sen; c.trn[3] = cen;
-#if MPC_STORE_TRIG
         S.w(rN + xTR) = spn; S.w(rN + xTR + 1) = cpn; S.w(rN + xTR + 2) = sen; S.w(rN + xTR + 3) = cen;
-#endif
       }
       // offset of lambda^+_t = A_t^T lambda^+_{t+1} + bl_t (current linearisation, staged by prep_factor)
       c.bl[0] = -(q0 + c.H[0]) * ds[0];
@@ -418,13 +416,7 @@ struct CoopSolver {
       poly_eval(S.cf, c.sn[0], p0, p1, p2, p3);
       const double psides = atan(p1);
       S.residual(c.sn, c.un, st[t + 1].sn, c.trn[0], c.trn[1], c.trn[2], p0, psides, cres);
-      S.store_psides(rN, psides);   // the thread-per-problem sweeps read it (MPC_STORE_PSIDES)
-      for (int k = 0; k < 6; ++k) {
-#if MPC_STORE_C
-        S.w(S.rec(t + 1) + kX * (pub->cur ^ 1) + xC + k) = cres[k];
-#endif
-        th += fabs(cres[k]); cm = dmax(cm, fabs(cres[k]));
-      }
+      for (int k = 0; k < 6; ++k) { th += fabs(cres[k]); cm = dmax(cm, fabs(cres[k])); }
       f += P.w_delta * (c.un[0] * c.un[0]) + P.w_a * (c.un[1] * c.un[1]);
       if (t > 0) {
         const double e0 = c.un[0] - st[t - 1].un[0], e1 = c.un[1] - st[t - 1].un[1];

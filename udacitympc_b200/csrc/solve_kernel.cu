@@ -6,8 +6,8 @@
 // workspace (each workspace access of a warp is one coalesced 256-byte row) and the 7x7 Riccati blocks live in
 // registers.  One interior-point iteration = three sweeps over the horizon, each its own kernel
 //   init | factor | forward | step        launched round after round on one stream (replayed as one CUDA graph),
-// with its own register budget (the Riccati factorisation needs ~250 registers, the step sweep 228 with its
-// stage-to-stage values in shared memory, the forward sweep 168) and a small instruction footprint.
+// with its own register budget (the Riccati factorisation needs ~250 registers, the step sweep ~240 with its
+// stage-to-stage values in registers, the forward sweep 168) and a small instruction footprint.
 // Between rounds mpc_repack_kernel compacts the problems that are still iterating into consecutive workspace slots
 // (second workspace region, slot -> problem map, level state in device memory), so late rounds run full warps.
 // Latency path (mpc_coop.cuh): one problem per warp, lane <-> stage.  mpc_coop_kernel finishes whatever is still
@@ -37,14 +37,6 @@ constexpr int kBlock = MPC_BLOCK;
 #ifndef MPC_FACTOR_BLOCKS
 #define MPC_FACTOR_BLOCKS 4
 #endif
-// stage-to-stage values of the step sweep: in registers (250 registers, nothing spilled, no shared memory; 0.6-0.8 % faster
-// than the shared-memory carry at 4 blocks per SM, gpurun_out/r2_creg_*.json, r2_psd_*.json) or in shared memory
-#ifndef MPC_STEP_CARRY_SMEM
-#define MPC_STEP_CARRY_SMEM 0
-#endif
-#ifndef MPC_STEPFACTOR_BLOCKS
-#define MPC_STEPFACTOR_BLOCKS 4
-#endif
 constexpr int kFwdBlocks = MPC_FWD_BLOCKS, kStepBlocks = MPC_STEP_BLOCKS, kFactorBlocks = MPC_FACTOR_BLOCKS;
 
 // One workspace region holds every problem of a batch; the buffer the handle allocates has two of them (the batch
@@ -58,6 +50,20 @@ static size_t region_doubles(int N, int B) {
 }
 static size_t aux_doubles(int B) { return ((size_t)B + 1) / 2 * 2 + kMaxParts * kDescInts; }   // 2 int maps + state
 size_t solve_workspace_doubles(int N, int B) { return 2 * region_doubles(N, B) + aux_doubles(B); }
+// the parts of a buffer of solve_workspace_doubles(N, B) doubles: region 0 | region 1 | map 0 | map 1 | compaction state
+struct WsLayout {
+  double* ws0;
+  double* ws1;
+  int* map0;
+  int* map1;
+  int* desc;
+};
+static WsLayout ws_layout(double* ws, int N, int B) {
+  const size_t reg = region_doubles(N, B);
+  int* ints = reinterpret_cast<int*>(ws + 2 * reg);
+  const size_t map_ints = ((size_t)B + 1) / 2 * 2;
+  return WsLayout{ws, ws + reg, ints, ints + map_ints, ints + 2 * map_ints};
+}
 
 struct SolveArgs {
   int B, steps, step, ncoef;
@@ -155,10 +161,8 @@ __global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
   Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
   if (S.load_phase() != PH_FACTOR) return;
-#if MPC_ASYNC_STAGE
   __shared__ double stage[2 * kStageVals * kBlock];   // [buffer][value][thread]
   S.sb = stage + threadIdx.x; S.sbs = kBlock;
-#endif
   load_coeffs(A, b, S.cf);
   S.kernel_factor();
   if (S.phase == PH_DONE) {   // inertia correction exhausted (IpPDPerturbationHandler.cpp:380-388)
@@ -187,53 +191,14 @@ __global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __g
     if (A.count_live && ph != PH_DONE) count_live(A.desc + kLive);
     return;
   }
-#if MPC_STEP_CARRY_SMEM
-  __shared__ double carry[kCarry * kBlock];   // stage-to-stage values of the sweep, [value][thread]
-  S.cr = carry + threadIdx.x; S.cs = kBlock;
-#else
   double carry[kCarry];
   S.cr = carry; S.cs = 1;
-#endif
-#if MPC_ASYNC_STAGE && MPC_STEP_ASYNC_STAGE
   __shared__ double stage[2 * kStepStageVals * kBlock];   // [buffer][value][thread]
   S.sb = stage + threadIdx.x; S.sbs = kBlock;
-#endif
   load_coeffs(A, b, S.cf);
   S.kernel_step();
   if (S.phase == PH_DONE) write_result(P, A, b, S);
   else if (A.count_live) count_live(A.desc + kLive);
-}
-
-#if MPC_FUSE_FACTOR
-// STEP sweep with the Riccati factorisation of the next iteration riding on it (Solver::kernel_stepfactor): the trial
-// iterate is factorised from the registers that have just produced it, so an accepted step is followed by the forward
-// sweep directly and the factor kernel only sees the rare cases (first iteration, rejected trial points, second-order
-// corrections, inertia corrections).  Both carry sets (24 + 39 doubles per thread) live in shared memory.
-__global__ void __launch_bounds__(kBlock, MPC_STEPFACTOR_BLOCKS) mpc_stepfactor_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
-  int slot, b;
-  double* ws;
-  if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
-  Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
-  const int ph = S.load_phase();
-  if (ph != PH_STEP) {
-    if (A.count_live && ph != PH_DONE) count_live(A.desc + kLive);
-    return;
-  }
-  __shared__ double carry[(kCarry + kRicCarry) * kBlock];   // [value][thread]
-  S.cr = carry + threadIdx.x; S.cs = kBlock;
-  S.rq = carry + kCarry * kBlock + threadIdx.x; S.rqs = kBlock;
-  load_coeffs(A, b, S.cf);
-  S.kernel_stepfactor();
-  if (S.phase == PH_DONE) write_result(P, A, b, S);
-  else if (A.count_live) count_live(A.desc + kLive);
-}
-#endif
-static void launch_step(const Params& P, const SolveArgs& A, const SolveConfig& cfg, int grid, cudaStream_t stream) {
-#if MPC_FUSE_FACTOR
-  if (cfg.fuse_factor) { mpc_stepfactor_kernel<<<grid, kBlock, 0, stream>>>(P, A); return; }
-#endif
-  (void)cfg;
-  mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, A);
 }
 
 // ---- batch compaction ------------------------------------------------------------------------------------------
@@ -373,20 +338,33 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
   }
 }
 
-// per-device, once (b200mpc_create): the cooperative kernel uses up to 200 KB of dynamic shared memory per block
+constexpr size_t kCoopSmemMax = 200 * 1024;   // dynamic shared memory of one cooperative block, at most
+// per-device, once (b200mpc_create)
 cudaError_t solver_prepare_device() {
-  return cudaFuncSetAttribute(mpc_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  return cudaFuncSetAttribute(mpc_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
 }
 
 static size_t coop_doubles_per_warp(int N) { return (size_t)N * kCoopStageDoubles + (sizeof(CoopPub) + 7) / 8; }
-// warps of the cooperative kernel that are resident on the device at once (0: the horizon does not fit): 128-thread blocks
-// of up to 4 problems, 2 blocks per SM by registers, per-problem scratch in shared memory
-static int coop_resident_warps(int N) {
-  const size_t per_warp = coop_doubles_per_warp(N) * sizeof(double), limit = 200 * 1024;
-  if (per_warp > limit) return 0;
-  int wpb = (int)(limit / per_warp);
+// block of the cooperative kernel at horizon N: up to 4 problems (warps), per-problem scratch in shared memory;
+// warps = 0: the horizon does not fit
+struct CoopShape {
+  int warps;
+  size_t smem;
+};
+static CoopShape coop_shape(int N) {
+  const size_t per_warp = coop_doubles_per_warp(N) * sizeof(double);
+  if (per_warp > kCoopSmemMax) return CoopShape{0, 0};
+  int wpb = (int)(kCoopSmemMax / per_warp);
   if (wpb > 4) wpb = 4;
-  int blocks = (int)((size_t)227 * 1024 / (per_warp * wpb));
+  return CoopShape{wpb, per_warp * wpb};
+}
+// warps of the cooperative kernel that are resident on the device at once (0: the horizon does not fit), 2 blocks per SM
+// by registers
+static int coop_resident_warps(int N) {
+  const CoopShape c = coop_shape(N);
+  if (c.warps == 0) return 0;
+  const int wpb = c.warps;
+  int blocks = (int)((size_t)227 * 1024 / c.smem);
   if (blocks > 2) blocks = 2;
   int sms = 148;
   int dev = 0;
@@ -396,19 +374,25 @@ static int coop_resident_warps(int N) {
 
 // launches the cooperative kernel if the horizon fits in shared memory; returns false otherwise
 static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, cudaStream_t stream, cudaError_t* err, int take_below = 0) {
-  const size_t per_warp = coop_doubles_per_warp(P.N) * sizeof(double);
-  const size_t limit = 200 * 1024;
-  if (per_warp > limit) return false;
-  int wpb = (int)(limit / per_warp);
-  if (wpb > 4) wpb = 4;
-  const size_t smem = per_warp * wpb;
+  const CoopShape c = coop_shape(P.N);
+  if (c.warps == 0) return false;
+  const int wpb = c.warps;
   const int n = take_below > 0 && take_below < A.b1 - A.b0 ? take_below : A.b1 - A.b0;
   int grid = (n + wpb - 1) / wpb;
   const int cap = 4 * coop_resident_warps(P.N) / wpb;   // four waves; the warps stride over the rest
   if (cap > 0 && grid > cap) grid = cap;
-  mpc_coop_kernel<<<grid, 32 * wpb, smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);   // no idle warps: their registers would stay allocated
+  mpc_coop_kernel<<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);   // no idle warps: their registers would stay allocated
   *err = cudaGetLastError();
   return true;
+}
+
+// rounds of the thread-per-problem sweeps after which the cooperative kernel takes every remaining problem over.
+// Longer horizons have a longer tail of iteration counts (N = 100: 3.6 % of the problems need more than 20, 1.8 % more
+// than 100) and a slower cooperative kernel (0.34 ms per problem and iteration at N = 100, 2 warps per SM), so the sweeps
+// keep the tail longer there: measured with 4 overlapped batches of 65 536 problems at N = 100, 20 rounds 267 ms per
+// batch, 120 rounds 225 ms; N <= 50 does not gain (profiles/r1_handover_sweep_long_horizons.log).
+static int handover_rounds(const Params& P, const SolveConfig& cfg) {
+  return cfg.handover_max_rounds > 0 ? cfg.handover_max_rounds : (P.N <= 50 ? 20 : 2 * P.N - 80);
 }
 
 // launches every kernel of the solve of problems [b0, b1) on one stream
@@ -432,7 +416,7 @@ static cudaError_t launch_part(const Params& P, SolveArgs A, const SolveConfig& 
         Ar.count_live = attempt ? 1 : 0;
         mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
         mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-        launch_step(P, Ar, cfg, grid, stream);
+        mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
         if (attempt) {
           mpc_repack_kernel<<<(nb + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, 0, nullptr, nullptr, nullptr);
           *n += 1;
@@ -460,28 +444,19 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6
                          double* ws, double* out8, double* traj, double* obj, int* status, int* iters,
                          const SolveConfig& cfg, cudaStream_t stream, const SplitStreams* ss, long long* n_launches, int io_aos) {
   if (B <= 0) return cudaSuccess;
-  // buffer layout: region 0 | region 1 | map 0 | map 1 | compaction state of every part
-  const size_t reg = region_doubles(P.N, B);
-  int* ints = reinterpret_cast<int*>(ws + 2 * reg);
-  const size_t map_ints = ((size_t)B + 1) / 2 * 2;
-  int* desc = ints + 2 * map_ints;
+  const WsLayout L = ws_layout(ws, P.N, B);   // the compaction state holds one record per part
   // a warm-started step reads the previous solution at the problem's own slot: no compaction then
-  if (!(cfg.compact_max_live > 0.0) || cfg.warm_start) desc = nullptr;
-  SolveArgs A{B, steps, 0, ncoef, io_aos ? 1 : 0, 0, B, cfg.warm_start ? 1 : 0, cfg.warm_mu, state6, coeffs, ws, ws + reg, ints, ints + map_ints, desc, 0,
+  int* desc = (!(cfg.compact_max_live > 0.0) || cfg.warm_start) ? nullptr : L.desc;
+  SolveArgs A{B, steps, 0, ncoef, io_aos ? 1 : 0, 0, B, cfg.warm_start ? 1 : 0, cfg.warm_mu, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, desc, 0,
               out8, traj, obj, status, iters};
   long long n = 0;
   int parts = 1;
   if (ss && cfg.mode == kModePerPass && cfg.split > 1 && B >= cfg.split * cfg.fused_below) parts = cfg.split < ss->n_aux + 1 ? cfg.split : ss->n_aux + 1;
-  // automatic setting: up to handover_max_rounds rounds, and after every late round the cooperative kernel takes the
+  // automatic setting: up to handover_rounds() rounds, and after every late round the cooperative kernel takes the
   // rest over as soon as the compacted batch fits its two waves (the launches after that find nothing to do); a fixed
   // number of rounds (b200mpc_set_solver_mode) hands over exactly there
   const bool adaptive = cfg.rounds <= 0 && desc != nullptr && cfg.coop && cfg.handover_below > 0;
-  // Longer horizons have a longer tail of iteration counts (N = 100: 3.6 % of the problems need more than 20, 1.8 % more
-  // than 100) and a slower cooperative kernel (0.34 ms per problem and iteration at N = 100, 2 warps per SM), so the sweeps
-  // keep the tail longer there: measured with 4 overlapped batches of 65 536 problems at N = 100, 20 rounds 267 ms per
-  // batch, 120 rounds 225 ms; N <= 50 does not gain (profiles/r1_handover_sweep_long_horizons.log).
-  const int max_rounds = cfg.handover_max_rounds > 0 ? cfg.handover_max_rounds : (P.N <= 50 ? 20 : 2 * P.N - 80);
-  const int rounds = cfg.rounds > 0 ? cfg.rounds : (adaptive ? max_rounds : (parts > 1 ? 16 : 18));
+  const int rounds = cfg.rounds > 0 ? cfg.rounds : (adaptive ? handover_rounds(P, cfg) : (parts > 1 ? 16 : 18));
   const int take_below = adaptive ? (cfg.handover_below / parts > 64 ? cfg.handover_below / parts : 64) : 0;
   cudaError_t e = cudaSuccess;
   if (parts == 1) {
@@ -520,28 +495,21 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6
 // problem is finished.
 static SolveArgs tail_args(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* out8, double* traj,
                            double* obj, int* status, int* iters, int io_aos, const TailCtx& tail) {
-  const size_t reg = region_doubles(P.N, tail.slots);
-  int* ints = reinterpret_cast<int*>(tail.ws + 2 * reg);
-  const size_t map_ints = ((size_t)tail.slots + 1) / 2 * 2;
-  return SolveArgs{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, tail.slots, 0, 0.0, state6, coeffs, tail.ws, tail.ws + reg, ints, ints + map_ints,
-                   ints + 2 * map_ints, 0, out8, traj, obj, status, iters};
-}
-static int auto_rounds(const Params& P, const SolveConfig& cfg) {
-  return cfg.rounds > 0 ? cfg.rounds : (cfg.handover_max_rounds > 0 ? cfg.handover_max_rounds : (P.N <= 50 ? 20 : 2 * P.N - 80));
+  const WsLayout L = ws_layout(tail.ws, P.N, tail.slots);
+  return SolveArgs{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, tail.slots, 0, 0.0, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, L.desc, 0,
+                   out8, traj, obj, status, iters};
 }
 
 cudaError_t launch_solve_bulk(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* ws, double* out8,
                               double* traj, double* obj, int* status, int* iters, const SolveConfig& cfg, cudaStream_t stream,
                               long long* n_launches, int io_aos, const TailCtx& tail) {
   if (B <= 0) return cudaSuccess;
-  const size_t reg = region_doubles(P.N, B);
-  int* ints = reinterpret_cast<int*>(ws + 2 * reg);
-  const size_t map_ints = ((size_t)B + 1) / 2 * 2;
-  SolveArgs A{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, B, 0, 0.0, state6, coeffs, ws, ws + reg, ints, ints + map_ints, ints + 2 * map_ints, 0,
+  const WsLayout L = ws_layout(ws, P.N, B);
+  SolveArgs A{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, B, 0, 0.0, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, L.desc, 0,
               out8, traj, obj, status, iters};
   const SolveArgs T = tail_args(P, B, state6, coeffs, ncoef, out8, traj, obj, status, iters, io_aos, tail);
   const int grid = (B + kBlock - 1) / kBlock;
-  const int rounds = auto_rounds(P, cfg);
+  const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P, cfg);
   long long n = 0;
   mpc_tail_reset_kernel<<<1, 32, 0, stream>>>(T.desc);
   mpc_init_kernel<<<grid, kBlock, 0, stream>>>(P, A);
@@ -552,7 +520,7 @@ cudaError_t launch_solve_bulk(const Params& P, int B, const double* state6, cons
     Ar.count_live = attempt ? 1 : 0;
     mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
     mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    launch_step(P, Ar, cfg, grid, stream);
+    mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
     n += 3;
     if (attempt) {
       mpc_repack_kernel<<<(B + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, tail.slots, T.ws1, T.map0, T.desc);
@@ -601,7 +569,7 @@ cudaError_t launch_solve_tail(const Params& P, int B, const double* state6, cons
     Ar.count_live = 1;
     mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
     mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    launch_step(P, Ar, cfg, grid, stream);
+    mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
     mpc_repack_kernel<<<(nb + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, 0, nullptr, nullptr, nullptr);
     n += 4;
     if (take_below > 0 && (r + 1) % coop_every == 0 && launch_coop(P, A, 0, stream, &ce, take_below)) {
