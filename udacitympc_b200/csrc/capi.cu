@@ -62,17 +62,21 @@ struct b200mpc_handle {
   b200mpc_params user_params;
   long long launches = 0;
   // CUDA graphs of whole solves (init + rounds x (factor, forward, step) + finisher), keyed by every launch argument
+  struct GraphKey {
+    int phase = 0, B = 0, steps = 0;   // phase: 0 whole solve, 1 bulk, 2 tail
+    SolveIO io;
+    const void *ws = nullptr, *tail = nullptr;   // the handle's workspace, the tail context of a pipelined solve
+    int config_gen = 0;
+  };
   struct GraphEntry {
-    int B, steps, ncoef, mode, rounds, fused_below, warm, split, repack_gen, io_aos, phase;   // phase: 0 whole solve, 1 bulk, 2 tail
-    const void* tail;
-    double warm_mu;
-    const void *st, *cf, *ws, *out8, *traj, *obj, *status, *iters;
+    GraphKey key;
     cudaGraphExec_t exec;
     long long n_kernels;
   };
   std::vector<GraphEntry> graphs;
   bool use_graphs = true;
-  int repack_gen = 0;   // bumped when the compaction schedule changes (part of the graph key)
+  // bumped by every setter that changes what a solve launches or the arguments it bakes in (part of the graph key)
+  int config_gen = 0;
   // pipelined solves (b200mpc_set_pipeline): tail contexts, used round robin, and the events that order the calls
   static constexpr int kMaxPipe = 32;
   int pipe_depth = 0, pipe_slots = 0;
@@ -112,16 +116,54 @@ int check_solve_args(const b200mpc_handle* h, int B, const void* st, const void*
   return 0;
 }
 
-int run_solve(b200mpc_handle* h, int B, int steps, const double* st, const double* cf, int ncoef, double* out8,
-              double* traj, double* obj, int* status, int* iters, cudaStream_t s, bool caller_captures, int io_aos,
-              int phase = 0, TailCtx tail = TailCtx());
+bool same_key(const b200mpc_handle::GraphKey& a, const b200mpc_handle::GraphKey& b) {
+  return a.phase == b.phase && a.B == b.B && a.steps == b.steps && a.io.state6 == b.io.state6 && a.io.coeffs == b.io.coeffs &&
+         a.io.ncoef == b.io.ncoef && a.io.out8 == b.io.out8 && a.io.traj == b.io.traj && a.io.obj == b.io.obj &&
+         a.io.status == b.io.status && a.io.iters == b.io.iters && a.io.io_aos == b.io.io_aos && a.ws == b.ws &&
+         a.tail == b.tail && a.config_gen == b.config_gen;
+}
+
+// One launch sequence (a whole solve, or one half of a pipelined one) on stream s.  One solve is ~85 dependent
+// launches; replaying a captured graph keeps the host out of the inner loop (several ranks / streams per host otherwise
+// become launch-bound).  The legacy default stream cannot be captured.
+int run_solve(b200mpc_handle* h, const b200mpc_handle::GraphKey& key, cudaStream_t s, bool caller_captures,
+              const std::function<cudaError_t(long long*)>& launch) {
+  if (h->use_graphs && !caller_captures && s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread) {
+    b200mpc_handle::GraphEntry* hit = nullptr;
+    for (auto& g : h->graphs)
+      if (same_key(g.key, key)) hit = &g;
+    if (!hit) {
+      cudaGraph_t graph = nullptr;
+      long long n = 0;
+      if (cudaStreamBeginCapture(s, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
+        cudaError_t le = launch(&n);
+        cudaError_t ce = cudaStreamEndCapture(s, &graph);
+        if (le == cudaSuccess && ce == cudaSuccess && graph) {
+          cudaGraphExec_t exec = nullptr;
+          if (cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
+            if (h->graphs.size() >= 96) { cudaGraphExecDestroy(h->graphs.front().exec); h->graphs.erase(h->graphs.begin()); }
+            h->graphs.push_back(b200mpc_handle::GraphEntry{key, exec, n});
+            hit = &h->graphs.back();
+          }
+        }
+        if (graph) cudaGraphDestroy(graph);
+      }
+      cudaGetLastError();   // a failed capture falls back to plain launches below
+    }
+    if (hit) {
+      CU(cudaGraphLaunch(hit->exec, s));
+      h->launches += hit->n_kernels;
+      return 0;
+    }
+  }
+  CU(launch(&h->launches));
+  return 0;
+}
 
 // One solve on stream s.  The handle owns ONE workspace and one set of auxiliary streams, so solves on a handle are
 // serialised on the device whatever streams the caller uses (an event recorded after each solve, waited for by the
 // next).  With b200mpc_set_timing a pair of events brackets the solver kernels for bench.py.
-// io_aos = 1: st / cf / out8 are in the reference's per-problem order (host entry points); traj stays field-major.
-int timed_solve(b200mpc_handle* h, int B, int steps, const double* st, const double* cf, int ncoef, double* out8,
-                double* traj, double* obj, int* status, int* iters, cudaStream_t s, int io_aos = 0) {
+int timed_solve(b200mpc_handle* h, int B, int steps, const SolveIO& io, cudaStream_t s) {
   // the caller may be capturing its stream into a graph of its own: then no nested capture, no external events
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   if (s != nullptr && s != cudaStreamLegacy) { if (cudaStreamIsCapturing(s, &cap) != cudaSuccess) { cudaGetLastError(); cap = cudaStreamCaptureStatusNone; } }
@@ -140,6 +182,8 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const double* st, const dou
     if (h->ws.cap < solve_workspace_doubles(h->P.N, B) * sizeof(double) && h->pipe_calls) CU(cudaDeviceSynchronize());
   }
   CU(h->ws.ensure(solve_workspace_doubles(h->P.N, B) * sizeof(double)));
+  b200mpc_handle::GraphKey key;   // what a graph of this call's launches bakes in
+  key.B = B; key.steps = steps; key.io = io; key.ws = h->ws.p; key.config_gen = h->config_gen;
   if (pipelined) {
     const size_t ctx = solve_workspace_doubles(h->P.N, h->pipe_slots);
     if (h->tail_ctx_N != h->P.N || h->tail_ctx_slots != h->pipe_slots || h->tail_ws.cap < ctx * h->pipe_depth * sizeof(double)) {
@@ -154,14 +198,16 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const double* st, const dou
     if (h->done_valid) { CU(cudaStreamWaitEvent(s, h->done, 0)); h->done_valid = false; }   // a plain solve queued before
     if (h->main_free_valid) CU(cudaStreamWaitEvent(s, h->main_free, 0));
     if (h->tail_free_valid[k]) CU(cudaStreamWaitEvent(s, h->tail_free[k], 0));
-    if (int rc = run_solve(h, B, 1, st, cf, ncoef, out8, traj, obj, status, iters, s, false, io_aos, 1, tail)) return rc;
+    key.phase = 1; key.tail = tail.ws;
+    if (int rc = run_solve(h, key, s, false, [&](long long* n) { return launch_solve_bulk(h->P, B, io, h->ws.as<double>(), tail, h->cfg, s, n); })) return rc;
     CU(cudaEventRecord(h->main_free, s));
     h->main_free_valid = true;
     // the tail runs on the context's own high-priority stream, behind the bulk; the caller's stream then waits for it,
     // so the call stays stream-ordered for its caller
     cudaStream_t ts = h->tail_stream[k] ? h->tail_stream[k] : s;
     if (ts != s) CU(cudaStreamWaitEvent(ts, h->main_free, 0));
-    if (int rc = run_solve(h, B, 1, st, cf, ncoef, out8, traj, obj, status, iters, ts, false, io_aos, 2, tail)) return rc;
+    key.phase = 2;
+    if (int rc = run_solve(h, key, ts, false, [&](long long* n) { return launch_solve_tail(h->P, B, io, tail, h->cfg, ts, n); })) return rc;
     CU(cudaEventRecord(h->tail_free[k], ts));
     h->tail_free_valid[k] = true;
     if (ts != s) CU(cudaStreamWaitEvent(s, h->tail_free[k], 0));
@@ -176,7 +222,8 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const double* st, const dou
     cudaError_t e = cudaEventRecord(e0, s);
     if (e != cudaSuccess) { cudaEventDestroy(e0); cudaEventDestroy(e1); return cuda_fail(e, "cudaEventRecord"); }
   }
-  int rc = run_solve(h, B, steps, st, cf, ncoef, out8, traj, obj, status, iters, s, caller_captures, io_aos);
+  int rc = run_solve(h, key, s, caller_captures,
+                     [&](long long* n) { return launch_solve(h->P, B, steps, io, h->ws.as<double>(), h->cfg, s, &h->ss, n); });
   if (rec) {
     cudaError_t e = rc == 0 ? cudaEventRecord(e1, s) : cudaErrorUnknown;
     if (e == cudaSuccess) h->timing.emplace_back(e0, e1);
@@ -187,56 +234,6 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const double* st, const dou
     h->done_valid = true;
   }
   return rc;
-}
-
-int run_solve(b200mpc_handle* h, int B, int steps, const double* st, const double* cf, int ncoef, double* out8,
-              double* traj, double* obj, int* status, int* iters, cudaStream_t s, bool caller_captures, int io_aos,
-              int phase, TailCtx tail) {
-  // the launch sequence: the whole solve, or one half of a pipelined one
-  auto launch = [&](long long* n) -> cudaError_t {
-    if (phase == 1) return launch_solve_bulk(h->P, B, st, cf, ncoef, h->ws.as<double>(), out8, traj, obj, status, iters, h->cfg, s, n, io_aos, tail);
-    if (phase == 2) return launch_solve_tail(h->P, B, st, cf, ncoef, out8, traj, obj, status, iters, h->cfg, s, n, io_aos, tail);
-    return launch_solve(h->P, B, steps, st, cf, ncoef, h->ws.as<double>(), out8, traj, obj, status, iters, h->cfg, s, &h->ss, n, io_aos);
-  };
-  // One solve is ~75 dependent launches; replaying a captured graph keeps the host out of the inner loop (several
-  // ranks / streams per host otherwise become launch-bound).  The legacy default stream cannot be captured.
-  bool done = false;
-  if (h->use_graphs && !caller_captures && s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread) {
-    b200mpc_handle::GraphEntry key{B, steps, ncoef, h->cfg.mode, h->cfg.rounds, h->cfg.fused_below, h->cfg.warm_start ? 1 : 0, h->cfg.split, h->repack_gen, io_aos, phase, tail.ws, h->cfg.warm_mu, st, cf, h->ws.p, out8, traj, obj, status, iters, nullptr, 0};
-    b200mpc_handle::GraphEntry* hit = nullptr;
-    for (auto& g : h->graphs)
-      if (g.B == key.B && g.steps == key.steps && g.ncoef == key.ncoef && g.mode == key.mode && g.rounds == key.rounds &&
-          g.fused_below == key.fused_below && g.warm == key.warm && g.split == key.split && g.repack_gen == key.repack_gen && g.io_aos == key.io_aos && g.phase == key.phase && g.tail == key.tail && g.warm_mu == key.warm_mu && g.st == key.st && g.cf == key.cf && g.ws == key.ws && g.out8 == key.out8 &&
-          g.traj == key.traj && g.obj == key.obj && g.status == key.status && g.iters == key.iters)
-        hit = &g;
-    if (!hit) {
-      cudaGraph_t graph = nullptr;
-      long long n = 0;
-      if (cudaStreamBeginCapture(s, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
-        cudaError_t le = launch(&n);
-        cudaError_t ce = cudaStreamEndCapture(s, &graph);
-        if (le == cudaSuccess && ce == cudaSuccess && graph) {
-          cudaGraphExec_t exec = nullptr;
-          if (cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
-            if (h->graphs.size() >= 96) { cudaGraphExecDestroy(h->graphs.front().exec); h->graphs.erase(h->graphs.begin()); }
-            key.exec = exec; key.n_kernels = n;
-            h->graphs.push_back(key);
-            hit = &h->graphs.back();
-          }
-        }
-        if (graph) cudaGraphDestroy(graph);
-      }
-      cudaGetLastError();   // a failed capture falls back to plain launches below
-    }
-    if (hit) {
-      CU(cudaGraphLaunch(hit->exec, s));
-      h->launches += hit->n_kernels;
-      done = true;
-    }
-  }
-  if (!done)
-    CU(launch(&h->launches));
-  return 0;
 }
 
 }  // namespace
@@ -390,6 +387,7 @@ int b200mpc_set_solver_mode(b200mpc_handle* h, int mode, int rounds, int fused_b
   h->cfg.mode = mode;
   if (rounds > 0) h->cfg.rounds = rounds;
   if (fused_below >= 0) h->cfg.fused_below = fused_below;
+  ++h->config_gen;
   return 0;
 }
 
@@ -398,6 +396,7 @@ int b200mpc_set_warm_start(b200mpc_handle* h, int enable, double mu_init) {
   if (enable && !(mu_init > 0.0 && mu_init <= 0.1)) return fail(B200MPC_ERR_ARG, "warm start: mu_init must be in (0, 0.1]");
   h->cfg.warm_start = enable != 0;
   if (enable) h->cfg.warm_mu = mu_init;
+  ++h->config_gen;
   return 0;
 }
 
@@ -405,6 +404,7 @@ int b200mpc_set_batch_split(b200mpc_handle* h, int parts) {
   if (!h) return fail(B200MPC_ERR_ARG, "null handle");
   if (parts < 1 || parts > 4) return fail(B200MPC_ERR_ARG, "batch split: parts must be 1..4");
   h->cfg.split = parts;
+  ++h->config_gen;
   return 0;
 }
 
@@ -414,7 +414,7 @@ int b200mpc_set_compaction(b200mpc_handle* h, double max_live_fraction, int from
   if (from_round < 1) return fail(B200MPC_ERR_ARG, "compaction: from_round must be >= 1");
   h->cfg.compact_max_live = max_live_fraction;
   h->cfg.compact_from = from_round;
-  ++h->repack_gen;
+  ++h->config_gen;
   return 0;
 }
 
@@ -424,7 +424,7 @@ int b200mpc_set_handover(b200mpc_handle* h, int occupied_slots, int from_round) 
   if (from_round < 1) return fail(B200MPC_ERR_ARG, "hand-over: from_round must be >= 1");
   h->cfg.handover_below = occupied_slots;
   h->cfg.handover_from = from_round;
-  ++h->repack_gen;   // part of the captured launch sequence
+  ++h->config_gen;
   return 0;
 }
 
@@ -446,7 +446,7 @@ int b200mpc_set_pipeline(b200mpc_handle* h, int depth, int tail_slots) {
   h->pipe_depth = depth;
   h->pipe_slots = depth > 0 ? (tail_slots + 63) / 64 * 64 : 0;
   h->pipe_calls = 0;
-  ++h->repack_gen;
+  ++h->config_gen;
   return 0;
 }
 
@@ -455,7 +455,7 @@ int b200mpc_set_restoration(b200mpc_handle* h, int mode) {
   if (mode < 0 || mode > 2) return fail(B200MPC_ERR_ARG, "restoration: mode must be 0, 1 or 2");
   h->P.resto = mode;
   h->resto_mode = mode;
-  ++h->repack_gen;   // the parameters are baked into captured graphs
+  ++h->config_gen;
   return 0;
 }
 
@@ -468,8 +468,22 @@ int b200mpc_solve_batch_device(b200mpc_handle* h, int B, const double* d_state6,
   if (int rc = check_solve_args(h, B, d_state6, d_coeffs, ncoef, d_out8)) return rc;
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
-  cudaStream_t s = stream ? (cudaStream_t)stream : h->stream;
-  return timed_solve(h, B, 1, d_state6, d_coeffs, ncoef, d_out8, d_traj, d_obj, d_status, d_iters, s);
+  SolveIO io;
+  io.state6 = d_state6; io.coeffs = d_coeffs; io.ncoef = ncoef;
+  io.out8 = d_out8; io.traj = d_traj; io.obj = d_obj; io.status = d_status; io.iters = d_iters;
+  return timed_solve(h, B, 1, io, stream ? (cudaStream_t)stream : h->stream);
+}
+
+// queues the copy of the host arrays state6 [B][6] and coeffs [B][ncoef] to in_aos and points io's inputs there (io_aos = 1)
+static int stage_inputs(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, SolveIO* io) {
+  const size_t nb = (size_t)B;
+  CU(h->in_aos.ensure(nb * (6 + ncoef) * sizeof(double)));
+  double* d_st = h->in_aos.as<double>();
+  double* d_cf = d_st + nb * 6;
+  CU(cudaMemcpyAsync(d_st, state6, nb * 6 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(d_cf, coeffs, nb * ncoef * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  io->state6 = d_st; io->coeffs = d_cf; io->ncoef = ncoef; io->io_aos = 1;
+  return 0;
 }
 
 // Everything b200mpc_solve_batch does except the final wait: copies, solve and copies back are queued on the handle's
@@ -485,19 +499,16 @@ static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, c
   // stage: H2D -> solve -> D2H.  The solver kernels read state6 / coeffs and write out8 in the reference's per-problem
   // order themselves (io_aos = 1: K6 fused into init / write_result); only the optional full trajectory goes through the
   // tiled transpose.
-  CU(h->in_aos.ensure(nb * (6 + ncoef) * sizeof(double)));
   CU(h->out_aos.ensure(nb * 8 * sizeof(double)));
   CU(h->obj.ensure(nb * sizeof(double)));
   CU(h->status.ensure(nb * sizeof(int)));
   CU(h->iters.ensure(nb * sizeof(int)));
   if (traj) { CU(h->traj_soa.ensure(nb * nv * sizeof(double))); CU(h->traj_aos.ensure(nb * nv * sizeof(double))); }
-  double* d_st = h->in_aos.as<double>();
-  double* d_cf = d_st + nb * 6;
-  CU(cudaMemcpyAsync(d_st, state6, nb * 6 * sizeof(double), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(d_cf, coeffs, nb * ncoef * sizeof(double), cudaMemcpyHostToDevice, s));
-  if (int rc = timed_solve(h, B, 1, d_st, d_cf, ncoef, h->out_aos.as<double>(), traj ? h->traj_soa.as<double>() : nullptr,
-                           h->obj.as<double>(), h->status.as<int>(), h->iters.as<int>(), s, 1))
-    return rc;
+  SolveIO io;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &io)) return rc;
+  io.out8 = h->out_aos.as<double>(); io.traj = traj ? h->traj_soa.as<double>() : nullptr;
+  io.obj = h->obj.as<double>(); io.status = h->status.as<int>(); io.iters = h->iters.as<int>();
+  if (int rc = timed_solve(h, B, 1, io, s)) return rc;
   CU(cudaMemcpyAsync(out8, h->out_aos.p, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (traj) {
     CU(launch_soa_to_aos(h->traj_soa.as<double>(), h->traj_aos.as<double>(), B, nv, s));
@@ -581,18 +592,14 @@ int b200mpc_closed_loop_batch(b200mpc_handle* h, int B, int steps, const double*
   CU(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
   const size_t nb = (size_t)B, ns = (size_t)steps;
-  CU(h->in_aos.ensure(nb * (6 + ncoef) * sizeof(double)));
   CU(h->out_aos.ensure(ns * nb * 8 * sizeof(double)));
   CU(h->obj.ensure(ns * nb * sizeof(double)));
   CU(h->iters.ensure(ns * nb * sizeof(int)));
-  double* d_st = h->in_aos.as<double>();
-  double* d_cf = d_st + nb * 6;
-  CU(cudaMemcpyAsync(d_st, state6, nb * 6 * sizeof(double), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(d_cf, coeffs, nb * ncoef * sizeof(double), cudaMemcpyHostToDevice, s));
+  SolveIO io;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &io)) return rc;
   // every step's 8-vector is written as [B][8] rows by the solver kernels (and read back as the next initial state)
-  if (int rc = timed_solve(h, B, steps, d_st, d_cf, ncoef, h->out_aos.as<double>(), nullptr, h->obj.as<double>(), nullptr,
-                           h->iters.as<int>(), s, 1))
-    return rc;
+  io.out8 = h->out_aos.as<double>(); io.obj = h->obj.as<double>(); io.iters = h->iters.as<int>();
+  if (int rc = timed_solve(h, B, steps, io, s)) return rc;
   CU(cudaMemcpyAsync(hist8, h->out_aos.p, ns * nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (cost) CU(cudaMemcpyAsync(cost, h->obj.p, ns * nb * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (iters) CU(cudaMemcpyAsync(iters, h->iters.p, ns * nb * sizeof(int), cudaMemcpyDeviceToHost, s));

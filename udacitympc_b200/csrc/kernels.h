@@ -9,10 +9,6 @@ namespace b200mpc {
 // doubles of workspace needed to solve B problems at horizon N
 size_t solve_workspace_doubles(int N, int B);
 
-// K1+K2+K3 fused: `steps` consecutive interior-point solves per problem (steps > 1 = closed loop, each solve
-// starting from the previous solve's predicted state).  All arrays field-major (SoA) over the batch.
-//   state6 [6][B], coeffs [ncoef][B], out8 [steps][8][B], traj [8N-2][B] (last step, optional),
-//   obj [steps][B] (optional), status [B] (last step, optional), iters [steps][B] (optional)
 // call once per device before the first solve on it
 cudaError_t solver_prepare_device();
 
@@ -26,13 +22,13 @@ struct SolveConfig {
   bool warm_start = false;   // closed loop only: steps after the first start from the shifted previous solution
   double warm_mu = 1e-4;     // barrier parameter a warm-started solve begins with
   int split = 4;             // large batches run as this many concurrent parts (see launch_solve)
-  // batch compaction: after every round from compact_from on, if the unfinished problems fill at most
-  // compact_max_live of the occupied workspace slots, they are moved to consecutive slots, so that later rounds run
-  // full warps on whole 32-byte sectors (0 = off)
   // adaptive hand-over (automatic rounds only): occupied slots (whole call) at which the cooperative kernel takes over
   int handover_below = 1184;      // one wave of 8 warps on 148 SMs
   int handover_from = 14;         // first round after which it may happen
   int handover_max_rounds = 0;    // 0 = by horizon: 20 up to N = 50, 2 N - 80 above (120 at N = 100); see handover_rounds (solve_kernel.cu)
+  // batch compaction: after every round from compact_from on, if the unfinished problems fill at most
+  // compact_max_live of the occupied workspace slots, they are moved to consecutive slots, so that later rounds run
+  // full warps on whole 32-byte sectors (0 = off)
   double compact_max_live = 0.7;
   int compact_from = 4;
   // pipelined solves (launch_solve_bulk / launch_solve_tail): rounds the tail context runs before its finisher (0 = by
@@ -46,23 +42,33 @@ struct SplitStreams {   // auxiliary streams / events owned by the handle (n_aux
   cudaStream_t aux[3] = {nullptr, nullptr, nullptr};
   cudaEvent_t fork = nullptr, join[3] = {nullptr, nullptr, nullptr};
 };
-cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6, const double* coeffs, int ncoef,
-                         double* ws, double* out8, double* traj, double* obj, int* status, int* iters,
-                         const SolveConfig& cfg, cudaStream_t stream, const SplitStreams* ss, long long* n_launches,
-                         int io_aos = 0);   // io_aos = 1: state6 [B][6], coeffs [B][ncoef], out8 [steps][B][8] (reference order)
+// The per-call buffers of a solve (device pointers).  io_aos = 0: field-major (SoA) over the batch
+//   state6 [6][B], coeffs [ncoef][B], out8 [steps][8][B], traj [8N-2][B] (last step, optional),
+//   obj [steps][B] (optional), status [B] (last step, optional), iters [steps][B] (optional);
+// io_aos = 1: state6 [B][6], coeffs [B][ncoef], out8 [steps][B][8] (reference order), the others as above
+struct SolveIO {
+  const double *state6 = nullptr, *coeffs = nullptr;
+  int ncoef = 0;
+  double *out8 = nullptr, *traj = nullptr, *obj = nullptr;
+  int *status = nullptr, *iters = nullptr;
+  int io_aos = 0;
+};
 
-// Pipelined solves: one solve as two launch sequences (see solve_kernel.cu).  A tail context is a workspace of
-// solve_workspace_doubles(N, slots) doubles.
+// K1+K2+K3 fused: `steps` consecutive interior-point solves per problem (steps > 1 = closed loop, each solve
+// starting from the previous solve's predicted state).  The launchers add one to *n_launches per kernel they launch.
+cudaError_t launch_solve(const Params& P, int B, int steps, const SolveIO& io, double* ws, const SolveConfig& cfg,
+                         cudaStream_t stream, const SplitStreams* ss, long long* n_launches);
+
+// Pipelined solves: one solve (steps = 1) as two launch sequences (see solve_kernel.cu).  A tail context is a workspace
+// of solve_workspace_doubles(N, slots) doubles.
 struct TailCtx {
   double* ws = nullptr;
   int slots = 0;
 };
-cudaError_t launch_solve_bulk(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* ws, double* out8,
-                              double* traj, double* obj, int* status, int* iters, const SolveConfig& cfg, cudaStream_t stream,
-                              long long* n_launches, int io_aos, const TailCtx& tail);
-cudaError_t launch_solve_tail(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* out8, double* traj,
-                              double* obj, int* status, int* iters, const SolveConfig& cfg, cudaStream_t stream, long long* n_launches,
-                              int io_aos, const TailCtx& tail);
+cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double* ws, const TailCtx& tail, const SolveConfig& cfg,
+                              cudaStream_t stream, long long* n_launches);
+cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const TailCtx& tail, const SolveConfig& cfg,
+                              cudaStream_t stream, long long* n_launches);
 
 // K6 batch I/O: [B][K] <-> [K][B]
 cudaError_t launch_aos_to_soa(const double* in, double* out, int B, int K, cudaStream_t stream);

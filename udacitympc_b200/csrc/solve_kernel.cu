@@ -372,16 +372,56 @@ static int coop_resident_warps(int N) {
   return sms * blocks * wpb;
 }
 
-// launches the cooperative kernel if the horizon fits in shared memory; returns false otherwise
-static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, cudaStream_t stream, cudaError_t* err, int take_below = 0) {
+// the kernels' parameter block for problems [b0, b1) of the B-problem batch in workspace L (desc: the compaction state
+// of these problems, or null: no compaction); warm_mu > 0: closed-loop steps after the first start from the shifted
+// previous solution with this barrier parameter
+static SolveArgs solve_args(int B, int steps, const SolveIO& io, const WsLayout& L, int* desc, int b0, int b1, double warm_mu) {
+  SolveArgs A{};
+  A.B = B; A.steps = steps; A.ncoef = io.ncoef; A.io_aos = io.io_aos ? 1 : 0; A.b0 = b0; A.b1 = b1;
+  A.warm = warm_mu > 0.0 ? 1 : 0; A.mu_warm = warm_mu;
+  A.state6 = io.state6; A.coeffs = io.coeffs;
+  A.ws = L.ws0; A.ws1 = L.ws1; A.map0 = L.map0; A.map1 = L.map1; A.desc = desc;
+  A.out8 = io.out8; A.traj = io.traj; A.obj = io.obj; A.status = io.status; A.iters = io.iters;
+  return A;
+}
+
+static int sweep_grid(const SolveArgs& A) { return (A.b1 - A.b0 + kBlock - 1) / kBlock; }
+
+// The launch helpers add one to *n per kernel they launch.  launch_round: one round of the thread-per-problem sweeps;
+// count_live: the step kernel counts the unfinished problems for the compaction attempt that follows
+static void launch_round(const Params& P, const SolveArgs& A, bool count_live, cudaStream_t stream, long long* n) {
+  SolveArgs As = A;
+  As.count_live = count_live ? 1 : 0;
+  mpc_factor_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  mpc_forward_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  mpc_step_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  *n += 3;
+}
+
+// a compaction attempt after a counting round; export_below > 0: a hand-off to the tail context T (mpc_repack_kernel)
+static void launch_repack(const Params& P, const SolveArgs& A, double max_live, cudaStream_t stream, long long* n,
+                          int export_below = 0, const WsLayout& T = WsLayout{}) {
+  mpc_repack_kernel<<<(A.b1 - A.b0 + 255) / 256, 256, 0, stream>>>(P, A, max_live, export_below, T.ws1, T.map0, T.desc);
+  *n += 1;
+}
+
+static void launch_fused(const Params& P, const SolveArgs& A, int fresh, cudaStream_t stream, long long* n) {
+  mpc_fused_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  *n += 1;
+}
+
+// launches the cooperative kernel if the horizon fits in shared memory (*err: the launch's error); returns false otherwise
+static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, int take_below, cudaStream_t stream, cudaError_t* err,
+                        long long* n) {
   const CoopShape c = coop_shape(P.N);
   if (c.warps == 0) return false;
   const int wpb = c.warps;
-  const int n = take_below > 0 && take_below < A.b1 - A.b0 ? take_below : A.b1 - A.b0;
-  int grid = (n + wpb - 1) / wpb;
+  const int nb = take_below > 0 && take_below < A.b1 - A.b0 ? take_below : A.b1 - A.b0;
+  int grid = (nb + wpb - 1) / wpb;
   const int cap = 4 * coop_resident_warps(P.N) / wpb;   // four waves; the warps stride over the rest
   if (cap > 0 && grid > cap) grid = cap;
   mpc_coop_kernel<<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);   // no idle warps: their registers would stay allocated
+  *n += 1;
   *err = cudaGetLastError();
   return true;
 }
@@ -397,40 +437,27 @@ static int handover_rounds(const Params& P, const SolveConfig& cfg) {
 
 // launches every kernel of the solve of problems [b0, b1) on one stream
 static cudaError_t launch_part(const Params& P, SolveArgs A, const SolveConfig& cfg, int rounds, int take_below, cudaStream_t stream, long long* n) {
-  const int nb = A.b1 - A.b0;
-  const int grid = (nb + kBlock - 1) / kBlock;
   for (int step = 0; step < A.steps; ++step) {
     A.step = step;
     cudaError_t ce = cudaSuccess;
     if (cfg.mode == kModeFused || A.B < cfg.fused_below) {
       A.desc = nullptr;
-      if (!(cfg.coop && cfg.mode != kModeFused && launch_coop(P, A, 1, stream, &ce))) mpc_fused_kernel<<<grid, kBlock, 0, stream>>>(P, A, 1);
-      if (ce != cudaSuccess) return ce;
-      *n += 1;
+      if (!(cfg.coop && cfg.mode != kModeFused && launch_coop(P, A, 1, 0, stream, &ce, n))) launch_fused(P, A, 1, stream, n);
     } else {
-      mpc_init_kernel<<<grid, kBlock, 0, stream>>>(P, A);
+      mpc_init_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+      *n += 1;
       for (int r = 0; r < rounds; ++r) {
         // a compaction attempt follows every round from compact_from on (not the last: only the finisher is left)
         const bool attempt = A.desc && r + 1 >= cfg.compact_from && r + 1 < rounds;
-        SolveArgs Ar = A;
-        Ar.count_live = attempt ? 1 : 0;
-        mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-        mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-        mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
-        if (attempt) {
-          mpc_repack_kernel<<<(nb + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, 0, nullptr, nullptr, nullptr);
-          *n += 1;
-          if (take_below > 0 && r + 1 >= cfg.handover_from && cfg.coop && launch_coop(P, A, 0, stream, &ce, take_below)) {
-            if (ce != cudaSuccess) return ce;
-            *n += 1;
-          }
-        }
+        launch_round(P, A, attempt, stream, n);
+        if (!attempt) continue;
+        launch_repack(P, A, cfg.compact_max_live, stream, n);
+        if (take_below > 0 && r + 1 >= cfg.handover_from && cfg.coop) launch_coop(P, A, 0, take_below, stream, &ce, n);
+        if (ce != cudaSuccess) return ce;
       }
-      if (!(cfg.coop && launch_coop(P, A, 0, stream, &ce))) mpc_fused_kernel<<<grid, kBlock, 0, stream>>>(P, A, 0);
-      if (ce != cudaSuccess) return ce;
-      *n += 2 + 3LL * rounds;
+      if (!(cfg.coop && launch_coop(P, A, 0, 0, stream, &ce, n))) launch_fused(P, A, 0, stream, n);
     }
-    ce = cudaGetLastError();
+    if (ce == cudaSuccess) ce = cudaGetLastError();
     if (ce != cudaSuccess) return ce;
   }
   return cudaSuccess;
@@ -440,16 +467,12 @@ static cudaError_t launch_part(const Params& P, SolveArgs A, const SolveConfig& 
 // streams (fork / join with events; capturable into a CUDA graph): the kernels of different parts are in different
 // sweeps at any moment, which fills the partial waves of the 252-register factor kernel and hides the thin tail of
 // one part behind the bulk of another even when the caller uses a single stream.
-cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6, const double* coeffs, int ncoef,
-                         double* ws, double* out8, double* traj, double* obj, int* status, int* iters,
-                         const SolveConfig& cfg, cudaStream_t stream, const SplitStreams* ss, long long* n_launches, int io_aos) {
+cudaError_t launch_solve(const Params& P, int B, int steps, const SolveIO& io, double* ws, const SolveConfig& cfg,
+                         cudaStream_t stream, const SplitStreams* ss, long long* n) {
   if (B <= 0) return cudaSuccess;
   const WsLayout L = ws_layout(ws, P.N, B);   // the compaction state holds one record per part
   // a warm-started step reads the previous solution at the problem's own slot: no compaction then
   int* desc = (!(cfg.compact_max_live > 0.0) || cfg.warm_start) ? nullptr : L.desc;
-  SolveArgs A{B, steps, 0, ncoef, io_aos ? 1 : 0, 0, B, cfg.warm_start ? 1 : 0, cfg.warm_mu, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, desc, 0,
-              out8, traj, obj, status, iters};
-  long long n = 0;
   int parts = 1;
   if (ss && cfg.mode == kModePerPass && cfg.split > 1 && B >= cfg.split * cfg.fused_below) parts = cfg.split < ss->n_aux + 1 ? cfg.split : ss->n_aux + 1;
   // automatic setting: up to handover_rounds() rounds, and after every late round the cooperative kernel takes the
@@ -459,28 +482,23 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6
   const int rounds = cfg.rounds > 0 ? cfg.rounds : (adaptive ? handover_rounds(P, cfg) : (parts > 1 ? 16 : 18));
   const int take_below = adaptive ? (cfg.handover_below / parts > 64 ? cfg.handover_below / parts : 64) : 0;
   cudaError_t e = cudaSuccess;
-  if (parts == 1) {
-    e = launch_part(P, A, cfg, rounds, take_below, stream, &n);
-  } else {
-    const int per = (((B + parts - 1) / parts) + 63) / 64 * 64;
+  if (parts > 1) {
     if ((e = cudaEventRecord(ss->fork, stream)) != cudaSuccess) return e;
     for (int p = 1; p < parts; ++p)
       if ((e = cudaStreamWaitEvent(ss->aux[p - 1], ss->fork, 0)) != cudaSuccess) return e;
-    for (int p = 0; p < parts && e == cudaSuccess; ++p) {
-      SolveArgs Ap = A;
-      Ap.b0 = p * per;
-      Ap.b1 = (p + 1) * per < B ? (p + 1) * per : B;
-      if (desc) Ap.desc = desc + p * kDescInts;
-      if (Ap.b0 >= Ap.b1) continue;
-      e = launch_part(P, Ap, cfg, rounds, take_below, p == 0 ? stream : ss->aux[p - 1], &n);
-    }
-    for (int p = 1; p < parts; ++p) {   // always join, also after an error, so a capture can end cleanly
-      cudaError_t e2 = cudaEventRecord(ss->join[p - 1], ss->aux[p - 1]);
-      if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(stream, ss->join[p - 1], 0);
-      if (e == cudaSuccess) e = e2;
-    }
   }
-  if (n_launches) *n_launches += n;
+  const int per = (((B + parts - 1) / parts) + 63) / 64 * 64;
+  for (int p = 0; p < parts && e == cudaSuccess; ++p) {
+    const int b0 = p * per, b1 = (p + 1) * per < B ? (p + 1) * per : B;
+    if (b0 >= b1) continue;
+    const SolveArgs A = solve_args(B, steps, io, L, desc ? desc + p * kDescInts : nullptr, b0, b1, cfg.warm_start ? cfg.warm_mu : 0.0);
+    e = launch_part(P, A, cfg, rounds, take_below, p == 0 ? stream : ss->aux[p - 1], n);
+  }
+  for (int p = 1; p < parts; ++p) {   // always join, also after an error, so a capture can end cleanly
+    cudaError_t e2 = cudaEventRecord(ss->join[p - 1], ss->aux[p - 1]);
+    if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(stream, ss->join[p - 1], 0);
+    if (e == cudaSuccess) e = e2;
+  }
   return e;
 }
 
@@ -493,57 +511,34 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const double* state6
 // the thin tail of one batch -- latency bound: a straggler needs up to hundreds of iterations at long horizons -- runs
 // under the bulk of the following batches instead of holding a full-size workspace.  Results do not depend on where a
 // problem is finished.
-static SolveArgs tail_args(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* out8, double* traj,
-                           double* obj, int* status, int* iters, int io_aos, const TailCtx& tail) {
-  const WsLayout L = ws_layout(tail.ws, P.N, tail.slots);
-  return SolveArgs{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, tail.slots, 0, 0.0, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, L.desc, 0,
-                   out8, traj, obj, status, iters};
-}
-
-cudaError_t launch_solve_bulk(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* ws, double* out8,
-                              double* traj, double* obj, int* status, int* iters, const SolveConfig& cfg, cudaStream_t stream,
-                              long long* n_launches, int io_aos, const TailCtx& tail) {
+cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double* ws, const TailCtx& tail, const SolveConfig& cfg,
+                              cudaStream_t stream, long long* n) {
   if (B <= 0) return cudaSuccess;
-  const WsLayout L = ws_layout(ws, P.N, B);
-  SolveArgs A{B, 1, 0, ncoef, io_aos ? 1 : 0, 0, B, 0, 0.0, state6, coeffs, L.ws0, L.ws1, L.map0, L.map1, L.desc, 0,
-              out8, traj, obj, status, iters};
-  const SolveArgs T = tail_args(P, B, state6, coeffs, ncoef, out8, traj, obj, status, iters, io_aos, tail);
-  const int grid = (B + kBlock - 1) / kBlock;
+  const WsLayout L = ws_layout(ws, P.N, B), T = ws_layout(tail.ws, P.N, tail.slots);
+  const SolveArgs A = solve_args(B, 1, io, L, L.desc, 0, B, 0.0);
   const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P, cfg);
-  long long n = 0;
   mpc_tail_reset_kernel<<<1, 32, 0, stream>>>(T.desc);
-  mpc_init_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-  n += 2;
+  *n += 1;
+  mpc_init_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  *n += 1;
   for (int r = 0; r < rounds; ++r) {
     const bool attempt = r + 1 >= cfg.compact_from;
-    SolveArgs Ar = A;
-    Ar.count_live = attempt ? 1 : 0;
-    mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
-    n += 3;
-    if (attempt) {
-      mpc_repack_kernel<<<(B + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, tail.slots, T.ws1, T.map0, T.desc);
-      n += 1;
-    }
+    launch_round(P, A, attempt, stream, n);
+    if (attempt) launch_repack(P, A, cfg.compact_max_live, stream, n, tail.slots, T);
   }
   // Whatever never fitted the tail context is finished in place, by the thread loop: in the normal case the workspace
   // is empty by now and the launch must be cheap -- a cooperative-kernel launch, even one that finds nothing to do,
   // asks for 100-200 KB of shared memory per block and has to wait for SMs to drain while the tails of the previous
   // batches keep them busy (measured at N = 100 with 32 tails in flight: ~150 ms per bulk).
-  mpc_fused_kernel<<<grid, kBlock, 0, stream>>>(P, A, 0);
-  n += 1;
-  cudaError_t ce = cudaGetLastError();
-  if (n_launches) *n_launches += n;
-  return ce;
+  launch_fused(P, A, 0, stream, n);
+  return cudaGetLastError();
 }
 
-cudaError_t launch_solve_tail(const Params& P, int B, const double* state6, const double* coeffs, int ncoef, double* out8, double* traj,
-                              double* obj, int* status, int* iters, const SolveConfig& cfg, cudaStream_t stream, long long* n_launches,
-                              int io_aos, const TailCtx& tail) {
+cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const TailCtx& tail, const SolveConfig& cfg,
+                              cudaStream_t stream, long long* n) {
   if (B <= 0) return cudaSuccess;
-  const SolveArgs A = tail_args(P, B, state6, coeffs, ncoef, out8, traj, obj, status, iters, io_aos, tail);
-  const int nb = tail.slots, grid = (nb + kBlock - 1) / kBlock;
+  const WsLayout L = ws_layout(tail.ws, P.N, tail.slots);
+  const SolveArgs A = solve_args(B, 1, io, L, L.desc, 0, tail.slots, 0.0);
   // Up to N = 50 the tail is short (the slowest problems need a few dozen iterations): a few rounds, after each of which
   // the cooperative kernel takes the rest over once it fits its resident warps, as in launch_solve.  Above that the tail
   // is long (N = 100: 2 % of the problems need more than 100 iterations, the slowest about 1000) and the tails of many
@@ -559,34 +554,21 @@ cudaError_t launch_solve_tail(const Params& P, int B, const double* state6, cons
     const int resident = coop_resident_warps(P.N);
     take_below = long_tail ? (cfg.tail_take_below > 0 ? cfg.tail_take_below : 32) : (cfg.handover_below < resident ? cfg.handover_below : resident);
     if (take_below > resident) take_below = resident;
-    if (take_below > nb) take_below = nb;
+    if (take_below > tail.slots) take_below = tail.slots;
   }
   const int coop_every = long_tail ? 8 : 1;
-  long long n = 0;
   cudaError_t ce = cudaSuccess;
   for (int r = 0; r < rounds; ++r) {
-    SolveArgs Ar = A;
-    Ar.count_live = 1;
-    mpc_factor_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    mpc_forward_kernel<<<grid, kBlock, 0, stream>>>(P, A);
-    mpc_step_kernel<<<grid, kBlock, 0, stream>>>(P, Ar);
-    mpc_repack_kernel<<<(nb + 255) / 256, 256, 0, stream>>>(P, A, cfg.compact_max_live, 0, nullptr, nullptr, nullptr);
-    n += 4;
-    if (take_below > 0 && (r + 1) % coop_every == 0 && launch_coop(P, A, 0, stream, &ce, take_below)) {
-      if (ce != cudaSuccess) return ce;
-      n += 1;
-    }
-  }
-  if (take_below > 0 && launch_coop(P, A, 0, stream, &ce, take_below)) {
+    launch_round(P, A, true, stream, n);
+    launch_repack(P, A, cfg.compact_max_live, stream, n);
+    if (take_below > 0 && (r + 1) % coop_every == 0) launch_coop(P, A, 0, take_below, stream, &ce, n);
     if (ce != cudaSuccess) return ce;
-    n += 1;
   }
+  if (take_below > 0) launch_coop(P, A, 0, take_below, stream, &ce, n);
+  if (ce != cudaSuccess) return ce;
   // what is left after the last round: the thread loop (the cooperative kernel took over above if the rest fits it)
-  mpc_fused_kernel<<<grid, kBlock, 0, stream>>>(P, A, 0);
-  n += 1;
-  if (ce == cudaSuccess) ce = cudaGetLastError();
-  if (n_launches) *n_launches += n;
-  return ce;
+  launch_fused(P, A, 0, stream, n);
+  return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------------
