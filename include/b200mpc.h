@@ -122,6 +122,35 @@ int b200mpc_solve_batch_multi(b200mpc_handle* const* hs, int n_handles, int B, c
 int b200mpc_closed_loop_batch(b200mpc_handle* h, int B, int steps, const double* state6, const double* coeffs,
                               int ncoef, double* hist8, double* cost, int* iters);
 
+/* 10N-4: length of the multiplier vector of one problem, in the reference's order: lambda of the constraint rows
+ * x_start+t .. epsi_start+t (6N, MPC.cpp:36-43, 120-138), then z_L of delta_t and a_t (2(N-1)), then z_U of delta_t and
+ * a_t (2(N-1)).  The states have no bounds in the reference (+-1e19, MPC.cpp:181-186), so they have no z. */
+int b200mpc_num_mults(const b200mpc_handle* h);
+
+/* b200mpc_solve_batch started from a caller-supplied primal-dual point, returning the multipliers.  NOT reference
+ * behaviour: the reference cold-starts every call (MPC.cpp:167-177) and reads only x and obj_value from the
+ * CppAD::ipopt::solve_result it receives (MPC.cpp:241-256); this is Ipopt's warm_start_init_point
+ * (IpWarmStartIterateInitializer) plus the lambda / zl / zu of that solve_result.  The use is a receding-horizon loop
+ * that refits the reference every step: start step k+1 from step k's traj and mult shifted by one stage
+ * (udacitympc_b200.shift_solution does that).
+ *   x_init     B x (8N-2) start point in the layout of traj, or NULL for the default start point.  Its s_0 is replaced by
+ *              state6; the controls are pushed 1e-3 max(1, |bound|) inside their bounds.
+ *   mult_init  B x (10N-4) multipliers in the layout of mult, or NULL: lambda = 0, z = mu / slack.  Bound multipliers are
+ *              kept >= 1e-3.  Needs x_init.
+ *   mu_init    initial barrier parameter, in (0, 0.1] (e.g. 1e-4); ignored without x_init
+ *   mult       B x (10N-4) the multipliers of the solution, unscaled as Ipopt returns them, or NULL
+ * x_init = NULL returns what b200mpc_solve_batch returns, bit for bit, plus mult.  A non-finite entry of a problem's
+ * x_init or mult_init gives that problem status -13 (Invalid_Number_Detected), 0 iterations.  The iterations start with
+ * a zero-length step that is not counted.  B200MPC_ERR_ARG for mult_init without x_init or mu_init outside (0, 0.1]. */
+int b200mpc_solve_batch_warm(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef,
+                             const double* x_init, const double* mult_init, double mu_init, double* out8, double* traj,
+                             double* mult, double* obj, int* status, int* iters);
+/* Same on device buffers, field-major like b200mpc_solve_batch_device: d_x_init[i*B+b], d_mult_init[i*B+b],
+ * d_mult[i*B+b].  Pipelined solves (b200mpc_set_pipeline) accept it like b200mpc_solve_batch_device. */
+int b200mpc_solve_batch_warm_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                    const double* d_x_init, const double* d_mult_init, double mu_init, double* d_out8,
+                                    double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters, void* stream);
+
 /* Warm start for b200mpc_closed_loop_batch (SURVEY 8f; NOT reference behaviour: the reference cold-starts every call,
  * MPC.cpp:167-177, and so does this library unless enabled here).  When enabled, every step after the first starts from
  * the previous step's solution shifted by one stage, with the barrier parameter at mu_init (e.g. 1e-4).  The optimum

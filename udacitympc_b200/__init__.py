@@ -30,7 +30,9 @@ from .api import (  # noqa: F401
     read_roadmap_csv,
     roadmap_reference_batch,
     rollout_batch,
+    shift_solution,
 )
 
 __all__ = ["B200MPCError", "MPC", "MPCParams", "global_kinematic", "lib_path", "load_library", "polyeval",
-           "polyeval_batch", "polyfit", "polyfit_batch", "read_roadmap_csv", "roadmap_reference_batch", "rollout_batch"]
+           "polyeval_batch", "polyfit", "polyfit_batch", "read_roadmap_csv", "roadmap_reference_batch", "rollout_batch",
+           "shift_solution"]

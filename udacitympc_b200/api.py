@@ -31,10 +31,15 @@ SYMBOLS = {
     "b200mpc_destroy": (None, [_vp]),
     "b200mpc_last_error": (ctypes.c_char_p, []),
     "b200mpc_num_vars": (ctypes.c_int, [_vp]),
+    "b200mpc_num_mults": (ctypes.c_int, [_vp]),
     "b200mpc_solve_batch": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _ip, _ip]),
     "b200mpc_solve_batch_async": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _ip, _ip]),
     "b200mpc_wait": (ctypes.c_int, [_vp]),
     "b200mpc_solve_batch_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200mpc_solve_batch_warm": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, ctypes.c_double, _dp, _dp,
+                                                _dp, _dp, _ip, _ip]),
+    "b200mpc_solve_batch_warm_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, ctypes.c_double, _vp,
+                                                       _vp, _vp, _vp, _vp, _vp, _vp]),
     "b200mpc_solve_batch_multi": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int,
                                                  _dp, _dp, _dp, _ip, _ip]),
     "b200mpc_closed_loop_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _ip]),
@@ -165,6 +170,11 @@ class MPC:
     def num_vars(self):
         return self._lib.b200mpc_num_vars(self._h)
 
+    @property
+    def num_mults(self):
+        """10N-4: lambda of the 6N constraint rows, then z_L and z_U of the 2(N-1) controls (b200mpc_num_mults)."""
+        return self._lib.b200mpc_num_mults(self._h)
+
     # -- the reference call
     def Solve(self, x0, coeffs):
         x0 = _f64(x0).ravel()
@@ -184,9 +194,13 @@ class MPC:
         return [float(v) for v in r["out8"][0]]
 
     # -- batched host-buffer call
-    def solve_batch(self, states, coeffs, want_traj=False):
+    def solve_batch(self, states, coeffs, want_traj=False, x_init=None, mult_init=None, mu_init=1e-4, want_mult=False):
         """states (B,6), coeffs (B,ncoef) or (ncoef,) shared by all problems.  Returns dict(out8 (B,8), cost (B,),
-        status (B,), iters (B,), traj (B,8N-2) if requested)."""
+        status (B,), iters (B,), traj (B,8N-2) if requested, mult (B,10N-4) if requested).
+
+        Warm start (not reference behaviour, b200mpc_solve_batch_warm): x_init (B,8N-2) in the layout of traj and
+        optionally mult_init (B,10N-4) in the layout of mult start the solve there with the barrier parameter mu_init;
+        shift_solution() turns one receding-horizon step's traj / mult into the next step's start."""
         states = _f64(states)
         if states.ndim != 2 or states.shape[1] != 6:
             raise ValueError("states must be (B, 6)")
@@ -202,12 +216,26 @@ class MPC:
         status = np.empty(B, dtype=np.int32)
         iters = np.empty(B, dtype=np.int32)
         traj = np.empty((B, self.num_vars)) if want_traj else None
-        _check(self._lib.b200mpc_solve_batch(self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(out8),
-                                             _ptr(traj) if want_traj else None, _ptr(cost),
-                                             status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
+        if x_init is None and mult_init is None and not want_mult:
+            _check(self._lib.b200mpc_solve_batch(self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(out8),
+                                                 _ptr(traj) if want_traj else None, _ptr(cost),
+                                                 status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
+        else:
+            if x_init is not None:
+                x_init = _f64(x_init, (B, self.num_vars))
+            if mult_init is not None:
+                mult_init = _f64(mult_init, (B, self.num_mults))
+            mult = np.empty((B, self.num_mults)) if want_mult else None
+            _check(self._lib.b200mpc_solve_batch_warm(
+                self._h, B, _ptr(states), _ptr(coeffs), ncoef, None if x_init is None else _ptr(x_init),
+                None if mult_init is None else _ptr(mult_init), float(mu_init), _ptr(out8),
+                _ptr(traj) if want_traj else None, _ptr(mult) if want_mult else None, _ptr(cost),
+                status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
         r = dict(out8=out8, cost=cost, status=status, iters=iters)
         if want_traj:
             r["traj"] = traj
+        if want_mult:
+            r["mult"] = mult
         return r
 
     def solve_batch_device(self, B, d_state6, d_coeffs, ncoef, d_out8, d_traj=0, d_obj=0, d_status=0, d_iters=0,
@@ -215,6 +243,15 @@ class MPC:
         """Raw device-pointer call (integers), field-major buffers; asynchronous on `stream`."""
         _check(self._lib.b200mpc_solve_batch_device(self._h, B, d_state6, d_coeffs, ncoef, d_out8, d_traj or None,
                                                     d_obj or None, d_status or None, d_iters or None, stream or None))
+
+    def solve_batch_warm_device(self, B, d_state6, d_coeffs, ncoef, d_x_init, d_mult_init, mu_init, d_out8, d_traj=0,
+                                d_mult=0, d_obj=0, d_status=0, d_iters=0, stream=0):
+        """Raw device-pointer warm start (integers), field-major buffers: d_x_init [8N-2][B] (0 = default start point),
+        d_mult_init / d_mult [10N-4][B] (0 = none); asynchronous on `stream`.  See b200mpc_solve_batch_warm_device."""
+        _check(self._lib.b200mpc_solve_batch_warm_device(self._h, B, d_state6, d_coeffs, ncoef, d_x_init or None,
+                                                         d_mult_init or None, float(mu_init), d_out8, d_traj or None,
+                                                         d_mult or None, d_obj or None, d_status or None, d_iters or None,
+                                                         stream or None))
 
     def wait(self):
         """Waits for everything queued on this handle's own stream (b200mpc_solve_batch_async calls)."""
@@ -268,7 +305,7 @@ class MPC:
         _check(self._lib.b200mpc_set_pipeline(self._h, int(depth), int(tail_slots)))
 
     def set_warm_start(self, enable=True, mu_init=1e-4):
-        """closed_loop() only: steps after the first start from the shifted previous solution (not reference behaviour)."""
+        """closed_loop() only (solve_batch takes x_init / mult_init instead): steps after the first start from the shifted previous solution (not reference behaviour)."""
         _check(self._lib.b200mpc_set_warm_start(self._h, int(enable), float(mu_init)))
 
     # -- measurement helpers
@@ -299,6 +336,48 @@ class MPC:
 
     def launch_count(self):
         return int(self._lib.b200mpc_launch_count(self._h))
+
+
+def _shift_index(N, mult):
+    """Source index of every entry of a solution (mult=False: 8N-2 variables, True: 10N-4 multipliers) shifted by one
+    stage: entry t of each per-stage block takes entry t+1, the last stage is repeated."""
+    M = N - 1
+    st = np.minimum(np.arange(N) + 1, N - 1)
+    ct = np.minimum(np.arange(M) + 1, M - 1)
+    blocks = [k * N + st for k in range(6)] + [6 * N + j * M + ct for j in range(4 if mult else 2)]
+    return np.concatenate(blocks)
+
+
+def shift_solution(traj, mult, N, field_major=None):
+    """One receding-horizon step: the solution (traj (8N-2 per problem), mult (10N-4 per problem) or None) shifted by one
+    stage -- states, controls and multipliers of stage t+1 move to stage t, the last stage is repeated -- as x_init /
+    mult_init of the next step's warm-started solve.  NumPy arrays or torch tensors (on any device: the shift runs
+    there), per-problem rows (B, 8N-2) as solve_batch returns them or field-major (8N-2, B) as the device entry points
+    use; field_major=None infers the layout from the shape.  Returns (x_init, mult_init) of the same kind and layout."""
+    nv = 8 * N - 2
+
+    def layout(a, n):
+        if field_major is not None:
+            return bool(field_major)
+        rows = a.ndim >= 1 and a.shape[-1] == n
+        fields = a.ndim == 2 and a.shape[0] == n
+        if rows == fields:
+            raise ValueError(f"cannot tell the layout of an array of shape {tuple(a.shape)}: pass field_major")
+        return fields
+
+    def shift(a, n, is_mult):
+        if a is None:
+            return None
+        if a.shape[0 if layout(a, n) else -1] != n:
+            raise ValueError(f"expected {n} entries per problem, got shape {tuple(a.shape)}")
+        idx = _shift_index(N, is_mult)
+        dim = 0 if layout(a, n) else a.ndim - 1
+        if isinstance(a, np.ndarray):
+            return np.ascontiguousarray(np.take(a, idx, axis=dim))
+        import torch
+        return a.index_select(dim, torch.as_tensor(idx, device=a.device)).contiguous()
+
+    return shift(traj, nv, False), shift(mult, 10 * N - 4, True)
 
 
 def solve_batch_multi(mpcs, states, coeffs, want_traj=False):

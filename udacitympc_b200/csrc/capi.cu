@@ -54,6 +54,7 @@ struct b200mpc_handle {
   int device = 0;
   cudaStream_t stream = nullptr;
   DevBuf ws, in_aos, out_aos, traj_soa, traj_aos, obj, status, iters, misc0, misc3;
+  DevBuf guess_aos, guess_soa, mult_soa, mult_aos;   // b200mpc_solve_batch_warm: x_init | mult_init rows and columns, mult
   bool timing_on = false;                                    // b200mpc_set_timing: measurement only, off by default
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timing;   // around every solve while timing_on
   cudaEvent_t done = nullptr;   // recorded after every solve: the next solve on this handle (any stream) waits for it
@@ -116,10 +117,17 @@ int check_solve_args(const b200mpc_handle* h, int B, const void* st, const void*
   return 0;
 }
 
+int check_guess_args(const void* x_init, const void* mult_init, double mu_init) {
+  if (mult_init && !x_init) return fail(B200MPC_ERR_ARG, "warm start: mult_init needs x_init");
+  if (x_init && !(mu_init > 0.0 && mu_init <= 0.1)) return fail(B200MPC_ERR_ARG, "warm start: mu_init must be in (0, 0.1]");
+  return 0;
+}
+
 bool same_key(const b200mpc_handle::GraphKey& a, const b200mpc_handle::GraphKey& b) {
   return a.phase == b.phase && a.B == b.B && a.steps == b.steps && a.io.state6 == b.io.state6 && a.io.coeffs == b.io.coeffs &&
          a.io.ncoef == b.io.ncoef && a.io.out8 == b.io.out8 && a.io.traj == b.io.traj && a.io.obj == b.io.obj &&
-         a.io.status == b.io.status && a.io.iters == b.io.iters && a.io.io_aos == b.io.io_aos && a.ws == b.ws &&
+         a.io.status == b.io.status && a.io.iters == b.io.iters && a.io.io_aos == b.io.io_aos && a.io.x_init == b.io.x_init &&
+         a.io.mult_init == b.io.mult_init && a.io.mu_init == b.io.mu_init && a.io.mult == b.io.mult && a.ws == b.ws &&
          a.tail == b.tail && a.config_gen == b.config_gen;
 }
 
@@ -374,7 +382,8 @@ void b200mpc_destroy(b200mpc_handle* h) {
     if (h->tail_stream[k]) cudaStreamDestroy(h->tail_stream[k]);
   }
   h->tail_ws.release();
-  DevBuf* bufs[] = {&h->ws, &h->in_aos, &h->out_aos, &h->traj_soa, &h->traj_aos, &h->obj, &h->status, &h->iters, &h->misc0, &h->misc3};
+  DevBuf* bufs[] = {&h->ws, &h->in_aos, &h->out_aos, &h->traj_soa, &h->traj_aos, &h->obj, &h->status, &h->iters, &h->misc0, &h->misc3,
+                    &h->guess_aos, &h->guess_soa, &h->mult_soa, &h->mult_aos};
   for (DevBuf* b : bufs) b->release();
   if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
@@ -460,17 +469,27 @@ int b200mpc_set_restoration(b200mpc_handle* h, int mode) {
 }
 
 int b200mpc_num_vars(const b200mpc_handle* h) { return h ? 8 * h->P.N - 2 : 0; }
+int b200mpc_num_mults(const b200mpc_handle* h) { return h ? 10 * h->P.N - 4 : 0; }
 long long b200mpc_launch_count(const b200mpc_handle* h) { return h ? h->launches : 0; }
 
 int b200mpc_solve_batch_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
                                double* d_out8, double* d_traj, double* d_obj, int* d_status, int* d_iters,
                                void* stream) {
+  return b200mpc_solve_batch_warm_device(h, B, d_state6, d_coeffs, ncoef, nullptr, nullptr, 0.0, d_out8, d_traj, nullptr, d_obj,
+                                         d_status, d_iters, stream);
+}
+
+int b200mpc_solve_batch_warm_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                    const double* d_x_init, const double* d_mult_init, double mu_init, double* d_out8,
+                                    double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters, void* stream) {
   if (int rc = check_solve_args(h, B, d_state6, d_coeffs, ncoef, d_out8)) return rc;
+  if (int rc = check_guess_args(d_x_init, d_mult_init, mu_init)) return rc;
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
   SolveIO io;
   io.state6 = d_state6; io.coeffs = d_coeffs; io.ncoef = ncoef;
   io.out8 = d_out8; io.traj = d_traj; io.obj = d_obj; io.status = d_status; io.iters = d_iters;
+  io.x_init = d_x_init; io.mult_init = d_mult_init; io.mu_init = d_x_init ? mu_init : 0.0; io.mult = d_mult;
   return timed_solve(h, B, 1, io, stream ? (cudaStream_t)stream : h->stream);
 }
 
@@ -488,9 +507,13 @@ static int stage_inputs(b200mpc_handle* h, int B, const double* state6, const do
 
 // Everything b200mpc_solve_batch does except the final wait: copies, solve and copies back are queued on the handle's
 // stream (asynchronous when the host buffers are pinned).
+// x_init / mult_init / mult (b200mpc_solve_batch_warm): per-problem rows on the host, moved through the tiled transposes
+// like traj.
 static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, double* out8,
-                               double* traj, double* obj, int* status, int* iters) {
+                               double* traj, double* obj, int* status, int* iters, const double* x_init = nullptr,
+                               const double* mult_init = nullptr, double mu_init = 0.0, double* mult = nullptr) {
   if (int rc = check_solve_args(h, B, state6, coeffs, ncoef, out8)) return rc;
+  if (int rc = check_guess_args(x_init, mult_init, mu_init)) return rc;
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
@@ -508,12 +531,39 @@ static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, c
   if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &io)) return rc;
   io.out8 = h->out_aos.as<double>(); io.traj = traj ? h->traj_soa.as<double>() : nullptr;
   io.obj = h->obj.as<double>(); io.status = h->status.as<int>(); io.iters = h->iters.as<int>();
+  const int nm = 10 * h->P.N - 4;
+  if (x_init) {
+    const size_t n = nb * (nv + (mult_init ? nm : 0));
+    CU(h->guess_aos.ensure(n * sizeof(double)));
+    CU(h->guess_soa.ensure(n * sizeof(double)));
+    double *ga = h->guess_aos.as<double>(), *gs = h->guess_soa.as<double>();
+    CU(cudaMemcpyAsync(ga, x_init, nb * nv * sizeof(double), cudaMemcpyHostToDevice, s));
+    CU(launch_aos_to_soa(ga, gs, B, nv, s));
+    h->launches += 1;
+    io.x_init = gs; io.mu_init = mu_init;
+    if (mult_init) {
+      CU(cudaMemcpyAsync(ga + nb * nv, mult_init, nb * nm * sizeof(double), cudaMemcpyHostToDevice, s));
+      CU(launch_aos_to_soa(ga + nb * nv, gs + nb * nv, B, nm, s));
+      h->launches += 1;
+      io.mult_init = gs + nb * nv;
+    }
+  }
+  if (mult) {
+    CU(h->mult_soa.ensure(nb * nm * sizeof(double)));
+    CU(h->mult_aos.ensure(nb * nm * sizeof(double)));
+    io.mult = h->mult_soa.as<double>();
+  }
   if (int rc = timed_solve(h, B, 1, io, s)) return rc;
   CU(cudaMemcpyAsync(out8, h->out_aos.p, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (traj) {
     CU(launch_soa_to_aos(h->traj_soa.as<double>(), h->traj_aos.as<double>(), B, nv, s));
     h->launches += 1;
     CU(cudaMemcpyAsync(traj, h->traj_aos.p, nb * nv * sizeof(double), cudaMemcpyDeviceToHost, s));
+  }
+  if (mult) {
+    CU(launch_soa_to_aos(h->mult_soa.as<double>(), h->mult_aos.as<double>(), B, nm, s));
+    h->launches += 1;
+    CU(cudaMemcpyAsync(mult, h->mult_aos.p, nb * nm * sizeof(double), cudaMemcpyDeviceToHost, s));
   }
   if (obj) CU(cudaMemcpyAsync(obj, h->obj.p, nb * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (status) CU(cudaMemcpyAsync(status, h->status.p, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -524,6 +574,17 @@ static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, c
 int b200mpc_solve_batch(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, double* out8,
                         double* traj, double* obj, int* status, int* iters) {
   if (int rc = enqueue_solve_batch(h, B, state6, coeffs, ncoef, out8, traj, obj, status, iters)) return rc;
+  if (B == 0) return 0;
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+int b200mpc_solve_batch_warm(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef,
+                             const double* x_init, const double* mult_init, double mu_init, double* out8, double* traj,
+                             double* mult, double* obj, int* status, int* iters) {
+  if (int rc = enqueue_solve_batch(h, B, state6, coeffs, ncoef, out8, traj, obj, status, iters, x_init, mult_init, mu_init, mult))
+    return rc;
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
   CU(cudaStreamSynchronize(h->stream));

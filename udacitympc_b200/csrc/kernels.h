@@ -44,7 +44,9 @@ struct SplitStreams {   // auxiliary streams / events owned by the handle (n_aux
 };
 // The per-call buffers of a solve (device pointers).  io_aos = 0: field-major (SoA) over the batch
 //   state6 [6][B], coeffs [ncoef][B], out8 [steps][8][B], traj [8N-2][B] (last step, optional),
-//   obj [steps][B] (optional), status [B] (last step, optional), iters [steps][B] (optional);
+//   obj [steps][B] (optional), status [B] (last step, optional), iters [steps][B] (optional),
+//   x_init [8N-2][B] + mult_init [10N-4][B] (optional: start from this point with barrier parameter mu_init instead of
+//   the default start point, Solver::init_guess; mult_init may be null), mult [10N-4][B] (last step, optional);
 // io_aos = 1: state6 [B][6], coeffs [B][ncoef], out8 [steps][B][8] (reference order), the others as above
 struct SolveIO {
   const double *state6 = nullptr, *coeffs = nullptr;
@@ -52,6 +54,9 @@ struct SolveIO {
   double *out8 = nullptr, *traj = nullptr, *obj = nullptr;
   int *status = nullptr, *iters = nullptr;
   int io_aos = 0;
+  const double *x_init = nullptr, *mult_init = nullptr;
+  double mu_init = 0.0;
+  double* mult = nullptr;
 };
 
 // K1+K2+K3 fused: `steps` consecutive interior-point solves per problem (steps > 1 = closed loop, each solve

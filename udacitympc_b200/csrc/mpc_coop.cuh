@@ -542,6 +542,41 @@ struct CoopSolver {
     }
     ex.sync();
   }
+  // warm starts, stage-parallel (Solver::init_warm / init_guess; the partial sums are added in stage order, so the result
+  // is bit-identical to the thread version)
+  MPC_HD void init_warm(const double* s0, double mu0) {
+    const int c = (int)S.w(iCUR);
+    const double df_old = S.w(dDF);
+    if (ex.lane0()) S.warm_shift(s0);
+    ex.sync();
+    warm_common(s0, c, mu0, df_old, true);
+  }
+  MPC_HD void init_guess(const double* s0, const double* x, size_t xs, const double* m, size_t ms, double mu0) {
+    ex.for_stages(N, [&](int t) { S.guess_stage(t, s0, x, xs, m, ms); });
+    ex.sync();
+    warm_common(s0, 0, mu0, 1.0, m != nullptr);
+    if (ex.lane0()) S.guess_check();
+    ex.sync();
+  }
+  MPC_HD void warm_common(const double* s0, int c, double mu0, double df_old, bool have_mult) {
+    static_assert(Solver<LANES>::kWarmRed <= sizeof(st->red) / sizeof(double), "warm-start partials must fit CoopStage::red");
+    const int b = kX * c;
+    ex.for_stages(M, [&](int t) { S.warm_push_stage(t, b); });
+    ex.sync();
+    ex.for_stages(N, [&](int t) { S.warm_stage(t, b, st[t].red); });
+    ex.sync();
+    if (ex.lane0()) {
+      double f = 0.0, th = 0.0, cm = 0.0, sl = 0.0, gmax = 0.0;
+      for (int t = 0; t < N; ++t) S.warm_add(t, st[t].red, f, th, cm, sl, gmax);
+      S.warm_scalars(s0, c, mu0, gmax);
+      S.warm_finish(f, th, cm, sl);
+      pub->df = S.df; pub->mu = S.mu;
+    }
+    ex.sync();
+    const double ratio = pub->df / df_old, mu = pub->mu;
+    ex.for_stages(N, [&](int t) { S.warm_mult_stage(t, b, ratio, mu, have_mult); });
+    ex.sync();
+  }
   // A problem taken over in the middle of an iteration (phase FORWARD, or STEP during backtracking): re-stage what
   // the earlier sweeps of this iteration left in shared memory, without touching the control state.
   MPC_HD void rebuild() {

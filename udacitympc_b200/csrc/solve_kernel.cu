@@ -87,6 +87,10 @@ struct SolveArgs {
   double* obj;            // [steps][B] or null
   int* status;            // [B] or null (last step)
   int* iters;             // [steps][B] or null
+  const double* x_init;   // [8N-2][B] or null: fresh solves start from this point (Solver::init_guess)
+  const double* mult_init;   // [10N-4][B] or null (with x_init)
+  double mu_init;
+  double* mult;           // [10N-4][B] or null (last step)
 };
 
 __device__ __forceinline__ double* slot_base(const Params& P, double* ws, int slot) {
@@ -123,6 +127,10 @@ __device__ __forceinline__ void load_state6(const SolveArgs& A, int b, double* s
   for (int k = 0; k < 6; ++k)
     s0[k] = A.step == 0 ? A.state6[A.io_aos ? (size_t)b * 6 + k : (size_t)k * A.B + b] : A.out8[out8_index(A, A.step - 1, k, b)];
 }
+// Warm-start I/O (SolveArgs::x_init / mult_init / mult) is compiled only into the WIO = true instance of each kernel that
+// starts or finishes problems, and that instance is launched only when a call uses it: a call without it runs kernels
+// that do not carry its code (the factor and step sweeps: the same machine code as without the feature).
+template <bool WIO>
 __device__ __forceinline__ void write_result(const Params& P, const SolveArgs& A, int b, Solver<32>& S) {
   Result R;
   S.finish(R, (A.traj && A.step == A.steps - 1) ? A.traj + b : nullptr, (size_t)A.B);
@@ -131,7 +139,10 @@ __device__ __forceinline__ void write_result(const Params& P, const SolveArgs& A
   if (A.obj) A.obj[(size_t)A.step * A.B + b] = R.obj;
   if (A.iters) A.iters[(size_t)A.step * A.B + b] = R.iters;
   if (A.status && A.step == A.steps - 1) A.status[b] = R.status;
+  if (WIO && A.mult && A.step == A.steps - 1) S.write_mult(A.mult + b, (size_t)A.B);
 }
+// the caller's multipliers of problem b for a fresh solve from its point (slot == problem), or null
+__device__ __forceinline__ const double* guess_mult(const SolveArgs& A, int b) { return A.mult_init ? A.mult_init + b : nullptr; }
 
 // one atomic per group of converged lanes
 __device__ __forceinline__ void count_live(int* counter) {
@@ -140,6 +151,7 @@ __device__ __forceinline__ void count_live(int* counter) {
 }
 
 // ---- per-pass kernels ---------------------------------------------------------------------------------------
+template <bool WIO>
 __global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
   const int b = A.b0 + blockIdx.x * blockDim.x + threadIdx.x;   // always launched on the uncompacted batch
   if (b >= A.b1) return;
@@ -150,11 +162,13 @@ __global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant_
   load_state6(A, b, s0);
   load_coeffs(A, b, cf);
   if (A.warm && A.step > 0) { S.set_coeffs(cf, A.ncoef); S.init_warm(s0, A.mu_warm); }
+  else if (WIO && A.x_init) { S.set_coeffs(cf, A.ncoef); S.init_guess(s0, A.x_init + b, (size_t)A.B, guess_mult(A, b), (size_t)A.B, A.mu_init); }
   else S.init(s0, cf, A.ncoef);
   S.store_state();
-  if (S.phase == PH_DONE) write_result(P, A, b, S);   // invalid number at the starting point
+  if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);   // invalid number at the starting point
 }
 
+template <bool WIO>
 __global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
   int slot, b;
   double* ws;
@@ -167,7 +181,7 @@ __global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const
   S.kernel_factor();
   if (S.phase == PH_DONE) {   // inertia correction exhausted (IpPDPerturbationHandler.cpp:380-388)
     S.load_state();
-    write_result(P, A, b, S);
+    write_result<WIO>(P, A, b, S);
   }
 }
 
@@ -181,6 +195,7 @@ __global__ void __launch_bounds__(kBlock, kFwdBlocks) mpc_forward_kernel(const _
   S.kernel_forward();
 }
 
+template <bool WIO>
 __global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
   int slot, b;
   double* ws;
@@ -197,7 +212,7 @@ __global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __g
   S.sb = stage + threadIdx.x; S.sbs = kBlock;
   load_coeffs(A, b, S.cf);
   S.kernel_step();
-  if (S.phase == PH_DONE) write_result(P, A, b, S);
+  if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);
   else if (A.count_live) count_live(A.desc + kLive);
 }
 
@@ -260,6 +275,7 @@ __global__ void mpc_tail_reset_kernel(int* t_desc) {
 }
 
 // ---- fused kernel: finishes whatever is still active (fresh == 1: starts from the inputs) ---------------------
+template <bool WIO>
 __global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A, int fresh) {
   int slot, b;
   double* ws;
@@ -272,6 +288,7 @@ __global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant
     double s0[6];
     load_state6(A, b, s0);
     if (A.warm && A.step > 0) S.init_warm(s0, A.mu_warm);
+    else if (WIO && A.x_init) S.init_guess(s0, A.x_init + b, (size_t)A.B, guess_mult(A, b), (size_t)A.B, A.mu_init);
     else S.init(s0, S.cf, kMaxCoef);
   } else {
     if (S.load_phase() == PH_DONE) return;
@@ -279,7 +296,7 @@ __global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant
   }
   while (S.phase != PH_DONE) S.trip();
   S.store_state();
-  write_result(P, A, b, S);
+  write_result<WIO>(P, A, b, S);
 }
 
 // ---- cooperative kernel: one problem per warp (latency path: small batches, the tail of a batch, stragglers) -----
@@ -296,6 +313,7 @@ struct DevExec {
 // take_below > 0: conditional hand-over after a round -- the kernel acts only once the batch has been compacted to at
 // most take_below occupied slots (two waves of the cooperative kernel); from then on the sweeps of later rounds find
 // nothing to do
+template <bool WIO>
 __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A, int fresh,
                                                        int warps_per_block, int doubles_per_warp, int take_below) {
   extern __shared__ double coop_smem[];
@@ -320,10 +338,9 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
     if (fresh) {
       double s0[6];
       load_state6(A, b, s0);
-      if (A.warm && A.step > 0) {
-        if (lane == 0) S.init_warm(s0, A.mu_warm);
-        __syncwarp();
-      } else C.init(s0);
+      if (A.warm && A.step > 0) C.init_warm(s0, A.mu_warm);
+      else if (WIO && A.x_init) C.init_guess(s0, A.x_init + b, (size_t)A.B, guess_mult(A, b), (size_t)A.B, A.mu_init);
+      else C.init(s0);
     } else {
       if (S.load_phase() == PH_DONE) continue;   // whole warp
       if (lane == 0) S.load_state();
@@ -332,7 +349,7 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
     C.run();
     if (lane == 0) {
       S.store_state();
-      write_result(P, A, b, S);
+      write_result<WIO>(P, A, b, S);
     }
     __syncwarp();
   }
@@ -341,7 +358,9 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
 constexpr size_t kCoopSmemMax = 200 * 1024;   // dynamic shared memory of one cooperative block, at most
 // per-device, once (b200mpc_create)
 cudaError_t solver_prepare_device() {
-  return cudaFuncSetAttribute(mpc_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  cudaError_t e = cudaFuncSetAttribute(mpc_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  return e;
 }
 
 static size_t coop_doubles_per_warp(int N) { return (size_t)N * kCoopStageDoubles + (sizeof(CoopPub) + 7) / 8; }
@@ -382,19 +401,29 @@ static SolveArgs solve_args(int B, int steps, const SolveIO& io, const WsLayout&
   A.state6 = io.state6; A.coeffs = io.coeffs;
   A.ws = L.ws0; A.ws1 = L.ws1; A.map0 = L.map0; A.map1 = L.map1; A.desc = desc;
   A.out8 = io.out8; A.traj = io.traj; A.obj = io.obj; A.status = io.status; A.iters = io.iters;
+  A.x_init = io.x_init; A.mult_init = io.mult_init; A.mu_init = io.mu_init; A.mult = io.mult;
   return A;
 }
 
 static int sweep_grid(const SolveArgs& A) { return (A.b1 - A.b0 + kBlock - 1) / kBlock; }
+// the call reads a start point or writes multipliers: the WIO = true kernel instances
+static bool warm_io(const SolveArgs& A) { return A.x_init != nullptr || A.mult != nullptr; }
+static void launch_init(const Params& P, const SolveArgs& A, cudaStream_t stream, long long* n) {
+  if (warm_io(A)) mpc_init_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else mpc_init_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  *n += 1;
+}
 
 // The launch helpers add one to *n per kernel they launch.  launch_round: one round of the thread-per-problem sweeps;
 // count_live: the step kernel counts the unfinished problems for the compaction attempt that follows
 static void launch_round(const Params& P, const SolveArgs& A, bool count_live, cudaStream_t stream, long long* n) {
   SolveArgs As = A;
   As.count_live = count_live ? 1 : 0;
-  mpc_factor_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  if (warm_io(A)) mpc_factor_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else mpc_factor_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
   mpc_forward_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  mpc_step_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  if (warm_io(A)) mpc_step_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  else mpc_step_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
   *n += 3;
 }
 
@@ -406,7 +435,8 @@ static void launch_repack(const Params& P, const SolveArgs& A, double max_live, 
 }
 
 static void launch_fused(const Params& P, const SolveArgs& A, int fresh, cudaStream_t stream, long long* n) {
-  mpc_fused_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  if (warm_io(A)) mpc_fused_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else mpc_fused_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
   *n += 1;
 }
 
@@ -420,7 +450,9 @@ static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, int take
   int grid = (nb + wpb - 1) / wpb;
   const int cap = 4 * coop_resident_warps(P.N) / wpb;   // four waves; the warps stride over the rest
   if (cap > 0 && grid > cap) grid = cap;
-  mpc_coop_kernel<<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);   // no idle warps: their registers would stay allocated
+  // no idle warps: their registers would stay allocated
+  if (warm_io(A)) mpc_coop_kernel<true><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);
+  else mpc_coop_kernel<false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);
   *n += 1;
   *err = cudaGetLastError();
   return true;
@@ -444,8 +476,7 @@ static cudaError_t launch_part(const Params& P, SolveArgs A, const SolveConfig& 
       A.desc = nullptr;
       if (!(cfg.coop && cfg.mode != kModeFused && launch_coop(P, A, 1, 0, stream, &ce, n))) launch_fused(P, A, 1, stream, n);
     } else {
-      mpc_init_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-      *n += 1;
+      launch_init(P, A, stream, n);
       for (int r = 0; r < rounds; ++r) {
         // a compaction attempt follows every round from compact_from on (not the last: only the finisher is left)
         const bool attempt = A.desc && r + 1 >= cfg.compact_from && r + 1 < rounds;
@@ -519,8 +550,7 @@ cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double*
   const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P, cfg);
   mpc_tail_reset_kernel<<<1, 32, 0, stream>>>(T.desc);
   *n += 1;
-  mpc_init_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  *n += 1;
+  launch_init(P, A, stream, n);
   for (int r = 0; r < rounds; ++r) {
     const bool attempt = r + 1 >= cfg.compact_from;
     launch_round(P, A, attempt, stream, n);
