@@ -151,6 +151,34 @@ int b200mpc_solve_batch_warm_device(b200mpc_handle* h, int B, const double* d_st
                                     const double* d_x_init, const double* d_mult_init, double mu_init, double* d_out8,
                                     double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters, void* stream);
 
+/* Adjoint sensitivities (vector-Jacobian product) of B solutions: the derivative of a scalar loss L(out8, traj, obj) of
+ * each problem's solution w.r.t. its initial state, its reference polynomial and the handle's cost parameters, by the
+ * implicit-function theorem at the returned primal-dual point (the differentiable-MPC layer; Ipopt's sIPOPT does the
+ * same).  NOT reference behaviour: the reference returns no derivatives.  One Riccati solve of the KKT system of the
+ * unscaled problem per problem (about one interior-point iteration), one kernel launch.
+ *   state6, coeffs   the inputs of the solve (B x 6, B x ncoef)
+ *   traj, mult       B x (8N-2), B x (10N-4): the solution and multipliers b200mpc_solve_batch_warm returned for them.
+ *                    They must come from a converged solve (status 0 or 1) on a handle with the same params; the
+ *                    derivative is taken at this point as given (its controls are not pushed inside the bounds).
+ *   g_out8 (B x 8), g_traj (B x (8N-2)), g_obj (B)   dL/d(out8, traj, obj), or NULL; at least one must be given.
+ *                    out8[0..5] is traj's state of t = 1, out8[6], out8[7] its controls of t = 0.
+ *   grad_state6 (B x 6), grad_coeffs (B x ncoef), grad_params (B x 8: ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta,
+ *                    w_da; per problem, a caller sums them), or NULL
+ *   status (B) or NULL: 0 ok; -3 a 2x2 control block of the adjoint factorisation is not positive definite at the point
+ *                    (not a strict local minimum, or not a point of this handle's problem); -13 a non-finite input.
+ *                    The problem's gradients are NaN then.
+ * B200MPC_ERR_ARG for a null handle, B <= 0, ncoef outside [2, 4], a null state6 / coeffs / traj / mult or no incoming
+ * gradient.  The call uses the handle's workspace and is ordered like a solve on the handle. */
+int b200mpc_solve_batch_vjp(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* traj,
+                            const double* mult, const double* g_out8, const double* g_traj, const double* g_obj,
+                            double* grad_state6, double* grad_coeffs, double* grad_params, int* status);
+/* Same on device buffers, field-major like b200mpc_solve_batch_warm_device (d_x[i*B+b] for every array), asynchronous
+ * on `stream` (NULL: the handle's stream).  Exactly one kernel launch. */
+int b200mpc_solve_batch_vjp_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                   const double* d_traj, const double* d_mult, const double* d_g_out8, const double* d_g_traj,
+                                   const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
+                                   int* d_status, void* stream);
+
 /* Warm start for b200mpc_closed_loop_batch (SURVEY 8f; NOT reference behaviour: the reference cold-starts every call,
  * MPC.cpp:167-177, and so does this library unless enabled here).  When enabled, every step after the first starts from
  * the previous step's solution shifted by one stage, with the barrier parameter at mu_init (e.g. 1e-4).  The optimum

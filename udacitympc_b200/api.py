@@ -40,6 +40,9 @@ SYMBOLS = {
                                                 _dp, _dp, _ip, _ip]),
     "b200mpc_solve_batch_warm_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, ctypes.c_double, _vp,
                                                        _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200mpc_solve_batch_vjp": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
+                                               _ip]),
+    "b200mpc_solve_batch_vjp_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 10),
     "b200mpc_solve_batch_multi": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int,
                                                  _dp, _dp, _dp, _ip, _ip]),
     "b200mpc_closed_loop_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _ip]),
@@ -119,6 +122,10 @@ def default_params(**kw):
             raise TypeError(f"unknown parameter {k}")
         setattr(p, k, v)
     return p
+
+
+# the parameters b200mpc_solve_batch_vjp differentiates, in the order of its grad_params
+PARAM_NAMES = ("ref_v", "w_cte", "w_epsi", "w_v", "w_delta", "w_a", "w_ddelta", "w_da")
 
 
 class MPC:
@@ -252,6 +259,47 @@ class MPC:
                                                          d_mult_init or None, float(mu_init), d_out8, d_traj or None,
                                                          d_mult or None, d_obj or None, d_status or None, d_iters or None,
                                                          stream or None))
+
+    def solve_batch_vjp(self, states, coeffs, traj, mult, g_out8=None, g_traj=None, g_obj=None, want_params=False):
+        """Adjoint sensitivities of solutions (b200mpc_solve_batch_vjp; not reference behaviour): for a loss L with the
+        incoming gradients g_out8 (B,8), g_traj (B,8N-2), g_obj (B,) -- any of them None, not all -- returns
+        dict(grad_state6 (B,6), grad_coeffs (B,ncoef) per problem, status (B,), and grad_params (B,8) in the order
+        PARAM_NAMES if want_params).  traj (B,8N-2) and mult (B,10N-4) must be a converged solution of (states, coeffs)
+        on a handle with these params, as solve_batch(..., want_traj=True, want_mult=True) returns it."""
+        states = _f64(states)
+        if states.ndim != 2 or states.shape[1] != 6:
+            raise ValueError("states must be (B, 6)")
+        B = states.shape[0]
+        coeffs = _f64(coeffs)
+        if coeffs.ndim == 1:
+            coeffs = np.ascontiguousarray(np.broadcast_to(coeffs, (B, coeffs.size)))
+        if coeffs.shape[0] != B:
+            raise ValueError("coeffs must be (B, ncoef)")
+        ncoef = coeffs.shape[1]
+        traj = _f64(traj, (B, self.num_vars))
+        mult = _f64(mult, (B, self.num_mults))
+        g_out8 = None if g_out8 is None else _f64(g_out8, (B, 8))
+        g_traj = None if g_traj is None else _f64(g_traj, (B, self.num_vars))
+        g_obj = None if g_obj is None else _f64(g_obj, (B,))
+        gs = np.empty((B, 6)); gc = np.empty((B, ncoef)); gp = np.empty((B, 8)) if want_params else None
+        status = np.empty(B, dtype=np.int32)
+        _check(self._lib.b200mpc_solve_batch_vjp(
+            self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(traj), _ptr(mult), None if g_out8 is None else _ptr(g_out8),
+            None if g_traj is None else _ptr(g_traj), None if g_obj is None else _ptr(g_obj), _ptr(gs), _ptr(gc),
+            None if gp is None else _ptr(gp), status.ctypes.data_as(_ip)))
+        r = dict(grad_state6=gs, grad_coeffs=gc, status=status)
+        if want_params:
+            r["grad_params"] = gp
+        return r
+
+    def solve_batch_vjp_device(self, B, d_state6, d_coeffs, ncoef, d_traj, d_mult, d_g_out8=0, d_g_traj=0, d_g_obj=0,
+                               d_grad_state6=0, d_grad_coeffs=0, d_grad_params=0, d_status=0, stream=0):
+        """Raw device-pointer VJP (integers, 0 = none), field-major buffers; one kernel launch, asynchronous on `stream`.
+        See b200mpc_solve_batch_vjp_device."""
+        _check(self._lib.b200mpc_solve_batch_vjp_device(self._h, B, d_state6, d_coeffs, ncoef, d_traj, d_mult,
+                                                        d_g_out8 or None, d_g_traj or None, d_g_obj or None,
+                                                        d_grad_state6 or None, d_grad_coeffs or None, d_grad_params or None,
+                                                        d_status or None, stream or None))
 
     def wait(self):
         """Waits for everything queued on this handle's own stream (b200mpc_solve_batch_async calls)."""

@@ -1,0 +1,99 @@
+"""Batched MPC solves as a differentiable PyTorch operation (not reference behaviour).
+
+    out8, traj, obj, status = udacitympc_b200.autograd.solve(mpc, states, coeffs)
+
+The forward pass is one batched solve (b200mpc_solve_batch_warm[_device] from the default start point, which also
+returns the multipliers); the backward pass is one adjoint solve at that solution (b200mpc_solve_batch_vjp[_device]).
+CUDA tensors stay on the device and run on torch's current stream of their device, which must be the MPC handle's
+device; CPU tensors go through the host entry points.  The only module of the package that imports torch.
+"""
+import torch
+
+__all__ = ["solve"]
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else 0
+
+
+def _stream(dev):
+    """torch's current stream on dev as the library's stream argument.  torch's default stream is the legacy default
+    stream, handle 0, which the library reads as "the handle's own stream": pass cudaStreamLegacy (1) for it instead, so
+    the library's work is ordered with torch's."""
+    return torch.cuda.current_stream(dev).cuda_stream or 1
+
+
+def _fields(t):
+    """(B, k) -> the field-major (k, B) float64 buffer the device entry points take."""
+    return t.detach().to(torch.float64).t().contiguous()
+
+
+class _Solve(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mpc, states, coeffs):
+        B = states.shape[0]
+        shared = coeffs.dim() == 1
+        cf = coeffs.detach().to(torch.float64).expand(B, -1) if shared else coeffs.detach().to(torch.float64)
+        st = states.detach().to(torch.float64)
+        nv, nm = mpc.num_vars, mpc.num_mults
+        if states.is_cuda:
+            if states.device.index != mpc.device or coeffs.device != states.device:
+                raise ValueError(f"states / coeffs must be on cuda:{mpc.device}, the MPC handle's device")
+            dev = states.device
+            st_f, cf_f = _fields(st), _fields(cf)
+            out8 = torch.empty(8, B, dtype=torch.float64, device=dev)
+            traj = torch.empty(nv, B, dtype=torch.float64, device=dev)
+            mult = torch.empty(nm, B, dtype=torch.float64, device=dev)
+            obj = torch.empty(B, dtype=torch.float64, device=dev)
+            status = torch.empty(B, dtype=torch.int32, device=dev)
+            mpc.solve_batch_warm_device(B, _ptr(st_f), _ptr(cf_f), cf.shape[1], 0, 0, 0.0, _ptr(out8), _ptr(traj),
+                                        _ptr(mult), _ptr(obj), _ptr(status), 0, _stream(dev))
+            out8, traj, mult = out8.t(), traj.t(), mult.t()
+        else:
+            r = mpc.solve_batch(st.numpy(), cf.contiguous().numpy(), want_traj=True, want_mult=True)
+            out8, traj, mult = torch.from_numpy(r["out8"]), torch.from_numpy(r["traj"]), torch.from_numpy(r["mult"])
+            obj, status = torch.from_numpy(r["cost"]), torch.from_numpy(r["status"])
+        ctx.mpc, ctx.shared = mpc, shared
+        ctx.dtypes = (states.dtype, coeffs.dtype)
+        ctx.save_for_backward(st, cf, traj, mult, status)
+        ctx.mark_non_differentiable(status)
+        dt = states.dtype
+        return out8.to(dt), traj.to(dt), obj.to(dt), status
+
+    @staticmethod
+    def backward(ctx, g_out8, g_traj, g_obj, _g_status):
+        st, cf, traj, mult, status = ctx.saved_tensors
+        mpc = ctx.mpc
+        B, ncoef = cf.shape
+        g = [None if v is None else v.detach().to(torch.float64) for v in (g_out8, g_traj, g_obj)]
+        if st.is_cuda:
+            dev = st.device
+            gs = torch.empty(6, B, dtype=torch.float64, device=dev)
+            gc = torch.empty(ncoef, B, dtype=torch.float64, device=dev)
+            vs = torch.empty(B, dtype=torch.int32, device=dev)
+            keep = [_fields(st), _fields(cf), traj.t().contiguous(), mult.t().contiguous(),
+                    None if g[0] is None else _fields(g[0]), None if g[1] is None else _fields(g[1]),
+                    None if g[2] is None else g[2].contiguous()]
+            mpc.solve_batch_vjp_device(B, *[_ptr(k) for k in keep[:2]], ncoef, *[_ptr(k) for k in keep[2:]], _ptr(gs),
+                                       _ptr(gc), 0, _ptr(vs), _stream(dev))
+            gs, gc = gs.t(), gc.t()
+        else:
+            r = mpc.solve_batch_vjp(st.numpy(), cf.contiguous().numpy(), traj.numpy(), mult.numpy(),
+                                    *[None if v is None else v.numpy() for v in g])
+            gs, gc = torch.from_numpy(r["grad_state6"]), torch.from_numpy(r["grad_coeffs"])
+        # the derivative exists only at a converged solution
+        bad = ~((status == 0) | (status == 1))
+        gs = gs.masked_fill(bad[:, None], float("nan"))
+        gc = gc.masked_fill(bad[:, None], float("nan"))
+        if ctx.shared:
+            gc = gc.sum(0)
+        return None, gs.to(ctx.dtypes[0]), gc.to(ctx.dtypes[1])
+
+
+def solve(mpc, states, coeffs):
+    """Differentiable batched solve on the MPC handle `mpc`: states (B, 6), coeffs (B, ncoef) or (ncoef,) shared by all
+    problems, torch tensors on the CPU or on the handle's CUDA device.  Returns (out8 (B, 8), traj (B, 8N-2), obj (B,),
+    status (B,) int32, not differentiable).  Backpropagating into states / coeffs runs one adjoint solve
+    (MPC.solve_batch_vjp); problems whose status is not 0 or 1 get NaN gradients.  For gradients w.r.t. the cost
+    parameters call MPC.solve_batch_vjp(..., want_params=True) directly."""
+    return _Solve.apply(mpc, states, coeffs)

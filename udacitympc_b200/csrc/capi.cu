@@ -55,6 +55,7 @@ struct b200mpc_handle {
   cudaStream_t stream = nullptr;
   DevBuf ws, in_aos, out_aos, traj_soa, traj_aos, obj, status, iters, misc0, misc3;
   DevBuf guess_aos, guess_soa, mult_soa, mult_aos;   // b200mpc_solve_batch_warm: x_init | mult_init rows and columns, mult
+  DevBuf vjp_aos, vjp_soa, vjp_io;   // b200mpc_solve_batch_vjp: traj | mult | g_traj rows and columns, the per-problem rest
   bool timing_on = false;                                    // b200mpc_set_timing: measurement only, off by default
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timing;   // around every solve while timing_on
   cudaEvent_t done = nullptr;   // recorded after every solve: the next solve on this handle (any stream) waits for it
@@ -244,6 +245,40 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const SolveIO& io, cudaStre
   return rc;
 }
 
+// One adjoint launch (b200mpc_solve_batch_vjp*) on stream s.  It uses the handle's workspace, so it is ordered like a plain
+// solve in timed_solve: after everything queued on this handle, pipelined tails included, and before the next call.
+int run_vjp(b200mpc_handle* h, const VjpIO& io, cudaStream_t s) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (s != nullptr && s != cudaStreamLegacy) { if (cudaStreamIsCapturing(s, &cap) != cudaSuccess) { cudaGetLastError(); cap = cudaStreamCaptureStatusNone; } }
+  const bool caller_captures = cap != cudaStreamCaptureStatusNone;
+  const size_t need = solve_workspace_doubles(h->P.N, io.B) * sizeof(double);
+  if (caller_captures && h->ws.cap < need)
+    return fail(B200MPC_ERR_ARG, "the stream is being captured and the workspace would have to grow: run one solve of this size first");
+  for (int k = 0; k < h->pipe_depth; ++k)
+    if (h->tail_free_valid[k]) CU(cudaStreamWaitEvent(s, h->tail_free[k], 0));
+  if (h->main_free_valid) CU(cudaStreamWaitEvent(s, h->main_free, 0));
+  if (h->ws.cap < need && h->pipe_calls) CU(cudaDeviceSynchronize());
+  CU(h->ws.ensure(need));
+  if (!caller_captures && h->done_valid) CU(cudaStreamWaitEvent(s, h->done, 0));
+  CU(launch_vjp(h->P, io, h->ws.as<double>(), s));
+  h->launches += 1;
+  if (!caller_captures) {
+    CU(cudaEventRecord(h->done, s));
+    h->done_valid = true;
+  }
+  return 0;
+}
+
+int check_vjp_args(const b200mpc_handle* h, int B, const void* st, const void* cf, int ncoef, const void* traj, const void* mult,
+                   const void* g_out8, const void* g_traj, const void* g_obj) {
+  if (!h) return fail(B200MPC_ERR_ARG, "null handle");
+  if (B <= 0) return fail(B200MPC_ERR_ARG, "vjp: B must be positive");
+  if (ncoef < 2 || ncoef > B200MPC_MAX_COEFFS) return fail(B200MPC_ERR_ARG, "ncoef must be in [2, 4] (polynomial degree 1..3)");
+  if (!st || !cf || !traj || !mult) return fail(B200MPC_ERR_ARG, "vjp: null state6 / coeffs / traj / mult");
+  if (!g_out8 && !g_traj && !g_obj) return fail(B200MPC_ERR_ARG, "vjp: no incoming gradient (g_out8, g_traj and g_obj are all null)");
+  return 0;
+}
+
 }  // namespace
 
 namespace {
@@ -383,7 +418,7 @@ void b200mpc_destroy(b200mpc_handle* h) {
   }
   h->tail_ws.release();
   DevBuf* bufs[] = {&h->ws, &h->in_aos, &h->out_aos, &h->traj_soa, &h->traj_aos, &h->obj, &h->status, &h->iters, &h->misc0, &h->misc3,
-                    &h->guess_aos, &h->guess_soa, &h->mult_soa, &h->mult_aos};
+                    &h->guess_aos, &h->guess_soa, &h->mult_soa, &h->mult_aos, &h->vjp_aos, &h->vjp_soa, &h->vjp_io};
   for (DevBuf* b : bufs) b->release();
   if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
@@ -588,6 +623,65 @@ int b200mpc_solve_batch_warm(b200mpc_handle* h, int B, const double* state6, con
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
   CU(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+int b200mpc_solve_batch_vjp_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                   const double* d_traj, const double* d_mult, const double* d_g_out8, const double* d_g_traj,
+                                   const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
+                                   int* d_status, void* stream) {
+  if (int rc = check_vjp_args(h, B, d_state6, d_coeffs, ncoef, d_traj, d_mult, d_g_out8, d_g_traj, d_g_obj)) return rc;
+  CU(cudaSetDevice(h->device));
+  VjpIO io;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 0;
+  io.state6 = d_state6; io.coeffs = d_coeffs; io.traj = d_traj; io.mult = d_mult;
+  io.g_out8 = d_g_out8; io.g_traj = d_g_traj; io.g_obj = d_g_obj;
+  io.grad_state6 = d_grad_state6; io.grad_coeffs = d_grad_coeffs; io.grad_params = d_grad_params; io.status = d_status;
+  return run_vjp(h, io, stream ? (cudaStream_t)stream : h->stream);
+}
+
+// Host buffers: state6 / coeffs / g_out8 / g_obj and the outputs are read and written per problem by the kernel (io_aos = 1);
+// traj / mult / g_traj go through the tiled transposes.
+int b200mpc_solve_batch_vjp(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* traj,
+                            const double* mult, const double* g_out8, const double* g_traj, const double* g_obj,
+                            double* grad_state6, double* grad_coeffs, double* grad_params, int* status) {
+  if (int rc = check_vjp_args(h, B, state6, coeffs, ncoef, traj, mult, g_out8, g_traj, g_obj)) return rc;
+  CU(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  const size_t nb = (size_t)B, nv = 8 * (size_t)h->P.N - 2, nm = 10 * (size_t)h->P.N - 4;
+  const size_t nrows = nv + nm + (g_traj ? nv : 0);
+  CU(h->vjp_aos.ensure(nb * nrows * sizeof(double)));
+  CU(h->vjp_soa.ensure(nb * nrows * sizeof(double)));
+  // per problem: g_out8 (8) | g_obj (1) | grad_state6 (6) | grad_coeffs (ncoef) | grad_params (8)
+  CU(h->vjp_io.ensure(nb * (23 + ncoef) * sizeof(double)));
+  CU(h->status.ensure(nb * sizeof(int)));
+  SolveIO in;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &in)) return rc;
+  double *ga = h->vjp_aos.as<double>(), *gs = h->vjp_soa.as<double>(), *d = h->vjp_io.as<double>();
+  const double* rows[3] = {traj, mult, g_traj};
+  const size_t len[3] = {nv, nm, nv};
+  size_t off = 0;
+  for (int i = 0; i < 3; ++i) {
+    if (!rows[i]) continue;
+    CU(cudaMemcpyAsync(ga + nb * off, rows[i], nb * len[i] * sizeof(double), cudaMemcpyHostToDevice, s));
+    CU(launch_aos_to_soa(ga + nb * off, gs + nb * off, B, (int)len[i], s));
+    h->launches += 1;
+    off += len[i];
+  }
+  if (g_out8) CU(cudaMemcpyAsync(d, g_out8, nb * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
+  if (g_obj) CU(cudaMemcpyAsync(d + nb * 8, g_obj, nb * sizeof(double), cudaMemcpyHostToDevice, s));
+  VjpIO io;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 1;
+  io.state6 = in.state6; io.coeffs = in.coeffs; io.traj = gs; io.mult = gs + nb * nv;
+  io.g_out8 = g_out8 ? d : nullptr; io.g_traj = g_traj ? gs + nb * (nv + nm) : nullptr; io.g_obj = g_obj ? d + nb * 8 : nullptr;
+  io.grad_state6 = d + nb * 9; io.grad_coeffs = d + nb * 15; io.grad_params = d + nb * (15 + ncoef);
+  io.status = h->status.as<int>();
+  if (int rc = run_vjp(h, io, s)) return rc;
+  if (grad_state6) CU(cudaMemcpyAsync(grad_state6, io.grad_state6, nb * 6 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (grad_coeffs) CU(cudaMemcpyAsync(grad_coeffs, io.grad_coeffs, nb * ncoef * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (grad_params) CU(cudaMemcpyAsync(grad_params, io.grad_params, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (status) CU(cudaMemcpyAsync(status, h->status.p, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
   return 0;
 }
 

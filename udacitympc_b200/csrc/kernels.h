@@ -75,6 +75,20 @@ cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double*
 cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const TailCtx& tail, const SolveConfig& cfg,
                               cudaStream_t stream, long long* n_launches);
 
+// Adjoint sensitivities of B returned solutions (Solver::vjp), one launch (mpc_vjp_kernel) in workspace region 0 of ws
+// (solve_workspace_doubles(N, B) doubles).  io_aos = 0: state6 [6][B], coeffs [ncoef][B], g_out8 [8][B],
+// grad_state6 [6][B], grad_coeffs [ncoef][B], grad_params [8][B]; io_aos = 1: the same per problem ([B][k]).  Always
+// field-major: traj, g_traj [8N-2][B], mult [10N-4][B].  g_out8, g_traj, g_obj [B], the gradients and status [B] may be
+// null.
+struct VjpIO {
+  int B = 0, ncoef = 0, io_aos = 0;
+  const double *state6 = nullptr, *coeffs = nullptr, *traj = nullptr, *mult = nullptr;
+  const double *g_out8 = nullptr, *g_traj = nullptr, *g_obj = nullptr;
+  double *grad_state6 = nullptr, *grad_coeffs = nullptr, *grad_params = nullptr;
+  int* status = nullptr;
+};
+cudaError_t launch_vjp(const Params& P, const VjpIO& io, double* ws, cudaStream_t stream);
+
 // K6 batch I/O: [B][K] <-> [K][B]
 cudaError_t launch_aos_to_soa(const double* in, double* out, int B, int K, cudaStream_t stream);
 cudaError_t launch_soa_to_aos(const double* in, double* out, int B, int K, cudaStream_t stream);

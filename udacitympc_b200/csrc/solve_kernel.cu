@@ -602,6 +602,41 @@ cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const T
 }
 
 // ---------------------------------------------------------------------------------------------
+// Adjoint sensitivities of returned solutions (Solver::vjp): one thread per problem, workspace region 0 (slot = problem).
+// state6 / coeffs / g_out8 / the three gradients in the layout io_aos selects, traj / mult / g_traj field-major.
+__global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__ Params P, const __grid_constant__ VjpIO A, double* ws) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= A.B) return;
+  const size_t nb = (size_t)A.B, bb = (size_t)b;
+  auto at = [&](int k, int n) { return A.io_aos ? bb * n + k : (size_t)k * nb + bb; };   // element k of n of problem b
+  Solver<32> S(P, slot_base(P, ws, b), b & 31);
+  double s0[6], cf[kMaxCoef], gs6[6], gcf[kMaxCoef], gpar[8];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) s0[k] = A.state6[at(k, 6)];
+#pragma unroll
+  for (int i = 0; i < kMaxCoef; ++i) cf[i] = i < A.ncoef ? A.coeffs[at(i, A.ncoef)] : 0.0;
+  S.set_coeffs(cf, kMaxCoef);
+  const int st = S.vjp(s0, A.traj + b, nb, A.mult + b, nb, A.g_out8 ? A.g_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb,
+                       A.g_traj ? A.g_traj + b : nullptr, nb, A.g_obj ? A.g_obj[b] : 0.0, gs6, gcf, gpar);
+  if (A.grad_state6)
+#pragma unroll
+    for (int k = 0; k < 6; ++k) A.grad_state6[at(k, 6)] = gs6[k];
+  if (A.grad_coeffs)
+#pragma unroll
+    for (int i = 0; i < kMaxCoef; ++i)
+      if (i < A.ncoef) A.grad_coeffs[at(i, A.ncoef)] = gcf[i];
+  if (A.grad_params)
+#pragma unroll
+    for (int i = 0; i < 8; ++i) A.grad_params[at(i, 8)] = gpar[i];
+  if (A.status) A.status[b] = st;
+}
+cudaError_t launch_vjp(const Params& P, const VjpIO& io, double* ws, cudaStream_t stream) {
+  if (io.B <= 0) return cudaSuccess;
+  mpc_vjp_kernel<<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
+  return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------
 // FP64 peak: 8 independent dependent-FMA chains per thread.
 __global__ void __launch_bounds__(256) fp64_peak_kernel(double* sink, int iters) {
   double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
