@@ -151,6 +151,25 @@ int b200mpc_solve_batch_warm_device(b200mpc_handle* h, int B, const double* d_st
                                     const double* d_x_init, const double* d_mult_init, double mu_init, double* d_out8,
                                     double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters, void* stream);
 
+/* b200mpc_solve_batch_warm with per-problem cost parameters.  NOT reference behaviour: the reference's cost has one
+ * ref_v and one set of weights (MPC.cpp:14-31, 57-76); here a batch of a fleet's vehicles, or of scenes whose weights a
+ * network predicts, is solved in one call with each problem's own values.
+ *   cost8  B x 8 per problem: ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da (the order of grad_params of
+ *          b200mpc_solve_batch_vjp), or NULL for the handle's values (then this is b200mpc_solve_batch_warm).  N, dt, Lf,
+ *          the bounds, tol and max_iter stay the handle's.  Weights are not range-checked, like the handle's.
+ * A non-finite entry of a problem's cost8 row gives that problem status -13 (Invalid_Number_Detected), 0 iterations.
+ * cost8 equal to the handle's values in every row gives what b200mpc_solve_batch_warm gives, bit for bit.  The other
+ * arguments and errors are those of b200mpc_solve_batch_warm. */
+int b200mpc_solve_batch_cost(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                             const double* x_init, const double* mult_init, double mu_init, double* out8, double* traj,
+                             double* mult, double* obj, int* status, int* iters);
+/* Same on device buffers, field-major like b200mpc_solve_batch_warm_device: d_cost8[k*B+b].  Pipelined solves
+ * (b200mpc_set_pipeline) accept it like b200mpc_solve_batch_device. */
+int b200mpc_solve_batch_cost_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                    const double* d_cost8, const double* d_x_init, const double* d_mult_init, double mu_init,
+                                    double* d_out8, double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters,
+                                    void* stream);
+
 /* Adjoint sensitivities (vector-Jacobian product) of B solutions: the derivative of a scalar loss L(out8, traj, obj) of
  * each problem's solution w.r.t. its initial state, its reference polynomial and the handle's cost parameters, by the
  * implicit-function theorem at the returned primal-dual point (the differentiable-MPC layer; Ipopt's sIPOPT does the
@@ -178,6 +197,22 @@ int b200mpc_solve_batch_vjp_device(b200mpc_handle* h, int B, const double* d_sta
                                    const double* d_traj, const double* d_mult, const double* d_g_out8, const double* d_g_traj,
                                    const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
                                    int* d_status, void* stream);
+
+/* b200mpc_solve_batch_vjp of solutions of b200mpc_solve_batch_cost: the derivative is taken at each problem's own cost
+ * parameters.  NOT reference behaviour.
+ *   cost8        B x 8 (ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da) the solve used, or NULL for the handle's
+ *                values (then this is b200mpc_solve_batch_vjp)
+ *   grad_params  B x 8 in the same order: dL/d(cost8 row) of each problem
+ * A non-finite entry of a problem's cost8 row gives that problem status -13 and NaN gradients.  The other arguments and
+ * errors are those of b200mpc_solve_batch_vjp. */
+int b200mpc_solve_batch_vjp_cost(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                                 const double* traj, const double* mult, const double* g_out8, const double* g_traj,
+                                 const double* g_obj, double* grad_state6, double* grad_coeffs, double* grad_params, int* status);
+/* Same on device buffers, field-major like b200mpc_solve_batch_vjp_device: d_cost8[k*B+b].  Exactly one kernel launch. */
+int b200mpc_solve_batch_vjp_cost_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                        const double* d_cost8, const double* d_traj, const double* d_mult, const double* d_g_out8,
+                                        const double* d_g_traj, const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs,
+                                        double* d_grad_params, int* d_status, void* stream);
 
 /* Warm start for b200mpc_closed_loop_batch (SURVEY 8f; NOT reference behaviour: the reference cold-starts every call,
  * MPC.cpp:167-177, and so does this library unless enabled here).  When enabled, every step after the first starts from

@@ -40,6 +40,12 @@ SYMBOLS = {
                                                 _dp, _dp, _ip, _ip]),
     "b200mpc_solve_batch_warm_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, ctypes.c_double, _vp,
                                                        _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200mpc_solve_batch_cost": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, ctypes.c_double, _dp,
+                                                _dp, _dp, _dp, _ip, _ip]),
+    "b200mpc_solve_batch_cost_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, _vp, ctypes.c_double,
+                                                       _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200mpc_solve_batch_vjp_cost": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int] + [_dp] * 9 + [_ip]),
+    "b200mpc_solve_batch_vjp_cost_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 11),
     "b200mpc_solve_batch_vjp": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
                                                _ip]),
     "b200mpc_solve_batch_vjp_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 10),
@@ -124,8 +130,18 @@ def default_params(**kw):
     return p
 
 
-# the parameters b200mpc_solve_batch_vjp differentiates, in the order of its grad_params
+# the parameters b200mpc_solve_batch_vjp differentiates, in the order of its grad_params (and of a cost8 row)
 PARAM_NAMES = ("ref_v", "w_cte", "w_epsi", "w_v", "w_delta", "w_a", "w_ddelta", "w_da")
+
+
+def _cost8(cost_params, B):
+    """(B, 8) or (8,) broadcast, in PARAM_NAMES order -> the (B, 8) float64 rows b200mpc_solve_batch_cost takes."""
+    c = _f64(cost_params)
+    if c.ndim == 1:
+        c = np.broadcast_to(c, (B, c.size))
+    if c.shape != (B, 8):
+        raise ValueError(f"cost_params must be (B, 8) or (8,) in the order {PARAM_NAMES}")
+    return np.ascontiguousarray(c)
 
 
 class MPC:
@@ -201,13 +217,17 @@ class MPC:
         return [float(v) for v in r["out8"][0]]
 
     # -- batched host-buffer call
-    def solve_batch(self, states, coeffs, want_traj=False, x_init=None, mult_init=None, mu_init=1e-4, want_mult=False):
+    def solve_batch(self, states, coeffs, want_traj=False, x_init=None, mult_init=None, mu_init=1e-4, want_mult=False,
+                    cost_params=None):
         """states (B,6), coeffs (B,ncoef) or (ncoef,) shared by all problems.  Returns dict(out8 (B,8), cost (B,),
         status (B,), iters (B,), traj (B,8N-2) if requested, mult (B,10N-4) if requested).
 
         Warm start (not reference behaviour, b200mpc_solve_batch_warm): x_init (B,8N-2) in the layout of traj and
         optionally mult_init (B,10N-4) in the layout of mult start the solve there with the barrier parameter mu_init;
-        shift_solution() turns one receding-horizon step's traj / mult into the next step's start."""
+        shift_solution() turns one receding-horizon step's traj / mult into the next step's start.
+
+        Per-problem costs (not reference behaviour, b200mpc_solve_batch_cost): cost_params (B,8) or (8,) shared, in the
+        order PARAM_NAMES, replaces the handle's ref_v and weights problem by problem; None uses the handle's."""
         states = _f64(states)
         if states.ndim != 2 or states.shape[1] != 6:
             raise ValueError("states must be (B, 6)")
@@ -223,7 +243,16 @@ class MPC:
         status = np.empty(B, dtype=np.int32)
         iters = np.empty(B, dtype=np.int32)
         traj = np.empty((B, self.num_vars)) if want_traj else None
-        if x_init is None and mult_init is None and not want_mult:
+        if cost_params is not None:
+            x_init = None if x_init is None else _f64(x_init, (B, self.num_vars))
+            mult_init = None if mult_init is None else _f64(mult_init, (B, self.num_mults))
+            mult = np.empty((B, self.num_mults)) if want_mult else None
+            _check(self._lib.b200mpc_solve_batch_cost(
+                self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(_cost8(cost_params, B)),
+                None if x_init is None else _ptr(x_init), None if mult_init is None else _ptr(mult_init), float(mu_init),
+                _ptr(out8), _ptr(traj) if want_traj else None, _ptr(mult) if want_mult else None, _ptr(cost),
+                status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
+        elif x_init is None and mult_init is None and not want_mult:
             _check(self._lib.b200mpc_solve_batch(self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(out8),
                                                  _ptr(traj) if want_traj else None, _ptr(cost),
                                                  status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
@@ -260,12 +289,23 @@ class MPC:
                                                          d_mult or None, d_obj or None, d_status or None, d_iters or None,
                                                          stream or None))
 
-    def solve_batch_vjp(self, states, coeffs, traj, mult, g_out8=None, g_traj=None, g_obj=None, want_params=False):
+    def solve_batch_cost_device(self, B, d_state6, d_coeffs, ncoef, d_cost8, d_x_init=0, d_mult_init=0, mu_init=1e-4,
+                                d_out8=0, d_traj=0, d_mult=0, d_obj=0, d_status=0, d_iters=0, stream=0):
+        """Raw device-pointer solve with per-problem costs (integers, 0 = none), field-major buffers: d_cost8 [8][B] in
+        the order PARAM_NAMES (0 = the handle's values); asynchronous on `stream`.  See b200mpc_solve_batch_cost_device."""
+        _check(self._lib.b200mpc_solve_batch_cost_device(self._h, B, d_state6, d_coeffs, ncoef, d_cost8 or None,
+                                                         d_x_init or None, d_mult_init or None, float(mu_init), d_out8,
+                                                         d_traj or None, d_mult or None, d_obj or None, d_status or None,
+                                                         d_iters or None, stream or None))
+
+    def solve_batch_vjp(self, states, coeffs, traj, mult, g_out8=None, g_traj=None, g_obj=None, want_params=False,
+                        cost_params=None):
         """Adjoint sensitivities of solutions (b200mpc_solve_batch_vjp; not reference behaviour): for a loss L with the
         incoming gradients g_out8 (B,8), g_traj (B,8N-2), g_obj (B,) -- any of them None, not all -- returns
         dict(grad_state6 (B,6), grad_coeffs (B,ncoef) per problem, status (B,), and grad_params (B,8) in the order
         PARAM_NAMES if want_params).  traj (B,8N-2) and mult (B,10N-4) must be a converged solution of (states, coeffs)
-        on a handle with these params, as solve_batch(..., want_traj=True, want_mult=True) returns it."""
+        on a handle with these params, as solve_batch(..., want_traj=True, want_mult=True) returns it.  cost_params (B,8)
+        or (8,): the per-problem costs the solve used (b200mpc_solve_batch_vjp_cost); grad_params is w.r.t. them."""
         states = _f64(states)
         if states.ndim != 2 or states.shape[1] != 6:
             raise ValueError("states must be (B, 6)")
@@ -283,10 +323,15 @@ class MPC:
         g_obj = None if g_obj is None else _f64(g_obj, (B,))
         gs = np.empty((B, 6)); gc = np.empty((B, ncoef)); gp = np.empty((B, 8)) if want_params else None
         status = np.empty(B, dtype=np.int32)
-        _check(self._lib.b200mpc_solve_batch_vjp(
-            self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(traj), _ptr(mult), None if g_out8 is None else _ptr(g_out8),
-            None if g_traj is None else _ptr(g_traj), None if g_obj is None else _ptr(g_obj), _ptr(gs), _ptr(gc),
-            None if gp is None else _ptr(gp), status.ctypes.data_as(_ip)))
+        grads = (None if g_out8 is None else _ptr(g_out8), None if g_traj is None else _ptr(g_traj),
+                 None if g_obj is None else _ptr(g_obj), _ptr(gs), _ptr(gc), None if gp is None else _ptr(gp),
+                 status.ctypes.data_as(_ip))
+        if cost_params is None:
+            _check(self._lib.b200mpc_solve_batch_vjp(self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(traj), _ptr(mult),
+                                                     *grads))
+        else:
+            _check(self._lib.b200mpc_solve_batch_vjp_cost(self._h, B, _ptr(states), _ptr(coeffs), ncoef,
+                                                          _ptr(_cost8(cost_params, B)), _ptr(traj), _ptr(mult), *grads))
         r = dict(grad_state6=gs, grad_coeffs=gc, status=status)
         if want_params:
             r["grad_params"] = gp
@@ -300,6 +345,15 @@ class MPC:
                                                         d_g_out8 or None, d_g_traj or None, d_g_obj or None,
                                                         d_grad_state6 or None, d_grad_coeffs or None, d_grad_params or None,
                                                         d_status or None, stream or None))
+
+    def solve_batch_vjp_cost_device(self, B, d_state6, d_coeffs, ncoef, d_cost8, d_traj, d_mult, d_g_out8=0, d_g_traj=0,
+                                    d_g_obj=0, d_grad_state6=0, d_grad_coeffs=0, d_grad_params=0, d_status=0, stream=0):
+        """Raw device-pointer VJP with per-problem costs (integers, 0 = none), field-major buffers, d_cost8 [8][B]; one
+        kernel launch, asynchronous on `stream`.  See b200mpc_solve_batch_vjp_cost_device."""
+        _check(self._lib.b200mpc_solve_batch_vjp_cost_device(self._h, B, d_state6, d_coeffs, ncoef, d_cost8 or None, d_traj,
+                                                             d_mult, d_g_out8 or None, d_g_traj or None, d_g_obj or None,
+                                                             d_grad_state6 or None, d_grad_coeffs or None,
+                                                             d_grad_params or None, d_status or None, stream or None))
 
     def wait(self):
         """Waits for everything queued on this handle's own stream (b200mpc_solve_batch_async calls)."""

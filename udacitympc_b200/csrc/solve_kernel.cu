@@ -14,6 +14,8 @@
 // iterating once the compacted batch fits one of its waves (or after the last round) and solves small batches on its own.
 // mpc_fused_kernel loops the three thread-per-problem sweeps in one launch (comparison / fallback for horizons whose
 // per-stage scratch does not fit the cooperative kernel's shared memory).
+#include <type_traits>
+
 #include "kernels.h"
 #include "mpc_coop.cuh"
 
@@ -93,6 +95,14 @@ struct SolveArgs {
   double* mult;           // [10N-4][B] or null (last step)
 };
 
+// Per-problem cost parameters (b200mpc_solve_batch_cost*): the kernel instances with COST = true take this parameter
+// block, every other instance SolveArgs, whose layout (and so the machine code of those instances) does not change.
+struct CostArgs : SolveArgs {
+  const double* cost8;    // [8][B] ([B][8] with io_aos) or null: ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da
+};
+template <bool COST>
+using ArgsT = typename std::conditional<COST, CostArgs, SolveArgs>::type;
+
 __device__ __forceinline__ double* slot_base(const Params& P, double* ws, int slot) {
   return ws + (size_t)(slot >> 5) * (size_t)workspace_doubles_per_problem(P.N) * 32 + (slot & 31);
 }
@@ -127,6 +137,33 @@ __device__ __forceinline__ void load_state6(const SolveArgs& A, int b, double* s
   for (int k = 0; k < 6; ++k)
     s0[k] = A.step == 0 ? A.state6[A.io_aos ? (size_t)b * 6 + k : (size_t)k * A.B + b] : A.out8[out8_index(A, A.step - 1, k, b)];
 }
+// Problem b's row of cost8 (layout io_aos) over the eight cost fields of Q, which is a copy of the handle's Params.  The
+// row is indexed by problem, not by workspace slot, like the coefficients, so compaction and hand-offs need nothing.
+// False: a non-finite entry (Q is left unchanged then).
+__device__ __forceinline__ bool cost_row(const double* cost8, int io_aos, int B, int b, Params& Q) {
+  double c[8];
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    c[k] = cost8[io_aos ? (size_t)b * 8 + k : (size_t)k * B + b];
+    ok &= fabs(c[k]) <= DBL_MAX;
+  }
+  if (ok) {
+    Q.ref_v = c[0]; Q.w_cte = c[1]; Q.w_epsi = c[2]; Q.w_v = c[3];
+    Q.w_delta = c[4]; Q.w_a = c[5]; Q.w_ddelta = c[6]; Q.w_da = c[7];
+  }
+  return ok;
+}
+// COST instances: the solver of problem b runs on Q with b's cost row.  A non-finite row makes ref_v NaN, so the
+// objective at the start point is NaN and the start-point check stops the problem with status -13 and 0 iterations
+// (Solver::init_finish / guess_check), as for a non-finite x_init; the later sweeps never see it.
+template <bool COST>
+__device__ __forceinline__ void load_cost(const ArgsT<COST>& A, int b, Params& Q) {
+  if constexpr (COST) {
+    if (!cost_row(A.cost8, A.io_aos, A.B, b, Q)) Q.ref_v = NAN;
+  }
+}
+
 // Warm-start I/O (SolveArgs::x_init / mult_init / mult) is compiled only into the WIO = true instance of each kernel that
 // starts or finishes problems, and that instance is launched only when a call uses it: a call without it runs kernels
 // that do not carry its code (the factor and step sweeps: the same machine code as without the feature).
@@ -151,13 +188,15 @@ __device__ __forceinline__ void count_live(int* counter) {
 }
 
 // ---- per-pass kernels ---------------------------------------------------------------------------------------
-template <bool WIO>
-__global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
+template <bool WIO, bool COST>
+__global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
   const int b = A.b0 + blockIdx.x * blockDim.x + threadIdx.x;   // always launched on the uncompacted batch
   if (b >= A.b1) return;
   if (b == A.b0 && A.desc)
     for (int k = 0; k < kDescInts; ++k) A.desc[k] = 0;
-  Solver<32> S(P, slot_base(P, A.ws, b), b & 31);
+  Params Q = P;
+  load_cost<COST>(A, b, Q);
+  Solver<32> S(COST ? Q : P, slot_base(P, A.ws, b), b & 31);
   double s0[6], cf[kMaxCoef];
   load_state6(A, b, s0);
   load_coeffs(A, b, cf);
@@ -168,13 +207,15 @@ __global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant_
   if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);   // invalid number at the starting point
 }
 
-template <bool WIO>
-__global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
+template <bool WIO, bool COST>
+__global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
-  Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
+  Params Q = P;
+  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
   if (S.load_phase() != PH_FACTOR) return;
+  load_cost<COST>(A, b, Q);
   __shared__ double stage[2 * kStageVals * kBlock];   // [buffer][value][thread]
   S.sb = stage + threadIdx.x; S.sbs = kBlock;
   load_coeffs(A, b, S.cf);
@@ -185,27 +226,32 @@ __global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const
   }
 }
 
-__global__ void __launch_bounds__(kBlock, kFwdBlocks) mpc_forward_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
+template <bool COST>
+__global__ void __launch_bounds__(kBlock, kFwdBlocks) mpc_forward_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
-  Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
+  Params Q = P;
+  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
   if (S.load_phase() != PH_FORWARD) return;
+  load_cost<COST>(A, b, Q);
   load_coeffs(A, b, S.cf);
   S.kernel_forward();
 }
 
-template <bool WIO>
-__global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A) {
+template <bool WIO, bool COST>
+__global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
-  Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
+  Params Q = P;
+  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
   const int ph = S.load_phase();
   if (ph != PH_STEP) {
     if (A.count_live && ph != PH_DONE) count_live(A.desc + kLive);
     return;
   }
+  load_cost<COST>(A, b, Q);
   double carry[kCarry];
   S.cr = carry; S.cs = 1;
   __shared__ double stage[2 * kStepStageVals * kBlock];   // [buffer][value][thread]
@@ -275,12 +321,14 @@ __global__ void mpc_tail_reset_kernel(int* t_desc) {
 }
 
 // ---- fused kernel: finishes whatever is still active (fresh == 1: starts from the inputs) ---------------------
-template <bool WIO>
-__global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A, int fresh) {
+template <bool WIO, bool COST>
+__global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A, int fresh) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws, false)) return;
-  Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
+  Params Q = P;
+  load_cost<COST>(A, b, Q);
+  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
   double carry[kCarry];
   S.cr = carry; S.cs = 1;
   load_coeffs(A, b, S.cf);
@@ -313,8 +361,8 @@ struct DevExec {
 // take_below > 0: conditional hand-over after a round -- the kernel acts only once the batch has been compacted to at
 // most take_below occupied slots (two waves of the cooperative kernel); from then on the sweeps of later rounds find
 // nothing to do
-template <bool WIO>
-__global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ Params P, const __grid_constant__ SolveArgs A, int fresh,
+template <bool WIO, bool COST>
+__global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A, int fresh,
                                                        int warps_per_block, int doubles_per_warp, int take_below) {
   extern __shared__ double coop_smem[];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -332,7 +380,9 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
     int slot, b;
     double* ws;
     if (!locate(A, idx, slot, b, ws, false)) return;
-    Solver<32> S(P, slot_base(P, ws, slot), slot & 31);
+    Params Q = P;
+    load_cost<COST>(A, b, Q);
+    Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
     load_coeffs(A, b, S.cf);
     CoopSolver<32, DevExec> C(S, st, pub, DevExec{lane});
     if (fresh) {
@@ -358,8 +408,9 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
 constexpr size_t kCoopSmemMax = 200 * 1024;   // dynamic shared memory of one cooperative block, at most
 // per-device, once (b200mpc_create)
 cudaError_t solver_prepare_device() {
-  cudaError_t e = cudaFuncSetAttribute(mpc_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  cudaError_t e = cudaFuncSetAttribute(mpc_coop_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
   return e;
 }
 
@@ -394,36 +445,45 @@ static int coop_resident_warps(int N) {
 // the kernels' parameter block for problems [b0, b1) of the B-problem batch in workspace L (desc: the compaction state
 // of these problems, or null: no compaction); warm_mu > 0: closed-loop steps after the first start from the shifted
 // previous solution with this barrier parameter
-static SolveArgs solve_args(int B, int steps, const SolveIO& io, const WsLayout& L, int* desc, int b0, int b1, double warm_mu) {
-  SolveArgs A{};
+static CostArgs solve_args(int B, int steps, const SolveIO& io, const WsLayout& L, int* desc, int b0, int b1, double warm_mu) {
+  CostArgs A{};
   A.B = B; A.steps = steps; A.ncoef = io.ncoef; A.io_aos = io.io_aos ? 1 : 0; A.b0 = b0; A.b1 = b1;
   A.warm = warm_mu > 0.0 ? 1 : 0; A.mu_warm = warm_mu;
   A.state6 = io.state6; A.coeffs = io.coeffs;
   A.ws = L.ws0; A.ws1 = L.ws1; A.map0 = L.map0; A.map1 = L.map1; A.desc = desc;
   A.out8 = io.out8; A.traj = io.traj; A.obj = io.obj; A.status = io.status; A.iters = io.iters;
   A.x_init = io.x_init; A.mult_init = io.mult_init; A.mu_init = io.mu_init; A.mult = io.mult;
+  A.cost8 = io.cost8;
   return A;
 }
 
 static int sweep_grid(const SolveArgs& A) { return (A.b1 - A.b0 + kBlock - 1) / kBlock; }
-// the call reads a start point or writes multipliers: the WIO = true kernel instances
+// the call reads a start point or writes multipliers: the WIO = true kernel instances.  A call with per-problem costs
+// runs the <true, true> instances (null x_init / mult do nothing there); the others get the SolveArgs part of A.
 static bool warm_io(const SolveArgs& A) { return A.x_init != nullptr || A.mult != nullptr; }
-static void launch_init(const Params& P, const SolveArgs& A, cudaStream_t stream, long long* n) {
-  if (warm_io(A)) mpc_init_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  else mpc_init_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+static void launch_init(const Params& P, const CostArgs& A, cudaStream_t stream, long long* n) {
+  if (A.cost8) mpc_init_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else if (warm_io(A)) mpc_init_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else mpc_init_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
   *n += 1;
 }
 
 // The launch helpers add one to *n per kernel they launch.  launch_round: one round of the thread-per-problem sweeps;
 // count_live: the step kernel counts the unfinished problems for the compaction attempt that follows
-static void launch_round(const Params& P, const SolveArgs& A, bool count_live, cudaStream_t stream, long long* n) {
-  SolveArgs As = A;
+static void launch_round(const Params& P, const CostArgs& A, bool count_live, cudaStream_t stream, long long* n) {
+  CostArgs As = A;
   As.count_live = count_live ? 1 : 0;
-  if (warm_io(A)) mpc_factor_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  else mpc_factor_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  mpc_forward_kernel<<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  if (warm_io(A)) mpc_step_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
-  else mpc_step_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  if (A.cost8) {
+    mpc_factor_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    mpc_forward_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    mpc_step_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  } else {
+    if (warm_io(A)) mpc_factor_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    else mpc_factor_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    mpc_forward_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    if (warm_io(A)) mpc_step_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+    else mpc_step_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  }
   *n += 3;
 }
 
@@ -434,14 +494,15 @@ static void launch_repack(const Params& P, const SolveArgs& A, double max_live, 
   *n += 1;
 }
 
-static void launch_fused(const Params& P, const SolveArgs& A, int fresh, cudaStream_t stream, long long* n) {
-  if (warm_io(A)) mpc_fused_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
-  else mpc_fused_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+static void launch_fused(const Params& P, const CostArgs& A, int fresh, cudaStream_t stream, long long* n) {
+  if (A.cost8) mpc_fused_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else if (warm_io(A)) mpc_fused_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else mpc_fused_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
   *n += 1;
 }
 
 // launches the cooperative kernel if the horizon fits in shared memory (*err: the launch's error); returns false otherwise
-static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, int take_below, cudaStream_t stream, cudaError_t* err,
+static bool launch_coop(const Params& P, const CostArgs& A, int fresh, int take_below, cudaStream_t stream, cudaError_t* err,
                         long long* n) {
   const CoopShape c = coop_shape(P.N);
   if (c.warps == 0) return false;
@@ -451,8 +512,10 @@ static bool launch_coop(const Params& P, const SolveArgs& A, int fresh, int take
   const int cap = 4 * coop_resident_warps(P.N) / wpb;   // four waves; the warps stride over the rest
   if (cap > 0 && grid > cap) grid = cap;
   // no idle warps: their registers would stay allocated
-  if (warm_io(A)) mpc_coop_kernel<true><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);
-  else mpc_coop_kernel<false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, (int)coop_doubles_per_warp(P.N), take_below);
+  const int dpw = (int)coop_doubles_per_warp(P.N);
+  if (A.cost8) mpc_coop_kernel<true, true><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  else if (warm_io(A)) mpc_coop_kernel<true, false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  else mpc_coop_kernel<false, false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
   *n += 1;
   *err = cudaGetLastError();
   return true;
@@ -468,7 +531,7 @@ static int handover_rounds(const Params& P, const SolveConfig& cfg) {
 }
 
 // launches every kernel of the solve of problems [b0, b1) on one stream
-static cudaError_t launch_part(const Params& P, SolveArgs A, const SolveConfig& cfg, int rounds, int take_below, cudaStream_t stream, long long* n) {
+static cudaError_t launch_part(const Params& P, CostArgs A, const SolveConfig& cfg, int rounds, int take_below, cudaStream_t stream, long long* n) {
   for (int step = 0; step < A.steps; ++step) {
     A.step = step;
     cudaError_t ce = cudaSuccess;
@@ -522,7 +585,7 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const SolveIO& io, d
   for (int p = 0; p < parts && e == cudaSuccess; ++p) {
     const int b0 = p * per, b1 = (p + 1) * per < B ? (p + 1) * per : B;
     if (b0 >= b1) continue;
-    const SolveArgs A = solve_args(B, steps, io, L, desc ? desc + p * kDescInts : nullptr, b0, b1, cfg.warm_start ? cfg.warm_mu : 0.0);
+    const CostArgs A = solve_args(B, steps, io, L, desc ? desc + p * kDescInts : nullptr, b0, b1, cfg.warm_start ? cfg.warm_mu : 0.0);
     e = launch_part(P, A, cfg, rounds, take_below, p == 0 ? stream : ss->aux[p - 1], n);
   }
   for (int p = 1; p < parts; ++p) {   // always join, also after an error, so a capture can end cleanly
@@ -546,7 +609,7 @@ cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double*
                               cudaStream_t stream, long long* n) {
   if (B <= 0) return cudaSuccess;
   const WsLayout L = ws_layout(ws, P.N, B), T = ws_layout(tail.ws, P.N, tail.slots);
-  const SolveArgs A = solve_args(B, 1, io, L, L.desc, 0, B, 0.0);
+  const CostArgs A = solve_args(B, 1, io, L, L.desc, 0, B, 0.0);
   const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P, cfg);
   mpc_tail_reset_kernel<<<1, 32, 0, stream>>>(T.desc);
   *n += 1;
@@ -568,7 +631,7 @@ cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const T
                               cudaStream_t stream, long long* n) {
   if (B <= 0) return cudaSuccess;
   const WsLayout L = ws_layout(tail.ws, P.N, tail.slots);
-  const SolveArgs A = solve_args(B, 1, io, L, L.desc, 0, tail.slots, 0.0);
+  const CostArgs A = solve_args(B, 1, io, L, L.desc, 0, tail.slots, 0.0);
   // Up to N = 50 the tail is short (the slowest problems need a few dozen iterations): a few rounds, after each of which
   // the cooperative kernel takes the rest over once it fits its resident warps, as in launch_solve.  Above that the tail
   // is long (N = 100: 2 % of the problems need more than 100 iterations, the slowest about 1000) and the tails of many
@@ -603,18 +666,27 @@ cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const T
 
 // ---------------------------------------------------------------------------------------------
 // Adjoint sensitivities of returned solutions (Solver::vjp): one thread per problem, workspace region 0 (slot = problem).
-// state6 / coeffs / g_out8 / the three gradients in the layout io_aos selects, traj / mult / g_traj field-major.
-__global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__ Params P, const __grid_constant__ VjpIO A, double* ws) {
+// state6 / coeffs / g_out8 / the three gradients (and cost8, COST = true) in the layout io_aos selects, traj / mult /
+// g_traj field-major.
+template <bool COST>
+using VjpArgsT = typename std::conditional<COST, VjpCostIO, VjpIO>::type;
+template <bool COST>
+__global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__ Params P, const __grid_constant__ VjpArgsT<COST> A, double* ws) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= A.B) return;
   const size_t nb = (size_t)A.B, bb = (size_t)b;
   auto at = [&](int k, int n) { return A.io_aos ? bb * n + k : (size_t)k * nb + bb; };   // element k of n of problem b
-  Solver<32> S(P, slot_base(P, ws, b), b & 31);
+  Params Q = P;
+  Solver<32> S(COST ? Q : P, slot_base(P, ws, b), b & 31);
   double s0[6], cf[kMaxCoef], gs6[6], gcf[kMaxCoef], gpar[8];
 #pragma unroll
   for (int k = 0; k < 6; ++k) s0[k] = A.state6[at(k, 6)];
 #pragma unroll
   for (int i = 0; i < kMaxCoef; ++i) cf[i] = i < A.ncoef ? A.coeffs[at(i, A.ncoef)] : 0.0;
+  // a non-finite cost row: a NaN coefficient makes Solver::vjp return -13 with NaN gradients
+  if constexpr (COST) {
+    if (!cost_row(A.cost8, A.io_aos, A.B, b, Q)) cf[0] = NAN;
+  }
   S.set_coeffs(cf, kMaxCoef);
   const int st = S.vjp(s0, A.traj + b, nb, A.mult + b, nb, A.g_out8 ? A.g_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb,
                        A.g_traj ? A.g_traj + b : nullptr, nb, A.g_obj ? A.g_obj[b] : 0.0, gs6, gcf, gpar);
@@ -630,9 +702,10 @@ __global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__
     for (int i = 0; i < 8; ++i) A.grad_params[at(i, 8)] = gpar[i];
   if (A.status) A.status[b] = st;
 }
-cudaError_t launch_vjp(const Params& P, const VjpIO& io, double* ws, cudaStream_t stream) {
+cudaError_t launch_vjp(const Params& P, const VjpCostIO& io, double* ws, cudaStream_t stream) {
   if (io.B <= 0) return cudaSuccess;
-  mpc_vjp_kernel<<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
+  if (io.cost8) mpc_vjp_kernel<true><<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
+  else mpc_vjp_kernel<false><<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
   return cudaGetLastError();
 }
 
