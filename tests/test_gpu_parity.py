@@ -785,9 +785,10 @@ def test_plain_launches_and_changing_batch_sizes():
 
 
 def test_long_horizon_falls_back_to_the_thread_finisher():
-    """N = 200 does not fit the cooperative kernel's shared memory: the fused thread-per-problem kernel finishes the
-    batch.  No oracle is fast enough at this size; check the size-independent properties instead."""
-    N = 200
+    """From N = 205 on the cooperative kernel does not fit its shared memory (N = 204 is the last horizon that does, with
+    one problem per block): the fused thread-per-problem kernel finishes the batch.  No oracle is fast enough at this
+    size; check the size-independent properties instead."""
+    N = 205
     st, cf = synth.line_problems(40)
     with mp.MPC(device=0, N=N, max_iter=400) as m:
         r = m.solve_batch(st, cf, want_traj=True)

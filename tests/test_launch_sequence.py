@@ -21,7 +21,7 @@ CASES = {
     "no_compaction": (25, 4096, [("set_compaction", 0.0)], "solve", 56),
     "no_handover": (25, 4096, [("set_handover", 0, 14)], "solve", 70),
     "pipelined": (25, 16384, [("set_pipeline", 2, 1024)], "solve", 132),   # bulk 80 + tail 52
-    "long_latency": (200, 40, [], "solve", 1),                    # N = 200 does not fit the cooperative kernel
+    "long_latency": (200, 40, [], "solve", 1),                    # the cooperative kernel, one problem per block
     "long_rounds": (200, 40, [("set_solver_mode", 0, 12, 0)], "solve", 46),
 }
 

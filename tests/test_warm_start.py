@@ -227,7 +227,7 @@ def test_gpu_warm_start_fused():
 @pytest.mark.gpu
 @pytest.mark.parametrize("N,B", [(10, 4096), (50, 4096), (100, 512), (200, 40)])
 def test_gpu_warm_start_horizons(N, B):
-    """N = 200 does not fit the cooperative kernel: the fused kernel starts from the guess"""
+    """N = 200: the cooperative kernel with one problem per block starts from the guess"""
     if N == 200:
         from udacitympc_b200 import synth
         st, cf = synth.line_problems(B)
