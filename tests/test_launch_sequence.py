@@ -21,6 +21,11 @@ CASES = {
     "no_compaction": (25, 4096, [("set_compaction", 0.0)], "solve", 56),
     "no_handover": (25, 4096, [("set_handover", 0, 14)], "solve", 70),
     "pipelined": (25, 16384, [("set_pipeline", 2, 1024)], "solve", 132),   # bulk 80 + tail 52
+    # N = 100: 4 parts of 584 (init, 120 x 3 sweeps, 116 repack attempts, 106 conditional hand-overs, the finisher)
+    "long_default": (100, 16384, [], "solve", 2336),
+    # N = 100: bulk 480 (reset, init, 120 x 3 sweeps, 117 repacks, finisher) + tail 2477 (600 x (3 sweeps, repack),
+    # 75 hand-overs to the cooperative kernel, one every 8 rounds, then one more and the finisher)
+    "long_pipelined": (100, 16384, [("set_pipeline", 2, 1024)], "solve", 2957),
     "long_latency": (200, 40, [], "solve", 1),                    # the cooperative kernel, one problem per block
     "long_rounds": (200, 40, [("set_solver_mode", 0, 12, 0)], "solve", 46),
 }

@@ -41,31 +41,6 @@ def _stale(out, deps):
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_variant(name, defines):
-    """Experiment helper: builds udacitympc_b200/lib/libb200mpc_<name>.so with extra -D flags on the solver kernels
-    (select it at run time with B200MPC_LIB=<path>)."""
-    os.makedirs(LIBDIR, exist_ok=True)
-    nvcc = _nvcc()
-    objs = []
-    for src, extra in UNITS:
-        s = os.path.join(CSRC, src)
-        o = os.path.join(LIBDIR, f"{name}_" + src.replace(".cu", ".o"))
-        cmd = [nvcc] + ARCH + COMMON + extra + (defines if src == "solve_kernel.cu" else []) + ["-c", s, "-o", o]
-        r = subprocess.run(cmd, capture_output=True, text=True)
-        if r.returncode != 0:
-            sys.stderr.write(r.stdout + r.stderr)
-            raise RuntimeError("nvcc failed on " + src)
-        objs.append(o)
-    out = os.path.join(LIBDIR, f"libb200mpc_{name}.so")
-    r = subprocess.run([nvcc] + ARCH + ["-shared", "-o", out] + objs, capture_output=True, text=True)
-    if r.returncode != 0:
-        sys.stderr.write(r.stdout + r.stderr)
-        raise RuntimeError("link failed")
-    for o in objs:
-        os.remove(o)
-    return out
-
-
 def build(force=False, verbose=False):
     os.makedirs(LIBDIR, exist_ok=True)
     nvcc = _nvcc()

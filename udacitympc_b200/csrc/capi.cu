@@ -60,7 +60,6 @@ struct b200mpc_handle {
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timing;   // around every solve while timing_on
   cudaEvent_t done = nullptr;   // recorded after every solve: the next solve on this handle (any stream) waits for it
   bool done_valid = false;
-  int resto_mode = 2;
   b200mpc_params user_params;
   long long launches = 0;
   // CUDA graphs of whole solves (init + rounds x (factor, forward, step) + finisher), keyed by every launch argument
@@ -368,8 +367,6 @@ int b200mpc_create(const b200mpc_params* p, int device, b200mpc_handle** out) {
   h->device = device;
   if (const char* e = getenv("B200MPC_NO_GRAPHS")) h->use_graphs = !(e[0] == '1');
   if (const char* e = getenv("B200MPC_NO_COOP")) h->cfg.coop = !(e[0] == '1');
-  if (const char* e = getenv("B200MPC_RESTORATION")) { int v = atoi(e); if (v >= 0 && v <= 2) h->P.resto = v; }
-  h->resto_mode = h->P.resto;
   e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
   if (e != cudaSuccess) { delete h; return cuda_fail(e, "cudaStreamCreate"); }
   e = cudaEventCreateWithFlags(&h->done, cudaEventDisableTiming);
@@ -380,20 +377,6 @@ int b200mpc_create(const b200mpc_params* p, int device, b200mpc_handle** out) {
     h->ss.n_aux = i + 1;
   }
   if (cudaEventCreateWithFlags(&h->ss.fork, cudaEventDisableTiming) != cudaSuccess) h->ss.n_aux = 0;
-  if (const char* rp = getenv("B200MPC_COMPACT")) {   // tuning override: "<max live fraction>[,<first round>]"
-    h->cfg.compact_max_live = atof(rp);
-    if (const char* c = strchr(rp, ',')) h->cfg.compact_from = atoi(c + 1) > 0 ? atoi(c + 1) : 1;
-  }
-  if (const char* hb = getenv("B200MPC_HANDOVER")) {   // tuning override: "<occupied slots>[,<max rounds>]" (0 = static rounds)
-    h->cfg.handover_below = atoi(hb);
-    if (const char* c = strchr(hb, ',')) { int v = atoi(c + 1); if (v > 0) h->cfg.handover_max_rounds = v; }
-  }
-  if (const char* tr = getenv("B200MPC_TAIL")) {   // tuning override: "<tail rounds>[,<occupied slots for the cooperative kernel>]"
-    h->cfg.tail_rounds = atoi(tr) > 0 ? atoi(tr) : 0;
-    if (const char* c = strchr(tr, ',')) h->cfg.tail_take_below = atoi(c + 1) > 0 ? atoi(c + 1) : 0;
-  }
-  if (const char* rr = getenv("B200MPC_ROUNDS")) { int v = atoi(rr); if (v > 0) h->cfg.rounds = v; }
-  if (const char* sp = getenv("B200MPC_SPLIT")) { int v = atoi(sp); if (v >= 1 && v <= 4) h->cfg.split = v; }
   *out = h;
   return 0;
 }
@@ -498,7 +481,6 @@ int b200mpc_set_restoration(b200mpc_handle* h, int mode) {
   if (!h) return fail(B200MPC_ERR_ARG, "null handle");
   if (mode < 0 || mode > 2) return fail(B200MPC_ERR_ARG, "restoration: mode must be 0, 1 or 2");
   h->P.resto = mode;
-  h->resto_mode = mode;
   ++h->config_gen;
   return 0;
 }
@@ -749,7 +731,7 @@ int b200mpc_solve_batch_multi(b200mpc_handle* const* hs, int n_handles, int B, c
   for (int g = 0; g < n_handles; ++g) {
     for (int k = 0; k < g; ++k)
       if (hs[k] == hs[g]) return fail(B200MPC_ERR_ARG, "handle " + std::to_string(g) + " repeats handle " + std::to_string(k));
-    if (!same_params(hs[g]->user_params, hs[0]->user_params) || hs[g]->resto_mode != hs[0]->resto_mode)
+    if (!same_params(hs[g]->user_params, hs[0]->user_params) || hs[g]->P.resto != hs[0]->P.resto)
       return fail(B200MPC_ERR_ARG, "handle " + std::to_string(g) + " was created with other parameters than handle 0");
   }
   if (int rc0 = check_solve_args(hs[0], B, state6, coeffs, ncoef, out8)) return rc0;

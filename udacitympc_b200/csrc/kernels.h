@@ -25,16 +25,11 @@ struct SolveConfig {
   // adaptive hand-over (automatic rounds only): occupied slots (whole call) at which the cooperative kernel takes over
   int handover_below = 1184;      // one wave of 8 warps on 148 SMs
   int handover_from = 14;         // first round after which it may happen
-  int handover_max_rounds = 0;    // 0 = by horizon: 20 up to N = 50, 2 N - 80 above (120 at N = 100); see handover_rounds (solve_kernel.cu)
   // batch compaction: after every round from compact_from on, if the unfinished problems fill at most
   // compact_max_live of the occupied workspace slots, they are moved to consecutive slots, so that later rounds run
   // full warps on whole 32-byte sectors (0 = off)
   double compact_max_live = 0.7;
   int compact_from = 4;
-  // pipelined solves (launch_solve_bulk / launch_solve_tail): rounds the tail context runs before its finisher (0 = by
-  // horizon: 10 up to N = 50, 2 N - 80 above)
-  int tail_rounds = 0;
-  int tail_take_below = 0;   // long horizons: occupied slots at which the cooperative kernel takes a tail over (0 = 32)
   bool coop = true;       // latency path = cooperative warp-per-problem kernel (false: thread-per-problem fused kernel)
 };
 struct SplitStreams {   // auxiliary streams / events owned by the handle (n_aux <= 3)

@@ -21,25 +21,13 @@
 
 namespace b200mpc {
 
-#ifndef MPC_BLOCK
-#define MPC_BLOCK 64
-#endif
-constexpr int kBlock = MPC_BLOCK;
-// resident blocks per SM the light sweeps are compiled for (register cap = 65536 / (64 * blocks))
-#ifndef MPC_FWD_BLOCKS
-#define MPC_FWD_BLOCKS 6
-#endif
+constexpr int kBlock = 64;
+// resident blocks per SM the light sweeps are compiled for (register cap = 65536 / (64 * blocks)).
 // The step sweep runs at 4 blocks per SM: 228 registers, nothing spilled.  At 6 blocks (168 registers, 240 B of spill
 // stores and 352 B of spill loads per thread and stage) it is 3 % slower with one caller and with overlapped callers
-// (gpurun_out/r2_sb*.json: 13.59 -> 14.05 M solves/s; 5 blocks: 13.57 M) -- the sweep is bound by its dependent
-// instruction chains, not by the number of resident warps.
-#ifndef MPC_STEP_BLOCKS
-#define MPC_STEP_BLOCKS 4
-#endif
-#ifndef MPC_FACTOR_BLOCKS
-#define MPC_FACTOR_BLOCKS 4
-#endif
-constexpr int kFwdBlocks = MPC_FWD_BLOCKS, kStepBlocks = MPC_STEP_BLOCKS, kFactorBlocks = MPC_FACTOR_BLOCKS;
+// (profiles/r2_sweep_tuning_ab.json, r2_sb*: 13.59 -> 14.05 M solves/s; 5 blocks: 13.57 M) -- the sweep is bound by
+// its dependent instruction chains, not by the number of resident warps.
+constexpr int kFwdBlocks = 6, kStepBlocks = 4, kFactorBlocks = 4;
 
 // One workspace region holds every problem of a batch; the buffer the handle allocates has two of them (the batch
 // compaction moves the unfinished problems back and forth), two slot -> problem maps and the counters.
@@ -526,9 +514,7 @@ static bool launch_coop(const Params& P, const CostArgs& A, int fresh, int take_
 // than 100) and a slower cooperative kernel (0.34 ms per problem and iteration at N = 100, 2 warps per SM), so the sweeps
 // keep the tail longer there: measured with 4 overlapped batches of 65 536 problems at N = 100, 20 rounds 267 ms per
 // batch, 120 rounds 225 ms; N <= 50 does not gain (profiles/r1_handover_sweep_long_horizons.log).
-static int handover_rounds(const Params& P, const SolveConfig& cfg) {
-  return cfg.handover_max_rounds > 0 ? cfg.handover_max_rounds : (P.N <= 50 ? 20 : 2 * P.N - 80);
-}
+static int handover_rounds(const Params& P) { return P.N <= 50 ? 20 : 2 * P.N - 80; }
 
 // launches every kernel of the solve of problems [b0, b1) on one stream
 static cudaError_t launch_part(const Params& P, CostArgs A, const SolveConfig& cfg, int rounds, int take_below, cudaStream_t stream, long long* n) {
@@ -573,7 +559,7 @@ cudaError_t launch_solve(const Params& P, int B, int steps, const SolveIO& io, d
   // rest over as soon as the compacted batch fits its two waves (the launches after that find nothing to do); a fixed
   // number of rounds (b200mpc_set_solver_mode) hands over exactly there
   const bool adaptive = cfg.rounds <= 0 && desc != nullptr && cfg.coop && cfg.handover_below > 0;
-  const int rounds = cfg.rounds > 0 ? cfg.rounds : (adaptive ? handover_rounds(P, cfg) : (parts > 1 ? 16 : 18));
+  const int rounds = cfg.rounds > 0 ? cfg.rounds : (adaptive ? handover_rounds(P) : (parts > 1 ? 16 : 18));
   const int take_below = adaptive ? (cfg.handover_below / parts > 64 ? cfg.handover_below / parts : 64) : 0;
   cudaError_t e = cudaSuccess;
   if (parts > 1) {
@@ -610,7 +596,7 @@ cudaError_t launch_solve_bulk(const Params& P, int B, const SolveIO& io, double*
   if (B <= 0) return cudaSuccess;
   const WsLayout L = ws_layout(ws, P.N, B), T = ws_layout(tail.ws, P.N, tail.slots);
   const CostArgs A = solve_args(B, 1, io, L, L.desc, 0, B, 0.0);
-  const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P, cfg);
+  const int rounds = cfg.rounds > 0 ? cfg.rounds : handover_rounds(P);
   mpc_tail_reset_kernel<<<1, 32, 0, stream>>>(T.desc);
   *n += 1;
   launch_init(P, A, stream, n);
@@ -641,11 +627,11 @@ cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const T
   // registers until the slowest problem of the block is done (measured: with either as the finisher of 32 tails in flight
   // the bulk of the following batches runs at a third of its speed).  Only the last few problems go to the cooperative kernel.
   const bool long_tail = P.N > 50;
-  const int rounds = cfg.tail_rounds > 0 ? cfg.tail_rounds : (long_tail ? 6 * P.N : 10);
+  const int rounds = long_tail ? 6 * P.N : 10;
   int take_below = 0;
   if (cfg.coop && cfg.handover_below > 0) {
     const int resident = coop_resident_warps(P.N);
-    take_below = long_tail ? (cfg.tail_take_below > 0 ? cfg.tail_take_below : 32) : (cfg.handover_below < resident ? cfg.handover_below : resident);
+    take_below = long_tail ? 32 : (cfg.handover_below < resident ? cfg.handover_below : resident);
     if (take_below > resident) take_below = resident;
     if (take_below > tail.slots) take_below = tail.slots;
   }
