@@ -280,13 +280,15 @@ int b200mpc_polyfit_batch(b200mpc_handle* h, int B, const double* xs, const doub
 int b200mpc_polyfit_batch_device(b200mpc_handle* h, int B, const double* d_xs, const double* d_ys, int m, int order,
                                  double* d_coeffs_out, void* stream);
 
-/* y[b] = sum_i coeffs[b][i] * x[b]^i  (helpers.h:13-19).  coeffs: B x ncoef. */
+/* y[b] = sum_i coeffs[b][i] * x[b]^i  (helpers.h:13-19).  coeffs: B x ncoef, 1 <= ncoef <= 64. */
 int b200mpc_polyeval_batch(b200mpc_handle* h, int B, const double* coeffs, int ncoef, const double* x, double* y);
+/* Device buffers, field-major: d_coeffs[i*B+b], d_x[b], d_y[b]; 1 <= ncoef <= 64. */
 int b200mpc_polyeval_batch_device(b200mpc_handle* h, int B, const double* d_coeffs, int ncoef, const double* d_x,
                                   double* d_y, void* stream);
 
 /* B bicycle-model rollouts of H Euler steps (global_kinematic_model/solution/main.cpp:36-62; H=1 is globalKinematic).
- *   state4 B x 4 (x,y,psi,v);  act B x H x 2 (delta,a);  out B x H x 4 (the state after each step). */
+ *   state4 B x 4 (x,y,psi,v);  act B x H x 2 (delta,a);  out B x H x 4 (the state after each step).
+ *   1 <= H <= 1024 on this host entry, 1 <= H <= 4096 on the device entry; Lf > 0. */
 int b200mpc_rollout_batch(b200mpc_handle* h, int B, int H, const double* state4, const double* act, double dt,
                           double Lf, double* out);
 /* Device buffers, field-major: d_state4[k*B+b], d_act[(s*2+j)*B+b], d_out[(s*4+k)*B+b]. */
@@ -297,7 +299,7 @@ int b200mpc_rollout_batch_device(b200mpc_handle* h, int B, int H, const double* 
  * nearest centre-line point (what mpc_to_line/src/custom_MPC.cpp:177-185 computes), the 6 consecutive centre-line
  * points from there, global -> vehicle frame, degree-3 polyfit, and the MPC inputs in the vehicle frame:
  * state6 = (0, 0, 0, v, cte = p(0), epsi = -atan(p'(0))) as solution/main.cpp:34-37 defines cte / epsi.
- *   pose4  B x 4 (x, y, psi, v);  centerline  n_wp x 2 (x, y), n_wp >= 6 (e.g. columns 4,5 of mpc_to_line/roadmap.csv)
+ *   pose4  B x 4 (x, y, psi, v);  centerline  n_wp x 2 (x, y), 6 <= n_wp <= 12000 (e.g. columns 4,5 of mpc_to_line/roadmap.csv)
  *   state6_out  B x 6;  coeffs_out  B x 4 -- ready for b200mpc_solve_batch(..., ncoef = 4, ...) */
 int b200mpc_roadmap_reference_batch(b200mpc_handle* h, int B, const double* pose4, const double* centerline, int n_wp,
                                     double* state6_out, double* coeffs_out);
