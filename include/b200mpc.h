@@ -170,6 +170,30 @@ int b200mpc_solve_batch_cost_device(b200mpc_handle* h, int B, const double* d_st
                                     double* d_out8, double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters,
                                     void* stream);
 
+/* b200mpc_solve_batch_cost with a per-problem vehicle model and actuator limits.  NOT reference behaviour: the reference
+ * has one dt, Lf and one pair of bounds (MPC.cpp:14-15, 194-203); here a fleet of vehicles with different wheelbases and
+ * steering / acceleration limits is solved in one call, each problem with its own values.
+ *   model4  B x 4 per problem: dt, Lf, delta_max, a_max (the fields of b200mpc_params, in that order; the order of
+ *           grad_model of b200mpc_solve_batch_vjp_model), or NULL for the handle's values.  N, tol, max_iter and the
+ *           restoration mode stay the handle's.
+ *   cost8   as in b200mpc_solve_batch_cost, or NULL; either row pointer may be NULL (both NULL: b200mpc_solve_batch_warm).
+ * A problem whose model4 row has an entry that is not finite and positive (what b200mpc_create rejects for a handle) gets
+ * status -13 (Invalid_Number_Detected) and 0 iterations; the other problems of the batch are unaffected.  model4 equal
+ * to the handle's values in every row gives what the call without it gives to the last bits (not bit for bit: the
+ * per-problem kernels hold dt, Lf and the bounds in registers, and a few operations round differently there); the same
+ * call is bitwise reproducible.  b200mpc_closed_loop_batch and
+ * b200mpc_solve_batch_multi do not take per-problem rows.  The other arguments and errors are those of
+ * b200mpc_solve_batch_warm. */
+int b200mpc_solve_batch_model(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                              const double* model4, const double* x_init, const double* mult_init, double mu_init, double* out8,
+                              double* traj, double* mult, double* obj, int* status, int* iters);
+/* Same on device buffers, field-major like b200mpc_solve_batch_warm_device: d_cost8[k*B+b], d_model4[k*B+b].  Pipelined
+ * solves (b200mpc_set_pipeline) accept it like b200mpc_solve_batch_device. */
+int b200mpc_solve_batch_model_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                     const double* d_cost8, const double* d_model4, const double* d_x_init,
+                                     const double* d_mult_init, double mu_init, double* d_out8, double* d_traj, double* d_mult,
+                                     double* d_obj, int* d_status, int* d_iters, void* stream);
+
 /* Adjoint sensitivities (vector-Jacobian product) of B solutions: the derivative of a scalar loss L(out8, traj, obj) of
  * each problem's solution w.r.t. its initial state, its reference polynomial and the handle's cost parameters, by the
  * implicit-function theorem at the returned primal-dual point (the differentiable-MPC layer; Ipopt's sIPOPT does the
@@ -213,6 +237,25 @@ int b200mpc_solve_batch_vjp_cost_device(b200mpc_handle* h, int B, const double* 
                                         const double* d_cost8, const double* d_traj, const double* d_mult, const double* d_g_out8,
                                         const double* d_g_traj, const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs,
                                         double* d_grad_params, int* d_status, void* stream);
+
+/* b200mpc_solve_batch_vjp_cost of solutions of b200mpc_solve_batch_model: the derivative is taken at each problem's own
+ * cost and model parameters, and also w.r.t. the model.  NOT reference behaviour.
+ *   cost8, model4  the rows the solve used, or NULL for the handle's values (either may be NULL)
+ *   grad_model     B x 4 (dt, Lf, delta_max, a_max): dL/d(model4 row) of each problem, or NULL.  With model4 NULL it is
+ *                  taken at the handle's values; summed over the batch, that is the gradient w.r.t. the shared model.
+ * A problem whose model4 row has an entry that is not finite and positive gets status -13 and NaN gradients.  The other
+ * arguments and errors are those of b200mpc_solve_batch_vjp_cost. */
+int b200mpc_solve_batch_vjp_model(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                                  const double* model4, const double* traj, const double* mult, const double* g_out8,
+                                  const double* g_traj, const double* g_obj, double* grad_state6, double* grad_coeffs,
+                                  double* grad_params, double* grad_model, int* status);
+/* Same on device buffers, field-major like b200mpc_solve_batch_vjp_device: d_model4[k*B+b], d_grad_model[k*B+b].  Exactly
+ * one kernel launch. */
+int b200mpc_solve_batch_vjp_model_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                         const double* d_cost8, const double* d_model4, const double* d_traj, const double* d_mult,
+                                         const double* d_g_out8, const double* d_g_traj, const double* d_g_obj,
+                                         double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
+                                         double* d_grad_model, int* d_status, void* stream);
 
 /* Warm start for b200mpc_closed_loop_batch (SURVEY 8f; NOT reference behaviour: the reference cold-starts every call,
  * MPC.cpp:167-177, and so does this library unless enabled here).  When enabled, every step after the first starts from

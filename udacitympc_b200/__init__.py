@@ -17,6 +17,8 @@ All arithmetic runs in the CUDA library; importing this package without libb200m
 CUDA device) raises -- there is no CPU fallback.
 """
 from .api import (  # noqa: F401
+    MODEL_NAMES,
+    PARAM_NAMES,
     B200MPCError,
     MPC,
     MPCParams,
@@ -33,6 +35,6 @@ from .api import (  # noqa: F401
     shift_solution,
 )
 
-__all__ = ["B200MPCError", "MPC", "MPCParams", "global_kinematic", "lib_path", "load_library", "polyeval",
+__all__ = ["MODEL_NAMES", "PARAM_NAMES", "B200MPCError", "MPC", "MPCParams", "global_kinematic", "lib_path", "load_library", "polyeval",
            "polyeval_batch", "polyfit", "polyfit_batch", "read_roadmap_csv", "roadmap_reference_batch", "rollout_batch",
            "shift_solution"]

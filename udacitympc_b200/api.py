@@ -46,6 +46,12 @@ SYMBOLS = {
                                                        _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "b200mpc_solve_batch_vjp_cost": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int] + [_dp] * 9 + [_ip]),
     "b200mpc_solve_batch_vjp_cost_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 11),
+    "b200mpc_solve_batch_model": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _dp, ctypes.c_double,
+                                                 _dp, _dp, _dp, _dp, _ip, _ip]),
+    "b200mpc_solve_batch_model_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp,
+                                                        ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200mpc_solve_batch_vjp_model": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int] + [_dp] * 11 + [_ip]),
+    "b200mpc_solve_batch_vjp_model_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 13),
     "b200mpc_solve_batch_vjp": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
                                                _ip]),
     "b200mpc_solve_batch_vjp_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 10),
@@ -144,6 +150,20 @@ def _cost8(cost_params, B):
     return np.ascontiguousarray(c)
 
 
+# the vehicle model parameters of a model4 row, in the order of b200mpc_params (and of grad_model)
+MODEL_NAMES = ("dt", "Lf", "delta_max", "a_max")
+
+
+def _model4(model_params, B):
+    """(B, 4) or (4,) broadcast, in MODEL_NAMES order -> the (B, 4) float64 rows b200mpc_solve_batch_model takes."""
+    c = _f64(model_params)
+    if c.ndim == 1:
+        c = np.broadcast_to(c, (B, c.size))
+    if c.shape != (B, 4):
+        raise ValueError(f"model_params must be (B, 4) or (4,) in the order {MODEL_NAMES}")
+    return np.ascontiguousarray(c)
+
+
 class MPC:
     """Drop-in for the reference's `class MPC` (mpc_to_line/src/MPC.h:7-17).
 
@@ -218,7 +238,7 @@ class MPC:
 
     # -- batched host-buffer call
     def solve_batch(self, states, coeffs, want_traj=False, x_init=None, mult_init=None, mu_init=1e-4, want_mult=False,
-                    cost_params=None):
+                    cost_params=None, model_params=None):
         """states (B,6), coeffs (B,ncoef) or (ncoef,) shared by all problems.  Returns dict(out8 (B,8), cost (B,),
         status (B,), iters (B,), traj (B,8N-2) if requested, mult (B,10N-4) if requested).
 
@@ -227,7 +247,11 @@ class MPC:
         shift_solution() turns one receding-horizon step's traj / mult into the next step's start.
 
         Per-problem costs (not reference behaviour, b200mpc_solve_batch_cost): cost_params (B,8) or (8,) shared, in the
-        order PARAM_NAMES, replaces the handle's ref_v and weights problem by problem; None uses the handle's."""
+        order PARAM_NAMES, replaces the handle's ref_v and weights problem by problem; None uses the handle's.
+
+        Per-problem vehicles (not reference behaviour, b200mpc_solve_batch_model): model_params (B,4) or (4,) shared, in
+        the order MODEL_NAMES, replaces the handle's dt, Lf, delta_max and a_max problem by problem; None uses the
+        handle's."""
         states = _f64(states)
         if states.ndim != 2 or states.shape[1] != 6:
             raise ValueError("states must be (B, 6)")
@@ -243,7 +267,18 @@ class MPC:
         status = np.empty(B, dtype=np.int32)
         iters = np.empty(B, dtype=np.int32)
         traj = np.empty((B, self.num_vars)) if want_traj else None
-        if cost_params is not None:
+        if model_params is not None:
+            m4 = _model4(model_params, B)
+            c8 = None if cost_params is None else _cost8(cost_params, B)
+            x_init = None if x_init is None else _f64(x_init, (B, self.num_vars))
+            mult_init = None if mult_init is None else _f64(mult_init, (B, self.num_mults))
+            mult = np.empty((B, self.num_mults)) if want_mult else None
+            _check(self._lib.b200mpc_solve_batch_model(
+                self._h, B, _ptr(states), _ptr(coeffs), ncoef, None if c8 is None else _ptr(c8), _ptr(m4),
+                None if x_init is None else _ptr(x_init), None if mult_init is None else _ptr(mult_init), float(mu_init),
+                _ptr(out8), _ptr(traj) if want_traj else None, _ptr(mult) if want_mult else None, _ptr(cost),
+                status.ctypes.data_as(_ip), iters.ctypes.data_as(_ip)))
+        elif cost_params is not None:
             x_init = None if x_init is None else _f64(x_init, (B, self.num_vars))
             mult_init = None if mult_init is None else _f64(mult_init, (B, self.num_mults))
             mult = np.empty((B, self.num_mults)) if want_mult else None
@@ -298,14 +333,26 @@ class MPC:
                                                          d_traj or None, d_mult or None, d_obj or None, d_status or None,
                                                          d_iters or None, stream or None))
 
+    def solve_batch_model_device(self, B, d_state6, d_coeffs, ncoef, d_cost8, d_model4, d_x_init=0, d_mult_init=0,
+                                 mu_init=1e-4, d_out8=0, d_traj=0, d_mult=0, d_obj=0, d_status=0, d_iters=0, stream=0):
+        """Raw device-pointer solve with per-problem costs and vehicle models (integers, 0 = none), field-major buffers:
+        d_cost8 [8][B] in the order PARAM_NAMES, d_model4 [4][B] in the order MODEL_NAMES (0 = the handle's values);
+        asynchronous on `stream`.  See b200mpc_solve_batch_model_device."""
+        _check(self._lib.b200mpc_solve_batch_model_device(self._h, B, d_state6, d_coeffs, ncoef, d_cost8 or None,
+                                                          d_model4 or None, d_x_init or None, d_mult_init or None,
+                                                          float(mu_init), d_out8, d_traj or None, d_mult or None,
+                                                          d_obj or None, d_status or None, d_iters or None, stream or None))
+
     def solve_batch_vjp(self, states, coeffs, traj, mult, g_out8=None, g_traj=None, g_obj=None, want_params=False,
-                        cost_params=None):
+                        cost_params=None, model_params=None, want_model=False):
         """Adjoint sensitivities of solutions (b200mpc_solve_batch_vjp; not reference behaviour): for a loss L with the
         incoming gradients g_out8 (B,8), g_traj (B,8N-2), g_obj (B,) -- any of them None, not all -- returns
         dict(grad_state6 (B,6), grad_coeffs (B,ncoef) per problem, status (B,), and grad_params (B,8) in the order
         PARAM_NAMES if want_params).  traj (B,8N-2) and mult (B,10N-4) must be a converged solution of (states, coeffs)
         on a handle with these params, as solve_batch(..., want_traj=True, want_mult=True) returns it.  cost_params (B,8)
-        or (8,): the per-problem costs the solve used (b200mpc_solve_batch_vjp_cost); grad_params is w.r.t. them."""
+        or (8,): the per-problem costs the solve used (b200mpc_solve_batch_vjp_cost); grad_params is w.r.t. them.
+        model_params (B,4) or (4,): the per-problem vehicle models the solve used; want_model adds grad_model (B,4) in the
+        order MODEL_NAMES, w.r.t. them or, without model_params, w.r.t. the handle's (b200mpc_solve_batch_vjp_model)."""
         states = _f64(states)
         if states.ndim != 2 or states.shape[1] != 6:
             raise ValueError("states must be (B, 6)")
@@ -326,7 +373,15 @@ class MPC:
         grads = (None if g_out8 is None else _ptr(g_out8), None if g_traj is None else _ptr(g_traj),
                  None if g_obj is None else _ptr(g_obj), _ptr(gs), _ptr(gc), None if gp is None else _ptr(gp),
                  status.ctypes.data_as(_ip))
-        if cost_params is None:
+        gm = np.empty((B, 4)) if want_model else None
+        if model_params is not None or want_model:
+            c8 = None if cost_params is None else _cost8(cost_params, B)
+            m4 = None if model_params is None else _model4(model_params, B)
+            _check(self._lib.b200mpc_solve_batch_vjp_model(
+                self._h, B, _ptr(states), _ptr(coeffs), ncoef, None if c8 is None else _ptr(c8),
+                None if m4 is None else _ptr(m4), _ptr(traj), _ptr(mult), *grads[:6], None if gm is None else _ptr(gm),
+                grads[6]))
+        elif cost_params is None:
             _check(self._lib.b200mpc_solve_batch_vjp(self._h, B, _ptr(states), _ptr(coeffs), ncoef, _ptr(traj), _ptr(mult),
                                                      *grads))
         else:
@@ -335,6 +390,8 @@ class MPC:
         r = dict(grad_state6=gs, grad_coeffs=gc, status=status)
         if want_params:
             r["grad_params"] = gp
+        if want_model:
+            r["grad_model"] = gm
         return r
 
     def solve_batch_vjp_device(self, B, d_state6, d_coeffs, ncoef, d_traj, d_mult, d_g_out8=0, d_g_traj=0, d_g_obj=0,
@@ -354,6 +411,18 @@ class MPC:
                                                              d_mult, d_g_out8 or None, d_g_traj or None, d_g_obj or None,
                                                              d_grad_state6 or None, d_grad_coeffs or None,
                                                              d_grad_params or None, d_status or None, stream or None))
+
+    def solve_batch_vjp_model_device(self, B, d_state6, d_coeffs, ncoef, d_cost8, d_model4, d_traj, d_mult, d_g_out8=0,
+                                     d_g_traj=0, d_g_obj=0, d_grad_state6=0, d_grad_coeffs=0, d_grad_params=0, d_grad_model=0,
+                                     d_status=0, stream=0):
+        """Raw device-pointer VJP with per-problem costs and vehicle models (integers, 0 = none), field-major buffers,
+        d_cost8 [8][B], d_model4 / d_grad_model [4][B]; one kernel launch, asynchronous on `stream`.  See
+        b200mpc_solve_batch_vjp_model_device."""
+        _check(self._lib.b200mpc_solve_batch_vjp_model_device(self._h, B, d_state6, d_coeffs, ncoef, d_cost8 or None,
+                                                              d_model4 or None, d_traj, d_mult, d_g_out8 or None,
+                                                              d_g_traj or None, d_g_obj or None, d_grad_state6 or None,
+                                                              d_grad_coeffs or None, d_grad_params or None,
+                                                              d_grad_model or None, d_status or None, stream or None))
 
     def wait(self):
         """Waits for everything queued on this handle's own stream (b200mpc_solve_batch_async calls)."""

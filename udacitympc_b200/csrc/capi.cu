@@ -127,8 +127,8 @@ bool same_key(const b200mpc_handle::GraphKey& a, const b200mpc_handle::GraphKey&
   return a.phase == b.phase && a.B == b.B && a.steps == b.steps && a.io.state6 == b.io.state6 && a.io.coeffs == b.io.coeffs &&
          a.io.ncoef == b.io.ncoef && a.io.out8 == b.io.out8 && a.io.traj == b.io.traj && a.io.obj == b.io.obj &&
          a.io.status == b.io.status && a.io.iters == b.io.iters && a.io.io_aos == b.io.io_aos && a.io.x_init == b.io.x_init &&
-         a.io.mult_init == b.io.mult_init && a.io.mu_init == b.io.mu_init && a.io.mult == b.io.mult && a.io.cost8 == b.io.cost8 && a.ws == b.ws &&
-         a.tail == b.tail && a.config_gen == b.config_gen;
+         a.io.mult_init == b.io.mult_init && a.io.mu_init == b.io.mu_init && a.io.mult == b.io.mult && a.io.cost8 == b.io.cost8 &&
+         a.io.model4 == b.io.model4 && a.ws == b.ws && a.tail == b.tail && a.config_gen == b.config_gen;
 }
 
 // One launch sequence (a whole solve, or one half of a pipelined one) on stream s.  One solve is ~85 dependent
@@ -507,6 +507,14 @@ int b200mpc_solve_batch_cost_device(b200mpc_handle* h, int B, const double* d_st
                                     const double* d_cost8, const double* d_x_init, const double* d_mult_init, double mu_init,
                                     double* d_out8, double* d_traj, double* d_mult, double* d_obj, int* d_status, int* d_iters,
                                     void* stream) {
+  return b200mpc_solve_batch_model_device(h, B, d_state6, d_coeffs, ncoef, d_cost8, nullptr, d_x_init, d_mult_init, mu_init, d_out8,
+                                          d_traj, d_mult, d_obj, d_status, d_iters, stream);
+}
+
+int b200mpc_solve_batch_model_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                     const double* d_cost8, const double* d_model4, const double* d_x_init,
+                                     const double* d_mult_init, double mu_init, double* d_out8, double* d_traj, double* d_mult,
+                                     double* d_obj, int* d_status, int* d_iters, void* stream) {
   if (int rc = check_solve_args(h, B, d_state6, d_coeffs, ncoef, d_out8)) return rc;
   if (int rc = check_guess_args(d_x_init, d_mult_init, mu_init)) return rc;
   if (B == 0) return 0;
@@ -515,16 +523,16 @@ int b200mpc_solve_batch_cost_device(b200mpc_handle* h, int B, const double* d_st
   io.state6 = d_state6; io.coeffs = d_coeffs; io.ncoef = ncoef;
   io.out8 = d_out8; io.traj = d_traj; io.obj = d_obj; io.status = d_status; io.iters = d_iters;
   io.x_init = d_x_init; io.mult_init = d_mult_init; io.mu_init = d_x_init ? mu_init : 0.0; io.mult = d_mult;
-  io.cost8 = d_cost8;
+  io.cost8 = d_cost8; io.model4 = d_model4;
   return timed_solve(h, B, 1, io, stream ? (cudaStream_t)stream : h->stream);
 }
 
-// queues the copy of the host arrays state6 [B][6], coeffs [B][ncoef] and cost8 [B][8] (if given) to in_aos and points
-// io's inputs there (io_aos = 1)
+// queues the copy of the host arrays state6 [B][6], coeffs [B][ncoef], cost8 [B][8] and model4 [B][4] (if given) to
+// in_aos and points io's inputs there (io_aos = 1)
 static int stage_inputs(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, SolveIO* io,
-                        const double* cost8 = nullptr) {
+                        const double* cost8 = nullptr, const double* model4 = nullptr) {
   const size_t nb = (size_t)B;
-  CU(h->in_aos.ensure(nb * (6 + ncoef + (cost8 ? 8 : 0)) * sizeof(double)));
+  CU(h->in_aos.ensure(nb * (6 + ncoef + (cost8 ? 8 : 0) + (model4 ? 4 : 0)) * sizeof(double)));
   double* d_st = h->in_aos.as<double>();
   double* d_cf = d_st + nb * 6;
   CU(cudaMemcpyAsync(d_st, state6, nb * 6 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -535,17 +543,22 @@ static int stage_inputs(b200mpc_handle* h, int B, const double* state6, const do
     CU(cudaMemcpyAsync(d_c8, cost8, nb * 8 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     io->cost8 = d_c8;
   }
+  if (model4) {
+    double* d_m4 = d_cf + nb * (ncoef + (cost8 ? 8 : 0));
+    CU(cudaMemcpyAsync(d_m4, model4, nb * 4 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    io->model4 = d_m4;
+  }
   return 0;
 }
 
 // Everything b200mpc_solve_batch does except the final wait: copies, solve and copies back are queued on the handle's
 // stream (asynchronous when the host buffers are pinned).
 // x_init / mult_init / mult (b200mpc_solve_batch_warm): per-problem rows on the host, moved through the tiled transposes
-// like traj.  cost8 (b200mpc_solve_batch_cost): per-problem rows, read by the kernels in that layout.
+// like traj.  cost8 / model4 (b200mpc_solve_batch_model): per-problem rows, read by the kernels in that layout.
 static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, double* out8,
                                double* traj, double* obj, int* status, int* iters, const double* x_init = nullptr,
                                const double* mult_init = nullptr, double mu_init = 0.0, double* mult = nullptr,
-                               const double* cost8 = nullptr) {
+                               const double* cost8 = nullptr, const double* model4 = nullptr) {
   if (int rc = check_solve_args(h, B, state6, coeffs, ncoef, out8)) return rc;
   if (int rc = check_guess_args(x_init, mult_init, mu_init)) return rc;
   if (B == 0) return 0;
@@ -562,7 +575,7 @@ static int enqueue_solve_batch(b200mpc_handle* h, int B, const double* state6, c
   CU(h->iters.ensure(nb * sizeof(int)));
   if (traj) { CU(h->traj_soa.ensure(nb * nv * sizeof(double))); CU(h->traj_aos.ensure(nb * nv * sizeof(double))); }
   SolveIO io;
-  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &io, cost8)) return rc;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &io, cost8, model4)) return rc;
   io.out8 = h->out_aos.as<double>(); io.traj = traj ? h->traj_soa.as<double>() : nullptr;
   io.obj = h->obj.as<double>(); io.status = h->status.as<int>(); io.iters = h->iters.as<int>();
   const int nm = 10 * h->P.N - 4;
@@ -624,8 +637,15 @@ int b200mpc_solve_batch_warm(b200mpc_handle* h, int B, const double* state6, con
 int b200mpc_solve_batch_cost(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
                              const double* x_init, const double* mult_init, double mu_init, double* out8, double* traj,
                              double* mult, double* obj, int* status, int* iters) {
+  return b200mpc_solve_batch_model(h, B, state6, coeffs, ncoef, cost8, nullptr, x_init, mult_init, mu_init, out8, traj, mult, obj,
+                                   status, iters);
+}
+
+int b200mpc_solve_batch_model(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                              const double* model4, const double* x_init, const double* mult_init, double mu_init, double* out8,
+                              double* traj, double* mult, double* obj, int* status, int* iters) {
   if (int rc = enqueue_solve_batch(h, B, state6, coeffs, ncoef, out8, traj, obj, status, iters, x_init, mult_init, mu_init, mult,
-                                   cost8))
+                                   cost8, model4))
     return rc;
   if (B == 0) return 0;
   CU(cudaSetDevice(h->device));
@@ -645,10 +665,19 @@ int b200mpc_solve_batch_vjp_cost_device(b200mpc_handle* h, int B, const double* 
                                         const double* d_cost8, const double* d_traj, const double* d_mult, const double* d_g_out8,
                                         const double* d_g_traj, const double* d_g_obj, double* d_grad_state6, double* d_grad_coeffs,
                                         double* d_grad_params, int* d_status, void* stream) {
+  return b200mpc_solve_batch_vjp_model_device(h, B, d_state6, d_coeffs, ncoef, d_cost8, nullptr, d_traj, d_mult, d_g_out8, d_g_traj,
+                                              d_g_obj, d_grad_state6, d_grad_coeffs, d_grad_params, nullptr, d_status, stream);
+}
+
+int b200mpc_solve_batch_vjp_model_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                         const double* d_cost8, const double* d_model4, const double* d_traj, const double* d_mult,
+                                         const double* d_g_out8, const double* d_g_traj, const double* d_g_obj,
+                                         double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
+                                         double* d_grad_model, int* d_status, void* stream) {
   if (int rc = check_vjp_args(h, B, d_state6, d_coeffs, ncoef, d_traj, d_mult, d_g_out8, d_g_traj, d_g_obj)) return rc;
   CU(cudaSetDevice(h->device));
   VjpCostIO io;
-  io.B = B; io.ncoef = ncoef; io.io_aos = 0; io.cost8 = d_cost8;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 0; io.cost8 = d_cost8; io.model4 = d_model4; io.grad_model = d_grad_model;
   io.state6 = d_state6; io.coeffs = d_coeffs; io.traj = d_traj; io.mult = d_mult;
   io.g_out8 = d_g_out8; io.g_traj = d_g_traj; io.g_obj = d_g_obj;
   io.grad_state6 = d_grad_state6; io.grad_coeffs = d_grad_coeffs; io.grad_params = d_grad_params; io.status = d_status;
@@ -667,6 +696,14 @@ int b200mpc_solve_batch_vjp(b200mpc_handle* h, int B, const double* state6, cons
 int b200mpc_solve_batch_vjp_cost(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
                                  const double* traj, const double* mult, const double* g_out8, const double* g_traj,
                                  const double* g_obj, double* grad_state6, double* grad_coeffs, double* grad_params, int* status) {
+  return b200mpc_solve_batch_vjp_model(h, B, state6, coeffs, ncoef, cost8, nullptr, traj, mult, g_out8, g_traj, g_obj, grad_state6,
+                                       grad_coeffs, grad_params, nullptr, status);
+}
+
+int b200mpc_solve_batch_vjp_model(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                                  const double* model4, const double* traj, const double* mult, const double* g_out8,
+                                  const double* g_traj, const double* g_obj, double* grad_state6, double* grad_coeffs,
+                                  double* grad_params, double* grad_model, int* status) {
   if (int rc = check_vjp_args(h, B, state6, coeffs, ncoef, traj, mult, g_out8, g_traj, g_obj)) return rc;
   CU(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
@@ -674,11 +711,11 @@ int b200mpc_solve_batch_vjp_cost(b200mpc_handle* h, int B, const double* state6,
   const size_t nrows = nv + nm + (g_traj ? nv : 0);
   CU(h->vjp_aos.ensure(nb * nrows * sizeof(double)));
   CU(h->vjp_soa.ensure(nb * nrows * sizeof(double)));
-  // per problem: g_out8 (8) | g_obj (1) | grad_state6 (6) | grad_coeffs (ncoef) | grad_params (8)
-  CU(h->vjp_io.ensure(nb * (23 + ncoef) * sizeof(double)));
+  // per problem: g_out8 (8) | g_obj (1) | grad_state6 (6) | grad_coeffs (ncoef) | grad_params (8) | grad_model (4, if asked)
+  CU(h->vjp_io.ensure(nb * (23 + ncoef + (grad_model ? 4 : 0)) * sizeof(double)));
   CU(h->status.ensure(nb * sizeof(int)));
   SolveIO in;
-  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &in, cost8)) return rc;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &in, cost8, model4)) return rc;
   double *ga = h->vjp_aos.as<double>(), *gs = h->vjp_soa.as<double>(), *d = h->vjp_io.as<double>();
   const double* rows[3] = {traj, mult, g_traj};
   const size_t len[3] = {nv, nm, nv};
@@ -693,15 +730,17 @@ int b200mpc_solve_batch_vjp_cost(b200mpc_handle* h, int B, const double* state6,
   if (g_out8) CU(cudaMemcpyAsync(d, g_out8, nb * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
   if (g_obj) CU(cudaMemcpyAsync(d + nb * 8, g_obj, nb * sizeof(double), cudaMemcpyHostToDevice, s));
   VjpCostIO io;
-  io.B = B; io.ncoef = ncoef; io.io_aos = 1; io.cost8 = in.cost8;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 1; io.cost8 = in.cost8; io.model4 = in.model4;
   io.state6 = in.state6; io.coeffs = in.coeffs; io.traj = gs; io.mult = gs + nb * nv;
   io.g_out8 = g_out8 ? d : nullptr; io.g_traj = g_traj ? gs + nb * (nv + nm) : nullptr; io.g_obj = g_obj ? d + nb * 8 : nullptr;
   io.grad_state6 = d + nb * 9; io.grad_coeffs = d + nb * 15; io.grad_params = d + nb * (15 + ncoef);
+  io.grad_model = grad_model ? d + nb * (23 + ncoef) : nullptr;
   io.status = h->status.as<int>();
   if (int rc = run_vjp(h, io, s)) return rc;
   if (grad_state6) CU(cudaMemcpyAsync(grad_state6, io.grad_state6, nb * 6 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (grad_coeffs) CU(cudaMemcpyAsync(grad_coeffs, io.grad_coeffs, nb * ncoef * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (grad_params) CU(cudaMemcpyAsync(grad_params, io.grad_params, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (grad_model) CU(cudaMemcpyAsync(grad_model, io.grad_model, nb * 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (status) CU(cudaMemcpyAsync(status, h->status.p, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   return 0;

@@ -42,8 +42,10 @@ struct SplitStreams {   // auxiliary streams / events owned by the handle (n_aux
 //   obj [steps][B] (optional), status [B] (last step, optional), iters [steps][B] (optional),
 //   x_init [8N-2][B] + mult_init [10N-4][B] (optional: start from this point with barrier parameter mu_init instead of
 //   the default start point, Solver::init_guess; mult_init may be null), mult [10N-4][B] (last step, optional),
-//   cost8 [8][B] (optional: per-problem ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da instead of the handle's);
-// io_aos = 1: state6 [B][6], coeffs [B][ncoef], out8 [steps][B][8] (reference order), cost8 [B][8], the others as above
+//   cost8 [8][B] (optional: per-problem ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da instead of the handle's),
+//   model4 [4][B] (optional: per-problem dt, Lf, delta_max, a_max instead of the handle's);
+// io_aos = 1: state6 [B][6], coeffs [B][ncoef], out8 [steps][B][8] (reference order), cost8 [B][8], model4 [B][4], the
+// others as above
 struct SolveIO {
   const double *state6 = nullptr, *coeffs = nullptr;
   int ncoef = 0;
@@ -54,6 +56,7 @@ struct SolveIO {
   double mu_init = 0.0;
   double* mult = nullptr;
   const double* cost8 = nullptr;
+  const double* model4 = nullptr;
 };
 
 // K1+K2+K3 fused: `steps` consecutive interior-point solves per problem (steps > 1 = closed loop, each solve
@@ -84,10 +87,13 @@ struct VjpIO {
   double *grad_state6 = nullptr, *grad_coeffs = nullptr, *grad_params = nullptr;
   int* status = nullptr;
 };
-// VjpIO plus per-problem cost parameters: cost8 [8][B] ([B][8] with io_aos), or null for the handle's.  A struct of its own
-// so that the kernel instance without them keeps VjpIO as its parameter block.
+// VjpIO plus per-problem cost and model parameters: cost8 [8][B], model4 [4][B] ([B][k] with io_aos), or null for the
+// handle's, and grad_model [4][B] (dt, Lf, delta_max, a_max; or null).  A struct of its own so that the kernel instance
+// without them keeps VjpIO as its parameter block.
 struct VjpCostIO : VjpIO {
   const double* cost8 = nullptr;
+  const double* model4 = nullptr;
+  double* grad_model = nullptr;
 };
 cudaError_t launch_vjp(const Params& P, const VjpCostIO& io, double* ws, cudaStream_t stream);
 

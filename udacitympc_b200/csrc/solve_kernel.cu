@@ -83,13 +83,18 @@ struct SolveArgs {
   double* mult;           // [10N-4][B] or null (last step)
 };
 
-// Per-problem cost parameters (b200mpc_solve_batch_cost*): the kernel instances with COST = true take this parameter
-// block, every other instance SolveArgs, whose layout (and so the machine code of those instances) does not change.
+// Per-problem rows (b200mpc_solve_batch_cost*, b200mpc_solve_batch_model*): the kernel instances with ROWS != kNoRows
+// take this parameter block, every other instance SolveArgs, whose layout (and so the machine code of those instances)
+// does not change.  kCostRows instances read cost8 only; kModelRows instances read model4 and, if given, cost8.  They are
+// kept apart because per-problem dt, Lf and bounds (registers instead of the handle's constants) change the code of the
+// sweeps, and the cost rows alone must not pay for that.
+enum Rows { kNoRows = 0, kCostRows = 1, kModelRows = 2 };
 struct CostArgs : SolveArgs {
   const double* cost8;    // [8][B] ([B][8] with io_aos) or null: ref_v, w_cte, w_epsi, w_v, w_delta, w_a, w_ddelta, w_da
+  const double* model4;   // [4][B] ([B][4] with io_aos) or null: dt, Lf, delta_max, a_max
 };
-template <bool COST>
-using ArgsT = typename std::conditional<COST, CostArgs, SolveArgs>::type;
+template <int ROWS>
+using ArgsT = typename std::conditional<ROWS != kNoRows, CostArgs, SolveArgs>::type;
 
 __device__ __forceinline__ double* slot_base(const Params& P, double* ws, int slot) {
   return ws + (size_t)(slot >> 5) * (size_t)workspace_doubles_per_problem(P.N) * 32 + (slot & 31);
@@ -142,13 +147,34 @@ __device__ __forceinline__ bool cost_row(const double* cost8, int io_aos, int B,
   }
   return ok;
 }
-// COST instances: the solver of problem b runs on Q with b's cost row.  A non-finite row makes ref_v NaN, so the
-// objective at the start point is NaN and the start-point check stops the problem with status -13 and 0 iterations
-// (Solver::init_finish / guess_check), as for a non-finite x_init; the later sweeps never see it.
-template <bool COST>
-__device__ __forceinline__ void load_cost(const ArgsT<COST>& A, int b, Params& Q) {
-  if constexpr (COST) {
+// Problem b's row of model4 over dt, Lf, delta_max, a_max of Q, and Q's derived constants recomputed.  False: an entry
+// that is not finite and positive, what b200mpc_create rejects for a handle (Q is left unchanged then).
+__device__ __forceinline__ bool model_row(const double* model4, int io_aos, int B, int b, Params& Q) {
+  double c[4];
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    c[k] = model4[io_aos ? (size_t)b * 4 + k : (size_t)k * B + b];
+    ok &= c[k] > 0.0 && c[k] <= DBL_MAX;
+  }
+  if (ok) {
+    Q.dt = c[0]; Q.Lf = c[1]; Q.delta_max = c[2]; Q.a_max = c[3];
+    Q.finalize();
+  }
+  return ok;
+}
+// Per-problem instances: the solver of problem b runs on Q with b's rows (kModelRows: model4 and cost8 if given).  An
+// invalid row makes ref_v NaN, so the objective at the start point is NaN and the start-point check stops the problem
+// with status -13 and 0 iterations (Solver::init_finish / guess_check), as for a non-finite x_init; the later sweeps
+// never see it.
+template <int ROWS>
+__device__ __forceinline__ void load_cost(const ArgsT<ROWS>& A, int b, Params& Q) {
+  if constexpr (ROWS == kCostRows) {
     if (!cost_row(A.cost8, A.io_aos, A.B, b, Q)) Q.ref_v = NAN;
+  } else if constexpr (ROWS == kModelRows) {
+    bool ok = !A.cost8 || cost_row(A.cost8, A.io_aos, A.B, b, Q);
+    ok &= model_row(A.model4, A.io_aos, A.B, b, Q);
+    if (!ok) Q.ref_v = NAN;
   }
 }
 
@@ -176,15 +202,15 @@ __device__ __forceinline__ void count_live(int* counter) {
 }
 
 // ---- per-pass kernels ---------------------------------------------------------------------------------------
-template <bool WIO, bool COST>
-__global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
+template <bool WIO, int ROWS>
+__global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A) {
   const int b = A.b0 + blockIdx.x * blockDim.x + threadIdx.x;   // always launched on the uncompacted batch
   if (b >= A.b1) return;
   if (b == A.b0 && A.desc)
     for (int k = 0; k < kDescInts; ++k) A.desc[k] = 0;
   Params Q = P;
-  load_cost<COST>(A, b, Q);
-  Solver<32> S(COST ? Q : P, slot_base(P, A.ws, b), b & 31);
+  load_cost<ROWS>(A, b, Q);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, A.ws, b), b & 31);
   double s0[6], cf[kMaxCoef];
   load_state6(A, b, s0);
   load_coeffs(A, b, cf);
@@ -195,15 +221,15 @@ __global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant_
   if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);   // invalid number at the starting point
 }
 
-template <bool WIO, bool COST>
-__global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
+template <bool WIO, int ROWS>
+__global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
   Params Q = P;
-  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, slot), slot & 31);
   if (S.load_phase() != PH_FACTOR) return;
-  load_cost<COST>(A, b, Q);
+  load_cost<ROWS>(A, b, Q);
   __shared__ double stage[2 * kStageVals * kBlock];   // [buffer][value][thread]
   S.sb = stage + threadIdx.x; S.sbs = kBlock;
   load_coeffs(A, b, S.cf);
@@ -214,32 +240,32 @@ __global__ void __launch_bounds__(kBlock, kFactorBlocks) mpc_factor_kernel(const
   }
 }
 
-template <bool COST>
-__global__ void __launch_bounds__(kBlock, kFwdBlocks) mpc_forward_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
+template <int ROWS>
+__global__ void __launch_bounds__(kBlock, kFwdBlocks) mpc_forward_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
   Params Q = P;
-  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, slot), slot & 31);
   if (S.load_phase() != PH_FORWARD) return;
-  load_cost<COST>(A, b, Q);
+  load_cost<ROWS>(A, b, Q);
   load_coeffs(A, b, S.cf);
   S.kernel_forward();
 }
 
-template <bool WIO, bool COST>
-__global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A) {
+template <bool WIO, int ROWS>
+__global__ void __launch_bounds__(kBlock, kStepBlocks) mpc_step_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws)) return;
   Params Q = P;
-  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, slot), slot & 31);
   const int ph = S.load_phase();
   if (ph != PH_STEP) {
     if (A.count_live && ph != PH_DONE) count_live(A.desc + kLive);
     return;
   }
-  load_cost<COST>(A, b, Q);
+  load_cost<ROWS>(A, b, Q);
   double carry[kCarry];
   S.cr = carry; S.cs = 1;
   __shared__ double stage[2 * kStepStageVals * kBlock];   // [buffer][value][thread]
@@ -309,14 +335,14 @@ __global__ void mpc_tail_reset_kernel(int* t_desc) {
 }
 
 // ---- fused kernel: finishes whatever is still active (fresh == 1: starts from the inputs) ---------------------
-template <bool WIO, bool COST>
-__global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A, int fresh) {
+template <bool WIO, int ROWS>
+__global__ void __launch_bounds__(kBlock) mpc_fused_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A, int fresh) {
   int slot, b;
   double* ws;
   if (!locate(A, blockIdx.x * blockDim.x + threadIdx.x, slot, b, ws, false)) return;
   Params Q = P;
-  load_cost<COST>(A, b, Q);
-  Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
+  load_cost<ROWS>(A, b, Q);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, slot), slot & 31);
   double carry[kCarry];
   S.cr = carry; S.cs = 1;
   load_coeffs(A, b, S.cf);
@@ -349,8 +375,8 @@ struct DevExec {
 // take_below > 0: conditional hand-over after a round -- the kernel acts only once the batch has been compacted to at
 // most take_below occupied slots (two waves of the cooperative kernel); from then on the sweeps of later rounds find
 // nothing to do
-template <bool WIO, bool COST>
-__global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<COST> A, int fresh,
+template <bool WIO, int ROWS>
+__global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ Params P, const __grid_constant__ ArgsT<ROWS> A, int fresh,
                                                        int warps_per_block, int doubles_per_warp, int take_below) {
   extern __shared__ double coop_smem[];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -369,8 +395,8 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
     double* ws;
     if (!locate(A, idx, slot, b, ws, false)) return;
     Params Q = P;
-    load_cost<COST>(A, b, Q);
-    Solver<32> S(COST ? Q : P, slot_base(P, ws, slot), slot & 31);
+    load_cost<ROWS>(A, b, Q);
+    Solver<32> S(ROWS ? Q : P, slot_base(P, ws, slot), slot & 31);
     load_coeffs(A, b, S.cf);
     CoopSolver<32, DevExec> C(S, st, pub, DevExec{lane});
     if (fresh) {
@@ -396,9 +422,10 @@ __global__ void __launch_bounds__(128) mpc_coop_kernel(const __grid_constant__ P
 constexpr size_t kCoopSmemMax = 200 * 1024;   // dynamic shared memory of one cooperative block, at most
 // per-device, once (b200mpc_create)
 cudaError_t solver_prepare_device() {
-  cudaError_t e = cudaFuncSetAttribute(mpc_coop_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  cudaError_t e = cudaFuncSetAttribute(mpc_coop_kernel<false, kNoRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, kNoRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, kCostRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_coop_kernel<true, kModelRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCoopSmemMax);
   return e;
 }
 
@@ -441,19 +468,29 @@ static CostArgs solve_args(int B, int steps, const SolveIO& io, const WsLayout& 
   A.ws = L.ws0; A.ws1 = L.ws1; A.map0 = L.map0; A.map1 = L.map1; A.desc = desc;
   A.out8 = io.out8; A.traj = io.traj; A.obj = io.obj; A.status = io.status; A.iters = io.iters;
   A.x_init = io.x_init; A.mult_init = io.mult_init; A.mu_init = io.mu_init; A.mult = io.mult;
-  A.cost8 = io.cost8;
+  A.cost8 = io.cost8; A.model4 = io.model4;
   return A;
 }
 
 static int sweep_grid(const SolveArgs& A) { return (A.b1 - A.b0 + kBlock - 1) / kBlock; }
-// the call reads a start point or writes multipliers: the WIO = true kernel instances.  A call with per-problem costs
-// runs the <true, true> instances (null x_init / mult do nothing there); the others get the SolveArgs part of A.
+// the call reads a start point or writes multipliers: the WIO = true kernel instances.  A call with per-problem cost or
+// model rows runs the <true, kCostRows> or <true, kModelRows> instances (null x_init / mult do nothing there); the others
+// get the SolveArgs part of A.
 static bool warm_io(const SolveArgs& A) { return A.x_init != nullptr || A.mult != nullptr; }
+static int rows_of(const CostArgs& A) { return A.model4 ? kModelRows : (A.cost8 ? kCostRows : kNoRows); }
 static void launch_init(const Params& P, const CostArgs& A, cudaStream_t stream, long long* n) {
-  if (A.cost8) mpc_init_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  else if (warm_io(A)) mpc_init_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-  else mpc_init_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  if (rows_of(A) == kModelRows) mpc_init_kernel<true, kModelRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else if (rows_of(A) == kCostRows) mpc_init_kernel<true, kCostRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else if (warm_io(A)) mpc_init_kernel<true, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  else mpc_init_kernel<false, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
   *n += 1;
+}
+
+template <int R>
+static void launch_round_rows(const Params& P, const CostArgs& A, const CostArgs& As, cudaStream_t stream) {
+  mpc_factor_kernel<true, R><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  mpc_forward_kernel<R><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+  mpc_step_kernel<true, R><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
 }
 
 // The launch helpers add one to *n per kernel they launch.  launch_round: one round of the thread-per-problem sweeps;
@@ -461,16 +498,16 @@ static void launch_init(const Params& P, const CostArgs& A, cudaStream_t stream,
 static void launch_round(const Params& P, const CostArgs& A, bool count_live, cudaStream_t stream, long long* n) {
   CostArgs As = A;
   As.count_live = count_live ? 1 : 0;
-  if (A.cost8) {
-    mpc_factor_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-    mpc_forward_kernel<true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-    mpc_step_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+  if (rows_of(A) == kModelRows) {
+    launch_round_rows<kModelRows>(P, A, As, stream);
+  } else if (rows_of(A) == kCostRows) {
+    launch_round_rows<kCostRows>(P, A, As, stream);
   } else {
-    if (warm_io(A)) mpc_factor_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-    else mpc_factor_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-    mpc_forward_kernel<false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
-    if (warm_io(A)) mpc_step_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
-    else mpc_step_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+    if (warm_io(A)) mpc_factor_kernel<true, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    else mpc_factor_kernel<false, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    mpc_forward_kernel<kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A);
+    if (warm_io(A)) mpc_step_kernel<true, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
+    else mpc_step_kernel<false, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, As);
   }
   *n += 3;
 }
@@ -483,9 +520,10 @@ static void launch_repack(const Params& P, const SolveArgs& A, double max_live, 
 }
 
 static void launch_fused(const Params& P, const CostArgs& A, int fresh, cudaStream_t stream, long long* n) {
-  if (A.cost8) mpc_fused_kernel<true, true><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
-  else if (warm_io(A)) mpc_fused_kernel<true, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
-  else mpc_fused_kernel<false, false><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  if (rows_of(A) == kModelRows) mpc_fused_kernel<true, kModelRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else if (rows_of(A) == kCostRows) mpc_fused_kernel<true, kCostRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else if (warm_io(A)) mpc_fused_kernel<true, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
+  else mpc_fused_kernel<false, kNoRows><<<sweep_grid(A), kBlock, 0, stream>>>(P, A, fresh);
   *n += 1;
 }
 
@@ -501,9 +539,10 @@ static bool launch_coop(const Params& P, const CostArgs& A, int fresh, int take_
   if (cap > 0 && grid > cap) grid = cap;
   // no idle warps: their registers would stay allocated
   const int dpw = (int)coop_doubles_per_warp(P.N);
-  if (A.cost8) mpc_coop_kernel<true, true><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
-  else if (warm_io(A)) mpc_coop_kernel<true, false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
-  else mpc_coop_kernel<false, false><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  if (rows_of(A) == kModelRows) mpc_coop_kernel<true, kModelRows><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  else if (rows_of(A) == kCostRows) mpc_coop_kernel<true, kCostRows><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  else if (warm_io(A)) mpc_coop_kernel<true, kNoRows><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
+  else mpc_coop_kernel<false, kNoRows><<<grid, 32 * wpb, c.smem, stream>>>(P, A, fresh, wpb, dpw, take_below);
   *n += 1;
   *err = cudaGetLastError();
   return true;
@@ -652,30 +691,44 @@ cudaError_t launch_solve_tail(const Params& P, int B, const SolveIO& io, const T
 
 // ---------------------------------------------------------------------------------------------
 // Adjoint sensitivities of returned solutions (Solver::vjp): one thread per problem, workspace region 0 (slot = problem).
-// state6 / coeffs / g_out8 / the three gradients (and cost8, COST = true) in the layout io_aos selects, traj / mult /
-// g_traj field-major.
-template <bool COST>
-using VjpArgsT = typename std::conditional<COST, VjpCostIO, VjpIO>::type;
-template <bool COST>
-__global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__ Params P, const __grid_constant__ VjpArgsT<COST> A, double* ws) {
+// state6 / coeffs / g_out8 / the gradients (and cost8 / model4, ROWS != kNoRows) in the layout io_aos selects, traj / mult
+// / g_traj field-major.  The kModelRows instance also returns grad_model, at the model row or at the handle's values.
+template <int ROWS>
+using VjpArgsT = typename std::conditional<ROWS != kNoRows, VjpCostIO, VjpIO>::type;
+template <int ROWS>
+__global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__ Params P, const __grid_constant__ VjpArgsT<ROWS> A, double* ws) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= A.B) return;
   const size_t nb = (size_t)A.B, bb = (size_t)b;
   auto at = [&](int k, int n) { return A.io_aos ? bb * n + k : (size_t)k * nb + bb; };   // element k of n of problem b
   Params Q = P;
-  Solver<32> S(COST ? Q : P, slot_base(P, ws, b), b & 31);
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, b), b & 31);
   double s0[6], cf[kMaxCoef], gs6[6], gcf[kMaxCoef], gpar[8];
 #pragma unroll
   for (int k = 0; k < 6; ++k) s0[k] = A.state6[at(k, 6)];
 #pragma unroll
   for (int i = 0; i < kMaxCoef; ++i) cf[i] = i < A.ncoef ? A.coeffs[at(i, A.ncoef)] : 0.0;
-  // a non-finite cost row: a NaN coefficient makes Solver::vjp return -13 with NaN gradients
-  if constexpr (COST) {
+  // an invalid cost or model row: a NaN coefficient makes Solver::vjp return -13 with NaN gradients
+  if constexpr (ROWS == kCostRows) {
     if (!cost_row(A.cost8, A.io_aos, A.B, b, Q)) cf[0] = NAN;
+  } else if constexpr (ROWS == kModelRows) {
+    bool ok = !A.cost8 || cost_row(A.cost8, A.io_aos, A.B, b, Q);
+    if (A.model4) ok &= model_row(A.model4, A.io_aos, A.B, b, Q);
+    if (!ok) cf[0] = NAN;
   }
   S.set_coeffs(cf, kMaxCoef);
-  const int st = S.vjp(s0, A.traj + b, nb, A.mult + b, nb, A.g_out8 ? A.g_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb,
-                       A.g_traj ? A.g_traj + b : nullptr, nb, A.g_obj ? A.g_obj[b] : 0.0, gs6, gcf, gpar);
+  int st;
+  if constexpr (ROWS == kModelRows) {
+    double gmod[4];
+    st = S.vjp<true>(s0, A.traj + b, nb, A.mult + b, nb, A.g_out8 ? A.g_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb,
+                     A.g_traj ? A.g_traj + b : nullptr, nb, A.g_obj ? A.g_obj[b] : 0.0, gs6, gcf, gpar, gmod);
+    if (A.grad_model)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) A.grad_model[at(i, 4)] = gmod[i];
+  } else {
+    st = S.vjp(s0, A.traj + b, nb, A.mult + b, nb, A.g_out8 ? A.g_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb,
+               A.g_traj ? A.g_traj + b : nullptr, nb, A.g_obj ? A.g_obj[b] : 0.0, gs6, gcf, gpar);
+  }
   if (A.grad_state6)
 #pragma unroll
     for (int k = 0; k < 6; ++k) A.grad_state6[at(k, 6)] = gs6[k];
@@ -690,8 +743,10 @@ __global__ void __launch_bounds__(kBlock) mpc_vjp_kernel(const __grid_constant__
 }
 cudaError_t launch_vjp(const Params& P, const VjpCostIO& io, double* ws, cudaStream_t stream) {
   if (io.B <= 0) return cudaSuccess;
-  if (io.cost8) mpc_vjp_kernel<true><<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
-  else mpc_vjp_kernel<false><<<(io.B + kBlock - 1) / kBlock, kBlock, 0, stream>>>(P, io, ws);
+  const int grid = (io.B + kBlock - 1) / kBlock;
+  if (io.model4 || io.grad_model) mpc_vjp_kernel<kModelRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
+  else if (io.cost8) mpc_vjp_kernel<kCostRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
+  else mpc_vjp_kernel<kNoRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
   return cudaGetLastError();
 }
 
