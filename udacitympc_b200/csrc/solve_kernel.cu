@@ -214,11 +214,13 @@ __global__ void __launch_bounds__(kBlock) mpc_init_kernel(const __grid_constant_
   double s0[6], cf[kMaxCoef];
   load_state6(A, b, s0);
   load_coeffs(A, b, cf);
+  const bool cold = !(A.warm && A.step > 0) && !(WIO && A.x_init);
   if (A.warm && A.step > 0) { S.set_coeffs(cf, A.ncoef); S.init_warm(s0, A.mu_warm); }
   else if (WIO && A.x_init) { S.set_coeffs(cf, A.ncoef); S.init_guess(s0, A.x_init + b, (size_t)A.B, guess_mult(A, b), (size_t)A.B, A.mu_init); }
   else S.init(s0, cf, A.ncoef);
   S.store_state();
-  if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);   // invalid number at the starting point
+  if (cold && S.phase == PH_FACTOR) S.kernel_ls_round(s0);   // the sweeps start at the first Newton round
+  if (S.phase == PH_DONE) write_result<WIO>(P, A, b, S);   // invalid number at the starting point, or converged there
 }
 
 template <bool WIO, int ROWS>
