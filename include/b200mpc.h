@@ -257,6 +257,36 @@ int b200mpc_solve_batch_vjp_model_device(b200mpc_handle* h, int B, const double*
                                          double* d_grad_state6, double* d_grad_coeffs, double* d_grad_params,
                                          double* d_grad_model, int* d_status, void* stream);
 
+/* Forward sensitivities (Jacobian-vector product) of B solutions: the derivative of each problem's solution (out8, traj,
+ * obj) along a tangent of its inputs -- initial state, reference polynomial, cost parameters and vehicle model -- by the
+ * implicit-function theorem at the returned primal-dual point: K [dx; dlam] = -dF/dtheta dtheta with the KKT matrix K of
+ * b200mpc_solve_batch_vjp (the transpose of that call: <v, J u> from this call equals <J^T v, u> from it up to
+ * rounding).  NOT reference behaviour: the reference returns no derivatives.  One Riccati solve of the KKT system of the
+ * unscaled problem per problem and tangent, one kernel launch.
+ *   state6, coeffs, cost8, model4, traj, mult   as for b200mpc_solve_batch_vjp_model (cost8 / model4 may be NULL: the
+ *                    handle's values)
+ *   t_state6 (B x 6), t_coeffs (B x ncoef), t_cost8 (B x 8), t_model4 (B x 4)   the tangent, in the orders of state6,
+ *                    coeffs, cost8 and model4, or NULL for zero; at least one must be given.  t_model4 with model4 NULL
+ *                    is taken at the handle's values.
+ *   t_out8 (B x 8), t_traj (B x (8N-2))   d out8, d traj, or NULL.  t_traj's states of t = 0 are t_state6; t_out8 is
+ *                    t_traj's state of t = 1 and controls of t = 0.  Controls are not clamped to the bounds as traj's are.
+ *   t_obj (B) or NULL   d obj in the envelope form df/dtheta + lambda^T dc/dtheta (bound terms included), the exact
+ *                    transpose of g_obj's term of the VJP; it agrees with grad f . dx + df/dtheta to the solver tolerance.
+ *   status (B) or NULL: as b200mpc_solve_batch_vjp (a non-finite tangent also gives -13); the outputs are NaN then.
+ * B200MPC_ERR_ARG for a null handle, B <= 0, ncoef outside [2, 4], a null state6 / coeffs / traj / mult or no tangent.
+ * The call uses the handle's workspace and is ordered like a solve on the handle. */
+int b200mpc_solve_batch_jvp(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                            const double* model4, const double* traj, const double* mult, const double* t_state6,
+                            const double* t_coeffs, const double* t_cost8, const double* t_model4, double* t_out8,
+                            double* t_traj, double* t_obj, int* status);
+/* Same on device buffers, field-major like b200mpc_solve_batch_vjp_device (d_x[i*B+b] for every array), asynchronous on
+ * `stream` (NULL: the handle's stream).  Exactly one kernel launch. */
+int b200mpc_solve_batch_jvp_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                   const double* d_cost8, const double* d_model4, const double* d_traj, const double* d_mult,
+                                   const double* d_t_state6, const double* d_t_coeffs, const double* d_t_cost8,
+                                   const double* d_t_model4, double* d_t_out8, double* d_t_traj, double* d_t_obj, int* d_status,
+                                   void* stream);
+
 /* Warm start for b200mpc_closed_loop_batch (SURVEY 8f; NOT reference behaviour: the reference cold-starts every call,
  * MPC.cpp:167-177, and so does this library unless enabled here).  When enabled, every step after the first starts from
  * the previous step's solution shifted by one stage, with the barrier parameter at mu_init (e.g. 1e-4).  The optimum

@@ -55,6 +55,8 @@ SYMBOLS = {
     "b200mpc_solve_batch_vjp": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
                                                _ip]),
     "b200mpc_solve_batch_vjp_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 10),
+    "b200mpc_solve_batch_jvp": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, ctypes.c_int] + [_dp] * 11 + [_ip]),
+    "b200mpc_solve_batch_jvp_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int] + [_vp] * 13),
     "b200mpc_solve_batch_multi": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int,
                                                  _dp, _dp, _dp, _ip, _ip]),
     "b200mpc_closed_loop_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _dp, _dp, ctypes.c_int, _dp, _dp, _ip]),
@@ -423,6 +425,60 @@ class MPC:
                                                               d_g_traj or None, d_g_obj or None, d_grad_state6 or None,
                                                               d_grad_coeffs or None, d_grad_params or None,
                                                               d_grad_model or None, d_status or None, stream or None))
+
+    def solve_batch_jvp(self, states, coeffs, traj, mult, t_state6=None, t_coeffs=None, t_cost=None, t_model=None,
+                        cost_params=None, model_params=None):
+        """Forward sensitivities of solutions (b200mpc_solve_batch_jvp; not reference behaviour): the derivative of each
+        problem's (out8, traj, obj) along the tangent t_state6 (B,6), t_coeffs (B,ncoef) or (ncoef,), t_cost (B,8) or (8,)
+        in the order PARAM_NAMES, t_model (B,4) or (4,) in the order MODEL_NAMES -- any of them None (zero), not all.
+        Returns dict(t_out8 (B,8), t_traj (B,8N-2), t_obj (B,), status (B,)).  states, coeffs, traj, mult, cost_params
+        and model_params as for solve_batch_vjp; t_cost / t_model are w.r.t. the per-problem rows or, without them, the
+        handle's values."""
+        states = _f64(states)
+        if states.ndim != 2 or states.shape[1] != 6:
+            raise ValueError("states must be (B, 6)")
+        B = states.shape[0]
+        coeffs = _f64(coeffs)
+        if coeffs.ndim == 1:
+            coeffs = np.ascontiguousarray(np.broadcast_to(coeffs, (B, coeffs.size)))
+        if coeffs.ndim != 2 or coeffs.shape[0] != B:
+            raise ValueError("coeffs must be (B, ncoef) or (ncoef,)")
+        ncoef = coeffs.shape[1]
+        traj = _f64(traj, (B, self.num_vars))
+        mult = _f64(mult, (B, self.num_mults))
+        if t_state6 is not None:
+            t_state6 = _f64(t_state6)
+            if t_state6.shape != (B, 6):
+                raise ValueError("t_state6 must be (B, 6)")
+        if t_coeffs is not None:
+            t_coeffs = _f64(t_coeffs)
+            if t_coeffs.ndim == 1:
+                t_coeffs = np.broadcast_to(t_coeffs, (B, t_coeffs.size))
+            if t_coeffs.shape != (B, ncoef):
+                raise ValueError("t_coeffs must be (B, ncoef) or (ncoef,), ncoef as coeffs")
+            t_coeffs = np.ascontiguousarray(t_coeffs)
+        t_cost = None if t_cost is None else _cost8(t_cost, B)
+        t_model = None if t_model is None else _model4(t_model, B)
+        c8 = None if cost_params is None else _cost8(cost_params, B)
+        m4 = None if model_params is None else _model4(model_params, B)
+        t_out8, t_traj, t_obj = np.empty((B, 8)), np.empty((B, self.num_vars)), np.empty(B)
+        status = np.empty(B, dtype=np.int32)
+        opt = lambda a: None if a is None else _ptr(a)
+        _check(self._lib.b200mpc_solve_batch_jvp(
+            self._h, B, _ptr(states), _ptr(coeffs), ncoef, opt(c8), opt(m4), _ptr(traj), _ptr(mult), opt(t_state6),
+            opt(t_coeffs), opt(t_cost), opt(t_model), _ptr(t_out8), _ptr(t_traj), _ptr(t_obj), status.ctypes.data_as(_ip)))
+        return dict(t_out8=t_out8, t_traj=t_traj, t_obj=t_obj, status=status)
+
+    def solve_batch_jvp_device(self, B, d_state6, d_coeffs, ncoef, d_cost8, d_model4, d_traj, d_mult, d_t_state6=0,
+                               d_t_coeffs=0, d_t_cost8=0, d_t_model4=0, d_t_out8=0, d_t_traj=0, d_t_obj=0, d_status=0,
+                               stream=0):
+        """Raw device-pointer JVP (integers, 0 = none), field-major buffers, d_cost8 [8][B], d_model4 / d_t_model4 [4][B];
+        one kernel launch, asynchronous on `stream`.  See b200mpc_solve_batch_jvp_device."""
+        _check(self._lib.b200mpc_solve_batch_jvp_device(self._h, B, d_state6, d_coeffs, ncoef, d_cost8 or None,
+                                                        d_model4 or None, d_traj, d_mult, d_t_state6 or None,
+                                                        d_t_coeffs or None, d_t_cost8 or None, d_t_model4 or None,
+                                                        d_t_out8 or None, d_t_traj or None, d_t_obj or None,
+                                                        d_status or None, stream or None))
 
     def wait(self):
         """Waits for everything queued on this handle's own stream (b200mpc_solve_batch_async calls)."""

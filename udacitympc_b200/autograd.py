@@ -5,7 +5,8 @@
 The forward pass is one batched solve (b200mpc_solve_batch_warm[_device] from the default start point, which also
 returns the multipliers); the backward pass is one adjoint solve at that solution (b200mpc_solve_batch_vjp[_device]).
 With cost_params the two calls are b200mpc_solve_batch_cost[_device] and b200mpc_solve_batch_vjp_cost[_device], with
-model_params b200mpc_solve_batch_model[_device] and b200mpc_solve_batch_vjp_model[_device].
+model_params b200mpc_solve_batch_model[_device] and b200mpc_solve_batch_vjp_model[_device].  Forward-mode AD
+(torch.autograd.forward_ad) runs one tangent solve at the solution (b200mpc_solve_batch_jvp[_device]).
 CUDA tensors stay on the device and run on torch's current stream of their device, which must be the MPC handle's
 device; CPU tensors go through the host entry points.  The only module of the package that imports torch.
 """
@@ -84,6 +85,7 @@ class _Solve(torch.autograd.Function):
         ctx.cost_shared = cost_params is not None and cost_params.dim() == 1
         ctx.model_shared = model_params is not None and model_params.dim() == 1
         ctx.save_for_backward(st, cf, traj, mult, status, c8, m4)
+        ctx.save_for_forward(st, cf, traj, mult, status, c8, m4)
         ctx.mark_non_differentiable(status)
         dt = states.dtype
         return out8.to(dt), traj.to(dt), obj.to(dt), status
@@ -151,6 +153,40 @@ class _Solve(torch.autograd.Function):
             gm = gm.to(ctx.dtypes[3])
         return None, gs.to(ctx.dtypes[0]), gc.to(ctx.dtypes[1]), gp, gm
 
+    @staticmethod
+    def jvp(ctx, _t_mpc, t_states, t_coeffs, t_cost, t_model):
+        st, cf, traj, mult, status, c8, m4 = ctx.saved_tensors
+        mpc = ctx.mpc
+        B, ncoef = cf.shape
+        shapes = ((B, 6), (B, ncoef), (B, 8), (B, 4))
+        t = [None if v is None else v.detach().to(torch.float64).expand(*s) for v, s in
+             zip((t_states, t_coeffs, t_cost, t_model), shapes)]
+        dt = ctx.dtypes[0]
+        # the derivative exists only at a converged solution.  The tangents are masked in place and keep the layout of
+        # their primal outputs (on CUDA, transposes of field-major buffers), which forward-mode AD requires.
+        bad = ~((status == 0) | (status == 1))
+        nan = float("nan")
+        if st.is_cuda:
+            dev = st.device
+            to8 = torch.empty(8, B, dtype=torch.float64, device=dev)
+            tt = torch.empty(mpc.num_vars, B, dtype=torch.float64, device=dev)
+            tob = torch.empty(B, dtype=torch.float64, device=dev)
+            vs = torch.empty(B, dtype=torch.int32, device=dev)
+            keep = [_fields(st), _fields(cf), None if c8 is None else _fields(c8), None if m4 is None else _fields(m4),
+                    traj.t().contiguous(), mult.t().contiguous()] + [None if v is None else _fields(v) for v in t]
+            mpc.solve_batch_jvp_device(B, _ptr(keep[0]), _ptr(keep[1]), ncoef, *[_ptr(k) for k in keep[2:]], _ptr(to8),
+                                       _ptr(tt), _ptr(tob), _ptr(vs), _stream(dev))
+            to8, tt = to8.masked_fill_(bad[None, :], nan).t(), tt.masked_fill_(bad[None, :], nan).t()
+        else:
+            r = mpc.solve_batch_jvp(st.numpy(), cf.contiguous().numpy(), traj.numpy(), mult.numpy(),
+                                    *[None if v is None else v.contiguous().numpy() for v in t],
+                                    cost_params=None if c8 is None else c8.contiguous().numpy(),
+                                    model_params=None if m4 is None else m4.contiguous().numpy())
+            to8, tt, tob = (torch.from_numpy(r[k]) for k in ("t_out8", "t_traj", "t_obj"))
+            to8, tt = to8.masked_fill_(bad[:, None], nan), tt.masked_fill_(bad[:, None], nan)
+        tob.masked_fill_(bad, nan)
+        return to8.to(dt), tt.to(dt), tob.to(dt), None
+
 
 def solve(mpc, states, coeffs, cost_params=None, model_params=None):
     """Differentiable batched solve on the MPC handle `mpc`: states (B, 6), coeffs (B, ncoef) or (ncoef,) shared by all
@@ -160,5 +196,8 @@ def solve(mpc, states, coeffs, cost_params=None, model_params=None):
     obj (B,), status (B,) int32, not differentiable).  Backpropagating into states / coeffs / cost_params runs one
     adjoint solve (MPC.solve_batch_vjp); problems whose status is not 0 or 1 get NaN gradients, and gradients of shared
     coeffs / cost_params are summed over the batch.  model_params (B, 4) or (4,) shared, in the order MODEL_NAMES (dt, Lf,
-    delta_max, a_max), likewise replaces the handle's vehicle model and actuator limits and is differentiated."""
+    delta_max, a_max), likewise replaces the handle's vehicle model and actuator limits and is differentiated.
+    Forward-mode AD (torch.autograd.forward_ad) through the solve runs one tangent solve (MPC.solve_batch_jvp) per
+    call: tangents of out8, traj and obj, NaN for problems whose status is not 0 or 1; tangents of shared coeffs /
+    cost_params / model_params apply to every problem."""
     return _Solve.apply(mpc, states, coeffs, cost_params, model_params)

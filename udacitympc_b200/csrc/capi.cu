@@ -244,13 +244,14 @@ int timed_solve(b200mpc_handle* h, int B, int steps, const SolveIO& io, cudaStre
   return rc;
 }
 
-// One adjoint launch (b200mpc_solve_batch_vjp*) on stream s.  It uses the handle's workspace, so it is ordered like a plain
-// solve in timed_solve: after everything queued on this handle, pipelined tails included, and before the next call.
-int run_vjp(b200mpc_handle* h, const VjpCostIO& io, cudaStream_t s) {
+// One sensitivity launch (b200mpc_solve_batch_vjp*, b200mpc_solve_batch_jvp*) of B problems on stream s.  It uses the
+// handle's workspace, so it is ordered like a plain solve in timed_solve: after everything queued on this handle,
+// pipelined tails included, and before the next call.
+int run_sens(b200mpc_handle* h, int B, cudaStream_t s, const std::function<cudaError_t(double*)>& launch) {
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   if (s != nullptr && s != cudaStreamLegacy) { if (cudaStreamIsCapturing(s, &cap) != cudaSuccess) { cudaGetLastError(); cap = cudaStreamCaptureStatusNone; } }
   const bool caller_captures = cap != cudaStreamCaptureStatusNone;
-  const size_t need = solve_workspace_doubles(h->P.N, io.B) * sizeof(double);
+  const size_t need = solve_workspace_doubles(h->P.N, B) * sizeof(double);
   if (caller_captures && h->ws.cap < need)
     return fail(B200MPC_ERR_ARG, "the stream is being captured and the workspace would have to grow: run one solve of this size first");
   for (int k = 0; k < h->pipe_depth; ++k)
@@ -259,13 +260,19 @@ int run_vjp(b200mpc_handle* h, const VjpCostIO& io, cudaStream_t s) {
   if (h->ws.cap < need && h->pipe_calls) CU(cudaDeviceSynchronize());
   CU(h->ws.ensure(need));
   if (!caller_captures && h->done_valid) CU(cudaStreamWaitEvent(s, h->done, 0));
-  CU(launch_vjp(h->P, io, h->ws.as<double>(), s));
+  CU(launch(h->ws.as<double>()));
   h->launches += 1;
   if (!caller_captures) {
     CU(cudaEventRecord(h->done, s));
     h->done_valid = true;
   }
   return 0;
+}
+int run_vjp(b200mpc_handle* h, const VjpCostIO& io, cudaStream_t s) {
+  return run_sens(h, io.B, s, [&](double* ws) { return launch_vjp(h->P, io, ws, s); });
+}
+int run_jvp(b200mpc_handle* h, const JvpIO& io, cudaStream_t s) {
+  return run_sens(h, io.B, s, [&](double* ws) { return launch_jvp(h->P, io, ws, s); });
 }
 
 int check_vjp_args(const b200mpc_handle* h, int B, const void* st, const void* cf, int ncoef, const void* traj, const void* mult,
@@ -275,6 +282,17 @@ int check_vjp_args(const b200mpc_handle* h, int B, const void* st, const void* c
   if (ncoef < 2 || ncoef > B200MPC_MAX_COEFFS) return fail(B200MPC_ERR_ARG, "ncoef must be in [2, 4] (polynomial degree 1..3)");
   if (!st || !cf || !traj || !mult) return fail(B200MPC_ERR_ARG, "vjp: null state6 / coeffs / traj / mult");
   if (!g_out8 && !g_traj && !g_obj) return fail(B200MPC_ERR_ARG, "vjp: no incoming gradient (g_out8, g_traj and g_obj are all null)");
+  return 0;
+}
+
+int check_jvp_args(const b200mpc_handle* h, int B, const void* st, const void* cf, int ncoef, const void* traj, const void* mult,
+                   const void* t_st, const void* t_cf, const void* t_c8, const void* t_m4) {
+  if (!h) return fail(B200MPC_ERR_ARG, "null handle");
+  if (B <= 0) return fail(B200MPC_ERR_ARG, "jvp: B must be positive");
+  if (ncoef < 2 || ncoef > B200MPC_MAX_COEFFS) return fail(B200MPC_ERR_ARG, "ncoef must be in [2, 4] (polynomial degree 1..3)");
+  if (!st || !cf || !traj || !mult) return fail(B200MPC_ERR_ARG, "jvp: null state6 / coeffs / traj / mult");
+  if (!t_st && !t_cf && !t_c8 && !t_m4)
+    return fail(B200MPC_ERR_ARG, "jvp: no tangent (t_state6, t_coeffs, t_cost8 and t_model4 are all null)");
   return 0;
 }
 
@@ -741,6 +759,76 @@ int b200mpc_solve_batch_vjp_model(b200mpc_handle* h, int B, const double* state6
   if (grad_coeffs) CU(cudaMemcpyAsync(grad_coeffs, io.grad_coeffs, nb * ncoef * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (grad_params) CU(cudaMemcpyAsync(grad_params, io.grad_params, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (grad_model) CU(cudaMemcpyAsync(grad_model, io.grad_model, nb * 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (status) CU(cudaMemcpyAsync(status, h->status.p, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  return 0;
+}
+
+int b200mpc_solve_batch_jvp_device(b200mpc_handle* h, int B, const double* d_state6, const double* d_coeffs, int ncoef,
+                                   const double* d_cost8, const double* d_model4, const double* d_traj, const double* d_mult,
+                                   const double* d_t_state6, const double* d_t_coeffs, const double* d_t_cost8,
+                                   const double* d_t_model4, double* d_t_out8, double* d_t_traj, double* d_t_obj, int* d_status,
+                                   void* stream) {
+  if (int rc = check_jvp_args(h, B, d_state6, d_coeffs, ncoef, d_traj, d_mult, d_t_state6, d_t_coeffs, d_t_cost8, d_t_model4))
+    return rc;
+  CU(cudaSetDevice(h->device));
+  JvpIO io;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 0;
+  io.state6 = d_state6; io.coeffs = d_coeffs; io.cost8 = d_cost8; io.model4 = d_model4; io.traj = d_traj; io.mult = d_mult;
+  io.t_state6 = d_t_state6; io.t_coeffs = d_t_coeffs; io.t_cost8 = d_t_cost8; io.t_model4 = d_t_model4;
+  io.t_out8 = d_t_out8; io.t_traj = d_t_traj; io.t_obj = d_t_obj; io.status = d_status;
+  return run_jvp(h, io, stream ? (cudaStream_t)stream : h->stream);
+}
+
+// Host buffers: the per-problem inputs, their tangents and t_out8 / t_obj are read and written per problem by the kernel
+// (io_aos = 1); traj / mult go in and t_traj comes out through the tiled transposes.
+int b200mpc_solve_batch_jvp(b200mpc_handle* h, int B, const double* state6, const double* coeffs, int ncoef, const double* cost8,
+                            const double* model4, const double* traj, const double* mult, const double* t_state6,
+                            const double* t_coeffs, const double* t_cost8, const double* t_model4, double* t_out8,
+                            double* t_traj, double* t_obj, int* status) {
+  if (int rc = check_jvp_args(h, B, state6, coeffs, ncoef, traj, mult, t_state6, t_coeffs, t_cost8, t_model4)) return rc;
+  CU(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  const size_t nb = (size_t)B, nv = 8 * (size_t)h->P.N - 2, nm = 10 * (size_t)h->P.N - 4;
+  // rows: traj | mult in, then t_traj out (its transpose reuses the input rows, which are consumed by then)
+  CU(h->vjp_aos.ensure(nb * (nv + nm) * sizeof(double)));
+  CU(h->vjp_soa.ensure(nb * (nv + nm + (t_traj ? nv : 0)) * sizeof(double)));
+  // per problem: t_state6 (6) | t_coeffs (ncoef) | t_cost8 (8) | t_model4 (4) | t_out8 (8) | t_obj (1)
+  CU(h->vjp_io.ensure(nb * (27 + ncoef) * sizeof(double)));
+  CU(h->status.ensure(nb * sizeof(int)));
+  SolveIO in;
+  if (int rc = stage_inputs(h, B, state6, coeffs, ncoef, &in, cost8, model4)) return rc;
+  double *ga = h->vjp_aos.as<double>(), *gs = h->vjp_soa.as<double>(), *d = h->vjp_io.as<double>();
+  CU(cudaMemcpyAsync(ga, traj, nb * nv * sizeof(double), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(ga + nb * nv, mult, nb * nm * sizeof(double), cudaMemcpyHostToDevice, s));
+  CU(launch_aos_to_soa(ga, gs, B, (int)nv, s));
+  CU(launch_aos_to_soa(ga + nb * nv, gs + nb * nv, B, (int)nm, s));
+  h->launches += 2;
+  const double* tin[4] = {t_state6, t_coeffs, t_cost8, t_model4};
+  const size_t tlen[4] = {6, (size_t)ncoef, 8, 4};
+  const double* tdev[4] = {nullptr, nullptr, nullptr, nullptr};
+  size_t off = 0;
+  for (int i = 0; i < 4; ++i) {
+    if (tin[i]) {
+      CU(cudaMemcpyAsync(d + nb * off, tin[i], nb * tlen[i] * sizeof(double), cudaMemcpyHostToDevice, s));
+      tdev[i] = d + nb * off;
+    }
+    off += tlen[i];
+  }
+  JvpIO io;
+  io.B = B; io.ncoef = ncoef; io.io_aos = 1;
+  io.state6 = in.state6; io.coeffs = in.coeffs; io.cost8 = in.cost8; io.model4 = in.model4; io.traj = gs; io.mult = gs + nb * nv;
+  io.t_state6 = tdev[0]; io.t_coeffs = tdev[1]; io.t_cost8 = tdev[2]; io.t_model4 = tdev[3];
+  io.t_out8 = d + nb * off; io.t_obj = d + nb * (off + 8); io.t_traj = t_traj ? gs + nb * (nv + nm) : nullptr;
+  io.status = h->status.as<int>();
+  if (int rc = run_jvp(h, io, s)) return rc;
+  if (t_traj) {
+    CU(launch_soa_to_aos(io.t_traj, ga, B, (int)nv, s));
+    h->launches += 1;
+    CU(cudaMemcpyAsync(t_traj, ga, nb * nv * sizeof(double), cudaMemcpyDeviceToHost, s));
+  }
+  if (t_out8) CU(cudaMemcpyAsync(t_out8, io.t_out8, nb * 8 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (t_obj) CU(cudaMemcpyAsync(t_obj, io.t_obj, nb * sizeof(double), cudaMemcpyDeviceToHost, s));
   if (status) CU(cudaMemcpyAsync(status, h->status.p, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   return 0;

@@ -97,6 +97,20 @@ struct VjpCostIO : VjpIO {
 };
 cudaError_t launch_vjp(const Params& P, const VjpCostIO& io, double* ws, cudaStream_t stream);
 
+// Forward sensitivities of B returned solutions (Solver::jvp), one launch (mpc_jvp_kernel) in workspace region 0 of ws.
+// io_aos = 0: state6 / t_state6 [6][B], coeffs / t_coeffs [ncoef][B], cost8 / t_cost8 [8][B], model4 / t_model4 [4][B],
+// t_out8 [8][B]; io_aos = 1: the same per problem ([B][k]).  Always field-major: traj, t_traj [8N-2][B], mult [10N-4][B].
+// cost8 / model4 null: the handle's values; a null tangent counts as zero; t_out8, t_traj, t_obj [B] and status [B] may
+// be null.
+struct JvpIO {
+  int B = 0, ncoef = 0, io_aos = 0;
+  const double *state6 = nullptr, *coeffs = nullptr, *cost8 = nullptr, *model4 = nullptr, *traj = nullptr, *mult = nullptr;
+  const double *t_state6 = nullptr, *t_coeffs = nullptr, *t_cost8 = nullptr, *t_model4 = nullptr;
+  double *t_out8 = nullptr, *t_traj = nullptr, *t_obj = nullptr;
+  int* status = nullptr;
+};
+cudaError_t launch_jvp(const Params& P, const JvpIO& io, double* ws, cudaStream_t stream);
+
 // K6 batch I/O: [B][K] <-> [K][B]
 cudaError_t launch_aos_to_soa(const double* in, double* out, int B, int K, cudaStream_t stream);
 cudaError_t launch_soa_to_aos(const double* in, double* out, int B, int K, cudaStream_t stream);

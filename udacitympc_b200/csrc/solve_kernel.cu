@@ -752,6 +752,52 @@ cudaError_t launch_vjp(const Params& P, const VjpCostIO& io, double* ws, cudaStr
   return cudaGetLastError();
 }
 
+// Forward sensitivities of returned solutions (Solver::jvp): one thread per problem, workspace region 0 (slot = problem).
+// The rows as in mpc_vjp_kernel; the kModelRows instance also reads t_model4, at the model row or at the handle's values.
+template <int ROWS>
+__global__ void __launch_bounds__(kBlock) mpc_jvp_kernel(const __grid_constant__ Params P, const __grid_constant__ JvpIO A, double* ws) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= A.B) return;
+  const size_t nb = (size_t)A.B, bb = (size_t)b;
+  auto at = [&](int k, int n) { return A.io_aos ? bb * n + k : (size_t)k * nb + bb; };   // element k of n of problem b
+  Params Q = P;
+  Solver<32> S(ROWS ? Q : P, slot_base(P, ws, b), b & 31);
+  double s0[6], cf[kMaxCoef], ts6[6], tcf[kMaxCoef], tpar[8], tmod[4];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) { s0[k] = A.state6[at(k, 6)]; ts6[k] = A.t_state6 ? A.t_state6[at(k, 6)] : 0.0; }
+#pragma unroll
+  for (int i = 0; i < kMaxCoef; ++i) {
+    cf[i] = i < A.ncoef ? A.coeffs[at(i, A.ncoef)] : 0.0;
+    tcf[i] = i < A.ncoef && A.t_coeffs ? A.t_coeffs[at(i, A.ncoef)] : 0.0;
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i) tpar[i] = A.t_cost8 ? A.t_cost8[at(i, 8)] : 0.0;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) tmod[i] = ROWS == kModelRows && A.t_model4 ? A.t_model4[at(i, 4)] : 0.0;
+  // an invalid cost or model row: a NaN coefficient makes Solver::jvp return -13 with NaN outputs
+  if constexpr (ROWS == kCostRows) {
+    if (!cost_row(A.cost8, A.io_aos, A.B, b, Q)) cf[0] = NAN;
+  } else if constexpr (ROWS == kModelRows) {
+    bool ok = !A.cost8 || cost_row(A.cost8, A.io_aos, A.B, b, Q);
+    if (A.model4) ok &= model_row(A.model4, A.io_aos, A.B, b, Q);
+    if (!ok) cf[0] = NAN;
+  }
+  S.set_coeffs(cf, kMaxCoef);
+  double tobj;
+  const int st = S.jvp<ROWS == kModelRows>(s0, A.traj + b, nb, A.mult + b, nb, ts6, tcf, tpar, tmod, A.t_traj ? A.t_traj + b : nullptr,
+                                           nb, A.t_out8 ? A.t_out8 + at(0, 8) : nullptr, A.io_aos ? 1 : nb, tobj);
+  if (A.t_obj) A.t_obj[b] = tobj;
+  if (A.status) A.status[b] = st;
+}
+cudaError_t launch_jvp(const Params& P, const JvpIO& io, double* ws, cudaStream_t stream) {
+  if (io.B <= 0) return cudaSuccess;
+  const int grid = (io.B + kBlock - 1) / kBlock;
+  if (io.model4 || io.t_model4) mpc_jvp_kernel<kModelRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
+  else if (io.cost8) mpc_jvp_kernel<kCostRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
+  else mpc_jvp_kernel<kNoRows><<<grid, kBlock, 0, stream>>>(P, io, ws);
+  return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------------------------
 // FP64 peak: 8 independent dependent-FMA chains per thread.
 __global__ void __launch_bounds__(256) fp64_peak_kernel(double* sink, int iters) {
